@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: SPFF-UNet bf16 training step, voxels/s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1], SURVEY.md §8d "C2"): per GPU a synthetic batch 8x5x128^3 presented
@@ -202,6 +202,32 @@ def workload_config(n_gpus: int, variant: str = "SPFF-UNet", samples: int = SAMP
     }
 
 
+DUMP_MAX_ELEMS = 6_000_000      # per array: SPFF-UNet's parameters and gradients fit whole; 3DUNet's are sampled
+
+
+def dump_outputs(path: str, lit, out) -> None:
+    """What one training step hands its caller, as <path>/<name>.npy: the loss and the loss / metric tally fit_step
+    returns, and the parameters (state_dict order) and gradients (fused_grads order) the step leaves behind, each
+    flattened. An array longer than DUMP_MAX_ELEMS keeps the entries at fixed positions (a seeded permutation), so
+    two builds of the project compare entry for entry. The step is not bit-reproducible: two runs of one build
+    (`--steps 5 --warmup 3`, one B200 at a 1000 W power limit) differed by 3e-6 in the loss and, as rel-L2, by 1.4e-3
+    in the parameters and 1e-2 in the gradients."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    t = out["tally"]
+    arrays = {"loss": out["loss"].double(), "tally_nll": t.nll.double(), "tally_count": t.count.double(),
+              "confusion": t.confusion.double()}
+    for name, parts in (("params", lit.state_dict().values()), ("grads", lit.fused_grads().values())):
+        v = torch.cat([p.detach().reshape(-1).float() for p in parts])
+        if v.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            v = v[idx.to(v.device)]
+        arrays[name] = v
+    for name, v in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), v.cpu().numpy())
+
+
 def conv_traffic():
     """Mean DRAM bytes (read + write) per conv3_fprop_kernel launch from the committed ncu capture
     (profiles/r01f_conv_traffic.json: every conv launch of `SPFF_BENCH_SAMPLES=256 bench.py`, i.e. the same 256-slice
@@ -326,8 +352,10 @@ def run_b200(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t) * 1e-3
 
+    last = {}
+
     def step_resident():
-        return lit.fit_step((x_dev, lab_dev))
+        last["out"] = lit.fit_step((x_dev, lab_dev))
 
     def step_e2e():
         out = lit.fit_step((x_host, lab_host))            # H2D of images + labels inside
@@ -360,6 +388,8 @@ def run_b200(args):
     launches = _lib.CALLS - calls0
     clk = clocks.stop()
     conv = prof.summary()
+    if args.dump_outputs and rank == 0:      # before the e2e steps below move the weights on
+        dump_outputs(args.dump_outputs, lit, last["out"])
     # ---- end-to-end steps from pinned host memory ----
     step_e2e()
     sec_e2e = timed(step_e2e, args.steps, tag="e2e_ms_per_step")
@@ -444,7 +474,7 @@ def run_extras(args):
     out = {}
     for key, mode, variant in (("plaincore", "train", "PlainCore_UNet"), ("unet3d", "train", "3DUNet"), ("infer", "infer", "SPFF-UNet")):
         a = copy.copy(args)
-        a.variant, a.mode, a.no_cpu, a.no_extras = variant, mode, True, True
+        a.variant, a.mode, a.no_cpu, a.no_extras, a.dump_outputs = variant, mode, True, True, None
         a.steps, a.warmup = min(args.steps, 3), 3
         buf = io.StringIO()
         try:
@@ -561,7 +591,13 @@ def main():
                     help="SPFF-UNet is the headline (BASELINE.json configs[1]); the others are the controls of configs[3]")
     ap.add_argument("--mode", default="train", choices=["train", "infer"],
                     help="train: the headline step (default); infer: BASELINE.json configs[4], an extra line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed training step's loss, tally, parameters and gradients as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "train"):
+        ap.error("--dump-outputs writes the outputs of the training step (--impl b200 --mode train)")
     if args.impl == "reference":
         run_reference(args)
     elif args.mode == "infer":

@@ -10,7 +10,8 @@ Two levels:
     -> epoch means in `trainer.callback_metrics` -> logger / callbacks), `ReduceLROnPlateau` monitoring, checkpoint
     files with Lightning's key names (`state_dict`, `optimizer_states`, `hyper_parameters`, `epoch`, `global_step`) and
     resume. `install()` registers these under the `pytorch_lightning` module names so that the reference's unmodified
-    `train.py` / `test.py` can drive this package on a machine without Lightning (tests/test_trainpy_*.py do that).
+    `train.py` / `test.py` can drive this package on a machine without Lightning (tests/test_trainpy_gpu.py runs the
+    fit loop, checkpoints, reload and resume).
     It is deliberately small: one optimizer, no distributed strategies, no sanity-check / test / predict loops.
 """
 from __future__ import annotations

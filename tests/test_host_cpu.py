@@ -59,6 +59,7 @@ def test_variants_registry_surface():
         assert isinstance(opt["optimizer"], torch.optim.Adam) and opt["lr_scheduler"]["monitor"] == "val_macro_dice"
 
 
+@pytest.mark.usefixtures("reference_threads")
 def test_same_seed_same_init_and_keys_as_reference():
     """Constructing with the same seed draws bit-identical weights to the reference's constructors
     (checksums in tests/golden/init_seed42.npz come from the reference itself)."""

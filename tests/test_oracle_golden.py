@@ -26,6 +26,7 @@ def test_fixtures_exist():
     assert len(CASES) >= 5 and os.path.exists(os.path.join(GOLD, "init_seed42.npz"))
 
 
+@pytest.mark.usefixtures("reference_threads")
 @pytest.mark.parametrize("path", CASES, ids=[os.path.basename(p) for p in CASES])
 def test_oracle_matches_reference(path):
     z, variant, b, h, w, ign, seed = _load(path)

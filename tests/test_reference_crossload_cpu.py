@@ -1,39 +1,37 @@
-"""CPU, build container only (skipped where /root/reference is absent): the drop-in contract against the LIVE reference —
-state_dicts cross-load strictly in both directions for every variant, and the reference's own `train.py`-style builder
-loop (`_build_lit`, train.py:1251-1271: call the zero-arg builder, else try (num_classes, lr) / (num_classes) / ()) works
-on this tree's VARIANTS. No compute runs (there is no CPU path); this is registry + parameter-surface parity."""
-import os
-import sys
+"""CPU: the drop-in contract against the reference's parameter surface — state_dicts cross-load strictly in both
+directions for every variant, and the reference's own `train.py`-style builder loop (`_build_lit`, train.py:1251-1271:
+call the zero-arg builder, else try (num_classes, lr) / (num_classes) / ()) works on this tree's VARIANTS. No compute
+runs (there is no CPU path); this is registry + parameter-surface parity.
 
+The reference's state_dict of each variant (keys in order, shapes) is the one stored in tests/golden/init_seed42.npz
+and tests/golden/cicek_init_seed42.npz, written from the reference's own constructors by oracle/make_golden.py and
+oracle/make_golden_3dunet.py. Those files do not record dtypes: the dtypes the test expects (fp32, int64 for
+BatchNorm's `num_batches_tracked`) are PyTorch's defaults for these modules, an assumption of the test rather than a
+comparison with the reference."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "innovative3D")), reason="reference tree not mounted")
-
-REF_CLASS = {"SPFF-UNet": "LitSPCT_EFiLM_FourierGate", "E_SP_UNet": "LitSPCT_EnergyFiLM", "FG_SP_UNet": "LitSPCT_FourierGate",
-             "SP_UNet": "LitSPCT_SEspec", "PlainCore_UNet": "LitSPCT_ControlUNet"}
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+VARIANTS = ["SPFF-UNet", "E_SP_UNet", "FG_SP_UNet", "SP_UNet", "PlainCore_UNet", "3DUNet"]
 
 
-@pytest.fixture(scope="module")
-def reference_models():
-    """The reference's innovative3D.models, imported under the stub shim in a way that leaves this tree's
-    `innovative3D` package importable afterwards (the two share a package name)."""
-    mine = {k: v for k, v in sys.modules.items() if k == "innovative3D" or k.startswith("innovative3D.")}
-    for k in mine:
-        del sys.modules[k]
-    path0 = list(sys.path)
-    from oracle.make_golden import import_reference
-    M, _ = import_reference()
-    ref_mods = {k: v for k, v in sys.modules.items() if k == "innovative3D" or k.startswith("innovative3D.")}
-    for k in ref_mods:
-        del sys.modules[k]
-    sys.path[:] = path0
-    sys.modules.update(mine)
-    yield M
-    for name in ("pytorch_lightning", "pytorch_lightning.callbacks", "pytorch_lightning.loggers", "torchmetrics", "matplotlib",
-                 "matplotlib.pyplot", "matplotlib.patches", "seaborn", "pydicom"):
-        sys.modules.pop(name, None)
+def reference_surface(variant):
+    """[(key, shape)] of the reference's state_dict, in its order."""
+    if variant == "3DUNet":
+        z = np.load(os.path.join(GOLD, "cicek_init_seed42.npz"))
+        return [(k, tuple(int(v) for v in z[k][:-2])) for k in z.files]
+    z = np.load(os.path.join(GOLD, "init_seed42.npz"))
+    return [(k.split("|", 1)[1], tuple(int(v) for v in z[k][:-2])) for k in z.files if k.split("|", 1)[0] == variant]
+
+
+def reference_state_dict(variant, seed):
+    """A state_dict with the reference's keys, order and shapes; fp32 values (BatchNorm's step counter: int64)."""
+    g = torch.Generator().manual_seed(seed)
+    return {k: torch.randint(0, 1000, shape, generator=g, dtype=torch.int64) if k.endswith("num_batches_tracked")
+            else torch.randn(shape, generator=g) for k, shape in reference_surface(variant)}
 
 
 def _mine():
@@ -41,26 +39,23 @@ def _mine():
     return dict((v[0], v[1]) for v in C.VARIANTS)
 
 
-@pytest.mark.parametrize("variant", list(REF_CLASS) + ["3DUNet"])
-def test_state_dicts_cross_load(reference_models, variant):
-    M = reference_models
-    torch.manual_seed(1)
-    if variant == "3DUNet":
-        ref = M.LitCicek3DUNet_DepthAdapter_Published(num_classes=13, target_depth=16)
-    else:
-        ref = getattr(M, REF_CLASS[variant])()
+@pytest.mark.parametrize("variant", VARIANTS)
+def test_state_dicts_cross_load(variant):
+    sd_ref = reference_state_dict(variant, seed=1)
     torch.manual_seed(2)
     mine = _mine()[variant]()
-    sd_ref, sd_mine = ref.state_dict(), mine.state_dict()
+    sd_mine = mine.state_dict()
     assert list(sd_ref) == list(sd_mine)                       # same keys in the same order
     assert all(sd_ref[k].shape == sd_mine[k].shape and sd_ref[k].dtype == sd_mine[k].dtype for k in sd_ref)
     mine.load_state_dict(sd_ref, strict=True)
     assert all(torch.equal(mine.state_dict()[k], sd_ref[k]) for k in sd_ref)
     torch.manual_seed(3)
-    other = _mine()[variant]()
-    ref.load_state_dict(other.state_dict(), strict=True)
-    assert all(torch.equal(ref.state_dict()[k], other.state_dict()[k]) for k in sd_ref)
-    assert sum(p.numel() for p in ref.parameters()) == sum(p.numel() for p in mine.parameters())
+    other = _mine()[variant]().state_dict()
+    # what the reference's load_state_dict(strict=True) checks of this tree's state_dict: the same keys, the same shapes
+    assert [(k, tuple(v.shape)) for k, v in other.items()] == reference_surface(variant)
+    buffers = {k for k, _ in mine.named_buffers()}
+    assert sum(int(np.prod(s)) for k, s in reference_surface(variant) if k not in buffers) == \
+        sum(p.numel() for p in mine.parameters())
 
 
 def test_train_py_builder_loop_on_this_trees_variants():

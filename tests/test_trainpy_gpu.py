@@ -1,31 +1,14 @@
-"""GPU: the reference's unmodified `train.py` drives this repo's `innovative3D` package (SURVEY.md §8b / §8f-2), and the
-Lightning step surface of the SPCT classes (`_shared_step`, `training_step`, `validation_step`, `apply_unified_loss`:
-reference models.py:479-588, unified_loss.py:114-144) is checked against the oracle.
-
-`train.train_and_log` (train.py:1398-1583) is run as is — seed, `DataMod(trainval_sets, ...)`, `_build_lit`, the compute
-read-out, `TrainValCSVLogger`, both `ModelCheckpoint`s, `EarlyStopping`, `Trainer(...).fit`, the custom test pass
-`write_test_metrics_csv_from_pass` (full sklearn path), `write_summary_csv` — with a synthetic
-DataModule in place of the DICOM one and FINAL_EPOCHS cut to 2; then the checkpoint is reloaded the way
-`test.py:626-644` does and a second call resumes from `last.ckpt`. Lightning itself is the repo's stand-in when the real
-package is absent (tests/_ref_env.py)."""
-import os
-import sys
-
+"""GPU: the Lightning surface this package's callers drive. The fit loop of the Lightning stand-in
+(`innovative3D._lightning`: `Trainer`, `ModelCheckpoint`, `EarlyStopping`, `CSVLogger`, checkpoint files, reload and
+resume) trains SPFF-UNet on a synthetic DataModule the way the reference's `train.py` sets it up (train.py:1398-1583)
+and reloads it the way `test.py:615-644` does. The step surface of the SPCT classes (`_shared_step`, `training_step`,
+`validation_step`, `apply_unified_loss`: reference models.py:479-588, unified_loss.py:114-144) is checked against the
+oracle. Lightning itself is the repo's stand-in when the real package is absent."""
 import numpy as np
 import pytest
 import torch
 
 pytestmark = pytest.mark.gpu
-
-sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-import _ref_env  # noqa: E402
-
-
-@pytest.fixture(scope="module")
-def env(tmp_path_factory):
-    tmp = tmp_path_factory.mktemp("trainpy")
-    ref = _ref_env.prepare(tmp)
-    return ref, tmp, _ref_env.import_script(ref, "train")
 
 
 def _synthetic_datamodule():
@@ -69,58 +52,61 @@ def _synthetic_datamodule():
     return SyntheticDataModule
 
 
-def test_train_py_runs_end_to_end_and_checkpoint_reloads(env, monkeypatch):
-    import pandas as pd
-    ref, tmp, train = env
-    test_py = _ref_env.import_script(ref, "test")
-    DM = _synthetic_datamodule()
-    variants = dict((v[0], v) for v in train.VARIANTS)
-    name, builder, _, base = variants["SPFF-UNet"]
-    monkeypatch.setattr(train, "FINAL_EPOCHS", 2)
-    monkeypatch.setattr(train, "FAST_SKIP_VIZ", True)
-    monkeypatch.setattr(train, "IMAGE_HEIGHT", 64)     # the compute read-out runs the core on CPU at this size: keep it small
-    monkeypatch.setattr(train, "IMAGE_WIDTH", 64)
-    out = train.train_and_log(name, builder, DM, base, 42)
-    folder = train.CHECKPOINT_DIR / name / "seed42"
+def _fit(builder, folder, max_epochs, ckpt_path=None):
+    """One `Trainer(...).fit` with the callbacks train.py:1430-1458 configures: last + best checkpoint on
+    val_macro_dice, early stopping on it, a CSV logger. Returns the module, its logger and its best-checkpoint callback."""
+    from innovative3D import _lightning as L
+    dm = _synthetic_datamodule()([], batch_size=1, num_frames=5)
+    dm.setup("fit")
+    lit = builder()
+    best = L.ModelCheckpoint(dirpath=folder, filename="best-{epoch:02d}-{val_macro_dice:.4f}", monitor="val_macro_dice",
+                             mode="max", save_last=True, save_top_k=1)
+    stop = L.EarlyStopping(monitor="val_macro_dice", mode="max", patience=10)
+    logger = L.CSVLogger(save_dir=str(folder), name="logs")
+    L.Trainer(max_epochs=max_epochs, accelerator="gpu", devices=1, logger=logger,
+              callbacks=[best, stop]).fit(lit, datamodule=dm, ckpt_path=ckpt_path)
+    return lit, logger, best
+
+
+def test_trainer_fit_checkpoints_reload_and_resume(tmp_path):
+    from innovative3D import _lightning as L
+    from innovative3D import config as C
+    variants = dict((v[0], v[1]) for v in C.VARIANTS)
+    builder = variants["SPFF-UNet"]
+    folder = tmp_path / "SPFF-UNet" / "seed42"
+    L.seed_everything(42)
+    lit, logger, best = _fit(builder, folder, max_epochs=2)
     assert (folder / "last.ckpt").is_file()
-    best = sorted(folder.glob("best-*.ckpt"))
-    assert len(best) == 1, best
-    # TrainValCSVLogger rows: one train and one val row per epoch, val_macro_dice monitored (train.py:1438-1458)
-    log = pd.read_csv(folder / "logs" / "metrics.csv")
-    assert sorted(log["phase"].tolist()) == ["train", "train", "val", "val"]
-    assert log[log.phase == "val"]["val_macro_dice"].notna().all() and log[log.phase == "train"]["train_loss"].notna().all()
-    assert float(log[log.phase == "train"]["train_loss"].iloc[-1]) < float(log[log.phase == "train"]["train_loss"].iloc[0])
-    # the custom test pass of train.py wrote its files from model(x) of this package
-    tm = pd.read_csv(folder / "logs" / "test_metrics.csv")
-    assert 0.0 <= float(tm["test_macro_dice"].iloc[-1]) <= 1.0 and "test_pr_auc_macro" in tm.columns
-    # (train.py:262-331 `write_test_details_3d` compares device predictions with host labels and raises on any CUDA
-    # model, the reference's own included; train.py:1549-1556 catches it and goes on - so no test_details.csv here)
-    assert out == "DONE" or 0.0 <= float(out) <= 1.0
+    best_files = sorted(folder.glob("best-*.ckpt"))
+    assert len(best_files) == 1 and str(best_files[0]) == best.best_model_path, best_files
+    # one train and one val row per epoch, val_macro_dice monitored
+    train_rows = [r for r in logger.rows if "train_loss" in r]
+    val_rows = [r for r in logger.rows if "val_macro_dice" in r]
+    assert [r["epoch"] for r in train_rows] == [0, 1] and [r["epoch"] for r in val_rows] == [0, 1]
+    assert all(np.isfinite(r["val_macro_dice"]) for r in val_rows) and all(np.isfinite(r["train_loss"]) for r in train_rows)
+    assert float(train_rows[-1]["train_loss"]) < float(train_rows[0]["train_loss"])
 
     # ---- reload like test.py:615-644: prototype from the registry, PL restore, manual fallback ------------------
     ckpt_path = str(folder / "last.ckpt")
     proto = builder()
     ModelCls = proto.__class__
     dev = torch.device("cuda")
-    try:      # "PL restore attempt" (test.py:626-630). For this class it raises with real Lightning and the reference's
-        # own module too: the saved hyper-parameter `is_3d` travels through **kw into UNet3D_SpectralCore.__init__
-        # (models.py:1558-1564 -> :1547-1555 -> :654) - which is why test.py carries the manual fallback below
-        restored = ModelCls.load_from_checkpoint(ckpt_path, map_location=dev)
-    except TypeError:
-        restored = None
-    assert restored is None
+    # "PL restore attempt" (test.py:626-630). For this class it raises with real Lightning and the reference's own
+    # module too: the saved hyper-parameter `is_3d` travels through **kw into UNet3D_SpectralCore.__init__
+    # (models.py:1558-1564 -> :1547-1555 -> :654) - which is why test.py carries the manual fallback below
+    with pytest.raises(TypeError):
+        ModelCls.load_from_checkpoint(ckpt_path, map_location=dev)
     ck = torch.load(ckpt_path, map_location=dev, weights_only=False)
     assert {"state_dict", "optimizer_states", "epoch", "global_step", "hyper_parameters"} <= set(ck)
     assert ck["epoch"] == 1 and ck["global_step"] == 12
-    sd = test_py._align_state_dict_keys(ck.get("state_dict", ck), proto.state_dict())
-    proto.load_state_dict(sd, strict=False)
+    proto.load_state_dict(ck["state_dict"], strict=False)
     manual = proto.to(dev).eval()
     x = _synthetic_datamodule()([], 1, 5)
     x.setup("test")
     xb, _ = next(iter(x.test_dataloader()))
     # a class without **kw restores through the PL path: SP_UNet (models.py:1585-1592)
-    sp = dict((v[0], v[1]) for v in train.VARIANTS)["SP_UNet"]()
-    sp_path = str(tmp / "sp_unet.ckpt")
+    sp = variants["SP_UNet"]()
+    sp_path = str(tmp_path / "sp_unet.ckpt")
     torch.save({"state_dict": sp.state_dict(), "hyper_parameters": dict(sp.hparams)}, sp_path)
     sp2 = type(sp).load_from_checkpoint(sp_path, map_location=dev)
     assert all(torch.equal(a.cpu(), b.cpu()) for a, b in zip(sp.state_dict().values(), sp2.state_dict().values()))
@@ -132,20 +118,17 @@ def test_train_py_runs_end_to_end_and_checkpoint_reloads(env, monkeypatch):
     fresh = builder().to(dev).eval()
     with torch.no_grad():
         assert not torch.equal(fresh(xb.to(dev)), a)
-    logits = test_py._extract_logits_from_output(a, prefer_classes=13)
-    assert logits is a
 
-    # ---- resume: a second call finds last.ckpt (train.py:504-509, 1509-1516) and runs only the missing epoch ----
-    monkeypatch.setattr(train, "FINAL_EPOCHS", 3)
-    train.train_and_log(name, builder, DM, base, 42)
-    log2 = pd.read_csv(folder / "logs" / "metrics.csv")
-    assert sorted(log2["epoch"].astype(int).tolist()) == [0, 0, 1, 1, 2, 2]
+    # ---- resume: a second fit from last.ckpt (train.py:504-509, 1509-1516) runs only the missing epoch ---------
+    _, logger2, _ = _fit(builder, folder, max_epochs=3, ckpt_path=ckpt_path)
+    epochs = sorted(int(r["epoch"]) for r in logger.rows + logger2.rows)
+    assert epochs == [0, 0, 1, 1, 2, 2]
     ck2 = torch.load(folder / "last.ckpt", map_location="cpu", weights_only=False)
     assert ck2["epoch"] == 2 and ck2["global_step"] == 18
 
 
 @pytest.mark.parametrize("variant", ["SPFF-UNet", "PlainCore_UNet", "SP_UNet"])
-def test_lightning_step_surface_matches_the_oracle(env, variant):
+def test_lightning_step_surface_matches_the_oracle(variant):
     """training_step returns the differentiable ce_plus_macro_dice loss and logs the reference's metric names;
     validation_step returns {'val_loss': ...} and logs val_macro_dice (the monitored quantity)."""
     from innovative3D import config as C
@@ -181,7 +164,7 @@ def test_lightning_step_surface_matches_the_oracle(env, variant):
     assert abs(float(t) - float(want)) < 1e-5 and "test_macro_dice" in lit.logged
 
 
-def test_apply_unified_loss_patches_every_lit_class(env):
+def test_apply_unified_loss_patches_every_lit_class():
     """unified_loss.apply_unified_loss (unified_loss.py:114-144): every Lightning class of innovative3D.models except
     BaseLitModel gets the unified train/val/test steps; they compute the same loss and log the macro/micro metrics."""
     from innovative3D import models as M
