@@ -243,6 +243,16 @@ int spff_head_loss_fused(const void* x, long long ldx, int cin, const float* w, 
                          const float* gscale, double* acc, long long* counts, long long* confusion, void* dx,
                          long long lddx, float* dw, float* db, float beta, void* workspace, size_t workspace_bytes,
                          void* stream);
+/* Fused EVALUATION head: head_fwd + ce_confusion in one pass over x, forward only; the logits are never
+ * materialised. acc/counts/confusion accumulate (+=) over the batch exactly as in spff_ce_confusion (labels
+ * uint8 or int64, ignore_index skipped, labels outside [0,K) counted in acc/counts but not in confusion), from
+ * the logits and first-maximum arg-max of spff_head_loss_fused. sample_acc[n], sample_counts[n],
+ * sample_confusion[n][K][K] receive (+=) the same tally per sample (all three NULL = off); labels_out uint8
+ * [N,D,H,W] receives the arg-max the tally counts (NULL = off). Any D*H*W; N <= 65535. */
+int spff_head_eval(const void* x, long long ldx, int cin, const float* w, const float* b, const void* labels,
+                   int label_bytes, int ignore_index, int k, spff_shape s, double* acc, long long* counts,
+                   long long* confusion, double* sample_acc, long long* sample_counts, long long* sample_confusion,
+                   uint8_t* labels_out, void* stream);
 
 /* ---- "3DUNet" control: Cicek3DUNet + depth adapter (models.py:718-777; config.py:283-311) ---------------
  * Its 3x3x3 convolutions, normalise + ReLU passes (slope 0), head and loss are the entry points above;

@@ -3,7 +3,7 @@
 //     with in_channels = 1, models.py:1551) — 27 taps x 32 outputs per voxel: forward on the CUDA cores,
 //     weight gradient as a warp-level mma.sync GEMM (the network input needs no gradient);
 //   * the 1x1x1 classification head nn.Conv3d(32, num_classes, 1) (models.py:674) forward, arg-max
-//     and backward;
+//     and backward, fused with the loss for training and, forward only, for evaluation;
 //   * cross-entropy with ignore_index + the hard confusion tally that macro_dice_loss and
 //     per_class_metrics_3d derive all their counts from (innovative3D/helpers.py:668-725, 782-803);
 //   * Adam (BaseLitModel.configure_optimizers, models.py:591-594).
@@ -993,6 +993,125 @@ __device__ __forceinline__ void split_bf16x2(float v0, float v1, uint32_t& hi, u
   lo = *reinterpret_cast<const uint32_t*>(&l);
 }
 
+// ---- pieces shared by the fused training head (head_loss_mma_kernel) and the fused evaluation head
+// (head_eval_mma_kernel): one warp works on tiles of 16 positions x 32 channels; g = lane / 4, t = lane % 4.
+
+// B fragments of the logits contraction: B[k=ch][n=class] as bf16 hi + lo of W, plus the bias (classes >= K are zero)
+struct HmLogitW {
+  uint32_t hi[2][2][2], lo[2][2][2];   // [class tile][k step][b0,b1]
+  float bias[2][2];
+};
+
+__device__ __forceinline__ void hm_logit_weights(int K, int g, int t, HmLogitW& w) {
+  auto wv = [&](int k, int c) -> float { return k < K ? c_head_w[k * kHeadC + c] : 0.f; };
+#pragma unroll
+  for (int nt = 0; nt < 2; ++nt)
+#pragma unroll
+    for (int ks = 0; ks < 2; ++ks)
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int cls = 8 * nt + g, ch = 16 * ks + 8 * h + 2 * t;
+        split_bf16x2(wv(cls, ch), wv(cls, ch + 1), w.hi[nt][ks][h], w.lo[nt][ks][h]);
+      }
+#pragma unroll
+  for (int nt = 0; nt < 2; ++nt)
+#pragma unroll
+    for (int e = 0; e < 2; ++e) w.bias[nt][e] = (8 * nt + 2 * t + e) < K ? c_head_b[8 * nt + 2 * t + e] : 0.f;
+}
+
+// x rows (two 16-byte halves per lane) and the labels of rows g, g + 8 of `tile`; zeros / ignore_index past `total`
+template <typename LabelT>
+__device__ __forceinline__ void hm_fetch(const __nv_bfloat16* __restrict__ x, long long ldx, const void* __restrict__ labels,
+                                         int ignore_index, long long total, long long ntiles, long long tile, int lane,
+                                         uint4& nx0, uint4& nx1, int (&nlab)[2]) {
+  const int g = lane >> 2;
+  nx0 = nx1 = make_uint4(0, 0, 0, 0);
+  nlab[0] = nlab[1] = ignore_index;
+  if (tile >= ntiles) return;
+  const long long q0 = tile * 16;
+  const int pos = lane >> 1, half = lane & 1;
+  if (q0 + pos < total) {
+    const uint4* src = reinterpret_cast<const uint4*>(x + (q0 + pos) * ldx + half * 16);
+    nx0 = __ldg(src);
+    nx1 = __ldg(src + 1);
+  }
+#pragma unroll
+  for (int rr = 0; rr < 2; ++rr)
+    if (q0 + g + 8 * rr < total) nlab[rr] = static_cast<int>(static_cast<const LabelT*>(labels)[q0 + g + 8 * rr]);
+}
+
+// stage the fetched 16 positions x 32 channels into the warp's tile
+__device__ __forceinline__ void hm_stage(__nv_bfloat16 (*xs)[kHmXPitch], int lane, const uint4& nx0, const uint4& nx1) {
+  const int pos = lane >> 1, half = lane & 1;
+  uint4* dst = reinterpret_cast<uint4*>(&xs[pos][half * 16]);
+  dst[0] = nx0;
+  dst[1] = nx1;
+}
+
+// logits of the staged tile: l[class tile][row g: 0..1 | row g + 8: 2..3] for classes 8 * tile + 2t + {0, 1}
+__device__ __forceinline__ void hm_logits(__nv_bfloat16 (*xs)[kHmXPitch], int lane, const HmLogitW& w, float (&l)[2][4]) {
+#pragma unroll
+  for (int nt = 0; nt < 2; ++nt) {
+    l[nt][0] = l[nt][2] = w.bias[nt][0];
+    l[nt][1] = l[nt][3] = w.bias[nt][1];
+  }
+#pragma unroll
+  for (int ks = 0; ks < 2; ++ks) {
+    uint32_t a[4];
+    const int mi = lane >> 3, r = lane & 7;
+    const uint32_t addr = smem_u32_local(&xs[r + 8 * (mi & 1)][16 * ks + 8 * (mi >> 1)]);
+    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
+                 : "=r"(a[0]), "=r"(a[1]), "=r"(a[2]), "=r"(a[3]) : "r"(addr));
+#pragma unroll
+    for (int nt = 0; nt < 2; ++nt) {
+      mma_bf16_16816(l[nt], a, w.hi[nt][ks]);
+      mma_bf16_16816(l[nt], a, w.lo[nt][ks]);
+    }
+  }
+}
+
+// softmax statistics of row g + 8 * rr (the 4 lanes of a quad hold 4 classes each): the row's maximum and its first
+// arg-max (torch.argmax), e[q] = exp(v[q] - max) of this lane's classes cls[q], their quad sum se, and the logit of
+// class `lab` (0 when `lab` is not a class)
+__device__ __forceinline__ void hm_row_softmax(const float (&l)[2][4], int rr, int t, int K, int lab, float (&v)[4],
+                                               int (&cls)[4], float& mx, int& arg, float (&e)[4], float& se, float& ll) {
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    cls[q] = 8 * (q >> 1) + 2 * t + (q & 1);
+    v[q] = cls[q] < K ? l[q >> 1][2 * rr + (q & 1)] : -INFINITY;
+  }
+  mx = v[0];
+  arg = cls[0];
+#pragma unroll
+  for (int q = 1; q < 4; ++q)
+    if (v[q] > mx) {   // ascending class order inside the thread: strict > keeps the first maximum
+      mx = v[q];
+      arg = cls[q];
+    }
+#pragma unroll
+  for (int o = 1; o <= 2; o <<= 1) {
+    const float om = __shfl_xor_sync(0xffffffffu, mx, o);
+    const int oa = __shfl_xor_sync(0xffffffffu, arg, o);
+    if (om > mx || (om == mx && oa < arg)) {
+      mx = om;
+      arg = oa;
+    }
+  }
+  se = 0.f;
+  ll = 0.f;
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    e[q] = cls[q] < K ? __expf(v[q] - mx) : 0.f;
+    se += e[q];
+    if (cls[q] == lab) ll = v[q];
+  }
+#pragma unroll
+  for (int o = 1; o <= 2; o <<= 1) {
+    se += __shfl_xor_sync(0xffffffffu, se, o);
+    ll += __shfl_xor_sync(0xffffffffu, ll, o);
+  }
+}
+
 template <typename LabelT>
 __global__ void __launch_bounds__(kHmWarps * 32, kHmBlocksPerSm)
 head_loss_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const void* __restrict__ labels, int ignore_index,
@@ -1017,16 +1136,8 @@ head_loss_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
 
   // weight fragments (constant memory -> registers), classes >= K are zero
   auto wv = [&](int k, int c) -> float { return k < K ? c_head_w[k * kHeadC + c] : 0.f; };
-  uint32_t wl_hi[2][2][2], wl_lo[2][2][2];   // logits: [class tile][k step][b0,b1]: B[k=ch][n=class]
-#pragma unroll
-  for (int nt = 0; nt < 2; ++nt)
-#pragma unroll
-    for (int ks = 0; ks < 2; ++ks)
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const int cls = 8 * nt + g, ch = 16 * ks + 8 * h + 2 * t;
-        split_bf16x2(wv(cls, ch), wv(cls, ch + 1), wl_hi[nt][ks][h], wl_lo[nt][ks][h]);
-      }
+  HmLogitW wl;
+  hm_logit_weights(K, g, t, wl);
   uint32_t wd_hi[4][2], wd_lo[4][2];          // dx: [channel tile][b0,b1]: B[k=class][n=ch]
 #pragma unroll
   for (int j = 0; j < 4; ++j)
@@ -1035,11 +1146,6 @@ head_loss_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
       const int cls = 8 * h + 2 * t, ch = 8 * j + g;
       split_bf16x2(wv(cls, ch), wv(cls + 1, ch), wd_hi[j][h], wd_lo[j][h]);
     }
-  float bias[2][2];
-#pragma unroll
-  for (int nt = 0; nt < 2; ++nt)
-#pragma unroll
-    for (int e = 0; e < 2; ++e) bias[nt][e] = (8 * nt + 2 * t + e) < K ? c_head_b[8 * nt + 2 * t + e] : 0.f;
 
   float dwacc[4][4], dbp[2][2];
 #pragma unroll
@@ -1056,53 +1162,17 @@ head_loss_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
   // computed, so the two global round trips per tile overlap the tensor-core work instead of preceding it
   uint4 nx0 = make_uint4(0, 0, 0, 0), nx1 = nx0;
   int nlab[2] = {ignore_index, ignore_index};
-  auto fetch = [&](long long tile) {
-    nx0 = nx1 = make_uint4(0, 0, 0, 0);
-    nlab[0] = nlab[1] = ignore_index;
-    if (tile >= ntiles) return;
-    const long long q0 = tile * 16;
-    const int pos = lane >> 1, half = lane & 1;
-    if (q0 + pos < total) {
-      const uint4* src = reinterpret_cast<const uint4*>(x + (q0 + pos) * ldx + half * 16);
-      nx0 = __ldg(src);
-      nx1 = __ldg(src + 1);
-    }
-#pragma unroll
-    for (int rr = 0; rr < 2; ++rr)
-      if (q0 + g + 8 * rr < total) nlab[rr] = static_cast<int>(static_cast<const LabelT*>(labels)[q0 + g + 8 * rr]);
-  };
-  fetch(static_cast<long long>(blockIdx.x) * kHmWarps + warp);
+  hm_fetch<LabelT>(x, ldx, labels, ignore_index, total, ntiles, static_cast<long long>(blockIdx.x) * kHmWarps + warp, lane,
+                   nx0, nx1, nlab);
   for (long long tile = static_cast<long long>(blockIdx.x) * kHmWarps + warp; tile < ntiles; tile += tstep) {
     const long long p0 = tile * 16;
     const int clab[2] = {nlab[0], nlab[1]};
-    {  // stage 16 positions x 32 channels (zeros past the end)
-      const int pos = lane >> 1, half = lane & 1;
-      uint4* dst = reinterpret_cast<uint4*>(&xs[warp][pos][half * 16]);
-      dst[0] = nx0;
-      dst[1] = nx1;
-    }
-    fetch(tile + tstep);
+    hm_stage(xs[warp], lane, nx0, nx1);   // 16 positions x 32 channels (zeros past the end)
+    hm_fetch<LabelT>(x, ldx, labels, ignore_index, total, ntiles, tile + tstep, lane, nx0, nx1, nlab);
     __syncwarp();
     // ---- logits
     float l[2][4];
-#pragma unroll
-    for (int nt = 0; nt < 2; ++nt) {
-      l[nt][0] = l[nt][2] = bias[nt][0];
-      l[nt][1] = l[nt][3] = bias[nt][1];
-    }
-#pragma unroll
-    for (int ks = 0; ks < 2; ++ks) {
-      uint32_t a[4];
-      const int mi = lane >> 3, r = lane & 7;
-      const uint32_t addr = smem_u32_local(&xs[warp][r + 8 * (mi & 1)][16 * ks + 8 * (mi >> 1)]);
-      asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-                   : "=r"(a[0]), "=r"(a[1]), "=r"(a[2]), "=r"(a[3]) : "r"(addr));
-#pragma unroll
-      for (int nt = 0; nt < 2; ++nt) {
-        mma_bf16_16816(l[nt], a, wl_hi[nt][ks]);
-        mma_bf16_16816(l[nt], a, wl_lo[nt][ks]);
-      }
-    }
+    hm_logits(xs[warp], lane, wl, l);
     // ---- per-row softmax / CE / arg-max: row g (values [nt][0..1]) and row g + 8 (values [nt][2..3])
     float dl[2][4];
 #pragma unroll
@@ -1111,42 +1181,9 @@ head_loss_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
       const bool inb = pos < total;
       const int lab = clab[rr];
       const bool valid = inb && lab != ignore_index;
-      float v[4];
-      int cls[4];
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        cls[q] = 8 * (q >> 1) + 2 * t + (q & 1);
-        v[q] = cls[q] < K ? l[q >> 1][2 * rr + (q & 1)] : -INFINITY;
-      }
-      float mx = v[0];
-      int arg = cls[0];
-#pragma unroll
-      for (int q = 1; q < 4; ++q)
-        if (v[q] > mx) {   // ascending class order inside the thread: strict > keeps the first maximum
-          mx = v[q];
-          arg = cls[q];
-        }
-#pragma unroll
-      for (int o = 1; o <= 2; o <<= 1) {
-        const float om = __shfl_xor_sync(0xffffffffu, mx, o);
-        const int oa = __shfl_xor_sync(0xffffffffu, arg, o);
-        if (om > mx || (om == mx && oa < arg)) {
-          mx = om;
-          arg = oa;
-        }
-      }
-      float e[4], se = 0.f, ll = 0.f;
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        e[q] = cls[q] < K ? __expf(v[q] - mx) : 0.f;
-        se += e[q];
-        if (cls[q] == lab) ll = v[q];
-      }
-#pragma unroll
-      for (int o = 1; o <= 2; o <<= 1) {
-        se += __shfl_xor_sync(0xffffffffu, se, o);
-        ll += __shfl_xor_sync(0xffffffffu, ll, o);
-      }
+      float v[4], mx, e[4], se, ll;
+      int cls[4], arg;
+      hm_row_softmax(l, rr, t, K, lab, v, cls, mx, arg, e, se, ll);
       if (valid && t == 0) {
         nll_sum += (mx + __logf(se)) - ll;
         ++cnt;
@@ -1274,6 +1311,102 @@ head_loss_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
   }
   for (int i = threadIdx.x; i < K * K; i += blockDim.x)
     if (s_conf[i]) atomicAdd(confusion + i, static_cast<unsigned long long>(s_conf[i]));
+}
+
+// ---------------------------------------------------------------------------------------------
+// Fused EVALUATION head: the logits / softmax / arg-max of head_loss_mma_kernel (same functions, so the same
+// numbers) followed by the CE / confusion tally of ce_kernel, with no gradient. Block (x, y) works on sample y
+// only, so a block's tally belongs to one sample: it is kept in shared memory and flushed once per block to
+// the batch arrays and, when given, to the sample's row of the per-sample arrays. Optionally the arg-max map
+// (the one the tally counts) is written. Traffic: the 64 B of x + the label per voxel (+ 1 B of arg-max).
+// ---------------------------------------------------------------------------------------------
+constexpr int kHeBlocksPerSm = 3;
+
+template <typename LabelT>
+__global__ void __launch_bounds__(kHmWarps * 32, kHeBlocksPerSm)
+head_eval_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const void* __restrict__ labels, int ignore_index,
+                     int K, long long dhw, double* __restrict__ acc, unsigned long long* __restrict__ counts,
+                     unsigned long long* __restrict__ confusion, double* __restrict__ sample_acc,
+                     unsigned long long* __restrict__ sample_counts, unsigned long long* __restrict__ sample_confusion,
+                     uint8_t* __restrict__ labels_out) {
+  __shared__ __align__(16) __nv_bfloat16 xs[kHmWarps][16][kHmXPitch];
+  __shared__ unsigned int s_conf[kMaxK * kMaxK];
+  __shared__ float s_nll[kHmWarps];
+  __shared__ unsigned int s_cnt[kHmWarps];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int g = lane >> 2, t = lane & 3;
+  for (int i = threadIdx.x; i < K * K; i += blockDim.x) s_conf[i] = 0;
+  __syncthreads();
+  HmLogitW wl;
+  hm_logit_weights(K, g, t, wl);
+  const long long n = blockIdx.y;
+  const long long base = n * dhw;   // this block's sample: positions [base, base + dhw)
+  x += base * ldx;
+  labels = static_cast<const LabelT*>(labels) + base;
+  if (labels_out) labels_out += base;
+  float nll_sum = 0.f;
+  unsigned int cnt = 0;
+  const long long ntiles = (dhw + 15) / 16;
+  const long long tstep = static_cast<long long>(gridDim.x) * kHmWarps;
+  uint4 nx0 = make_uint4(0, 0, 0, 0), nx1 = nx0;
+  int nlab[2] = {ignore_index, ignore_index};
+  hm_fetch<LabelT>(x, ldx, labels, ignore_index, dhw, ntiles, static_cast<long long>(blockIdx.x) * kHmWarps + warp, lane,
+                   nx0, nx1, nlab);
+  for (long long tile = static_cast<long long>(blockIdx.x) * kHmWarps + warp; tile < ntiles; tile += tstep) {
+    const long long p0 = tile * 16;
+    const int clab[2] = {nlab[0], nlab[1]};
+    hm_stage(xs[warp], lane, nx0, nx1);
+    hm_fetch<LabelT>(x, ldx, labels, ignore_index, dhw, ntiles, tile + tstep, lane, nx0, nx1, nlab);
+    __syncwarp();
+    float l[2][4];
+    hm_logits(xs[warp], lane, wl, l);
+#pragma unroll
+    for (int rr = 0; rr < 2; ++rr) {
+      const long long pos = p0 + g + 8 * rr;
+      const bool inb = pos < dhw;
+      const int lab = clab[rr];
+      float v[4], mx, e[4], se, ll;
+      int cls[4], arg;
+      hm_row_softmax(l, rr, t, K, lab, v, cls, mx, arg, e, se, ll);
+      if (inb && t == 0) {
+        if (labels_out) labels_out[pos] = static_cast<uint8_t>(arg);
+        if (lab != ignore_index) {
+          nll_sum += (mx + __logf(se)) - ll;
+          ++cnt;
+          if (lab >= 0 && lab < K) atomicAdd(&s_conf[lab * K + arg], 1u);
+        }
+      }
+    }
+    __syncwarp();   // the tile is read before the next iteration overwrites it
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    nll_sum += __shfl_xor_sync(0xffffffffu, nll_sum, o);
+    cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+  }
+  if (lane == 0) {
+    s_nll[warp] = nll_sum;
+    s_cnt[warp] = cnt;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double tt = 0;
+    unsigned long long c = 0;
+    for (int wvv = 0; wvv < kHmWarps; ++wvv) {
+      tt += s_nll[wvv];
+      c += s_cnt[wvv];
+    }
+    atomicAdd(acc, tt);
+    atomicAdd(counts, c);
+    if (sample_acc) {
+      atomicAdd(sample_acc + n, tt);
+      atomicAdd(sample_counts + n, c);
+    }
+  }
+  for (int i = threadIdx.x; i < K * K; i += blockDim.x)
+    if (s_conf[i]) {
+      atomicAdd(confusion + i, static_cast<unsigned long long>(s_conf[i]));
+      if (sample_confusion) atomicAdd(sample_confusion + n * K * K + i, static_cast<unsigned long long>(s_conf[i]));
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1547,6 +1680,42 @@ int spff_head_loss_fused(const void* x, long long ldx, int cin, const float* w, 
   const int tot = k * spff::kHeadC + k;
   spff::head_bwd_reduce_kernel<<<(tot + 127) / 128, 128, 0, st>>>(static_cast<const float*>(workspace), blocks, k, beta,
                                                                  dw, db);
+  SPFF_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int spff_head_eval(const void* x, long long ldx, int cin, const float* w, const float* b, const void* labels,
+                   int label_bytes, int ignore_index, int k, spff_shape s, double* acc, long long* counts,
+                   long long* confusion, double* sample_acc, long long* sample_counts, long long* sample_confusion,
+                   uint8_t* labels_out, void* stream) {
+  SPFF_ENTRY_CHECK();
+  SPFF_REQUIRE(x && w && b && labels && acc && counts && confusion, "head_eval: null pointer");
+  SPFF_REQUIRE((sample_acc != nullptr) == (sample_counts != nullptr) && (sample_acc != nullptr) == (sample_confusion != nullptr),
+               "head_eval: the per-sample arrays are given together or not at all");
+  SPFF_REQUIRE(label_bytes == 1 || label_bytes == 8, "head_eval: labels must be uint8 or int64");
+  SPFF_REQUIRE(ldx >= cin && ldx % 8 == 0, "head_eval: bad channel pitch");
+  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "head_eval: bad shape");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int e = spff::upload_head(w, b, k, cin, st);
+  if (e) return e;
+  const long long dhw = static_cast<long long>(s.d) * s.h * s.w;
+  // blocks never straddle samples (grid.y = sample); grid.x spreads a sample over enough blocks for ~4 waves of
+  // kHeBlocksPerSm resident blocks per SM, and no more blocks than the sample has warp tiles for
+  const long long warp_tiles = ((dhw + 15) / 16 + spff::kHmWarps - 1) / spff::kHmWarps;
+  long long per = (4LL * spff::kHeBlocksPerSm * spff::num_sms() + s.n - 1) / s.n;
+  if (per > warp_tiles) per = warp_tiles;
+  if (per < 1) per = 1;
+  const dim3 grid(static_cast<unsigned>(per), s.n);
+  auto cnt = reinterpret_cast<unsigned long long*>(counts);
+  auto conf = reinterpret_cast<unsigned long long*>(confusion);
+  auto scnt = reinterpret_cast<unsigned long long*>(sample_counts);
+  auto sconf = reinterpret_cast<unsigned long long*>(sample_confusion);
+  if (label_bytes == 1)
+    spff::head_eval_mma_kernel<uint8_t><<<grid, spff::kHmWarps * 32, 0, st>>>(
+        static_cast<const bf16*>(x), ldx, labels, ignore_index, k, dhw, acc, cnt, conf, sample_acc, scnt, sconf, labels_out);
+  else
+    spff::head_eval_mma_kernel<long long><<<grid, spff::kHmWarps * 32, 0, st>>>(
+        static_cast<const bf16*>(x), ldx, labels, ignore_index, k, dhw, acc, cnt, conf, sample_acc, scnt, sconf, labels_out);
   SPFF_CUDA(cudaGetLastError());
   return 0;
 }

@@ -173,6 +173,15 @@ def per_class_metrics_3d(preds, labels, num_classes, smooth=1e-6, ignore_index=N
     return metrics_from_confusion(cm, labels.numel(), smooth)
 
 
+def sample_metrics(per_sample, voxels_per_sample: int, smooth: float = 1e-6) -> List[tuple]:
+    """Per-case metrics: one per_class_metrics_3d 9-tuple per sample from the per-sample tallies of `eval_step`
+    (`per_sample` = (nll [B], count [B], confusion [B,K,K]); only the confusion rows are read). `voxels_per_sample`
+    counts every voxel of one sample as given, ignored ones included (metrics_from_confusion)."""
+    cm = per_sample[2]
+    cm = cm.cpu().numpy() if torch.is_tensor(cm) else np.asarray(cm)
+    return [metrics_from_confusion(row, voxels_per_sample, smooth) for row in cm]
+
+
 def per_class_metrics_2d(preds, labels, num_classes, smooth=1e-6, ignore_index=None):
     """2-D twin (helpers.py:728-779): same counting rules on [B,K,H,W] logits."""
     return per_class_metrics_3d(preds, labels, num_classes, smooth, ignore_index)

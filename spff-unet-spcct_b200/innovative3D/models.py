@@ -651,6 +651,88 @@ class BaseLitModel(pl.LightningModule):
         """per_class_metrics_3d's 9-tuple from a fit_step tally (one device->host copy)."""
         return metrics_from_confusion(tally.confusion.cpu().numpy(), total_voxels)
 
+    # -- B200-native fused evaluation step --------------------------------------------------------
+    @torch.no_grad()
+    def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False,
+                  sample_group: Optional[int] = None):
+        """The loss statistics of `ce_plus_macro_dice_loss(model(x), y)` and `per_class_metrics_3d` without the logits:
+        forward, head, CE and confusion tally in the engine's sample-group schedule. Takes the batch forms `fit_step`
+        takes (tuple or dict; host or device; uint8 or int64 labels) and accumulates into `tally` (a fresh LossTally when
+        None). Touches no parameter, gradient or optimizer state and does not synchronise the host.
+
+        Returns {"loss": device scalar of the tally so far, "tally", "per_sample": (nll fp64 [B], count int64 [B],
+        confusion int64 [B,K,K]) or None, "labels": uint8 arg-max map [B,F,H,W] or None}."""
+        imgs, lbls = batch if isinstance(batch, (list, tuple)) else (batch["image"], batch["label"])
+        imgs, lbls = _pick_first_if_seq(imgs), _pick_first_if_seq(lbls)
+        core: UNet3D_SpectralCore = self.model
+        if imgs.ndim == 4:
+            imgs = imgs.unsqueeze(1)
+        core.materialize(imgs.shape[2])
+        dev = core._flat.device
+        if lbls.dtype not in (torch.uint8, torch.int64):
+            lbls = lbls.long()
+        group = sample_group or core.sample_group
+        staged = None
+        if not imgs.is_cuda and not lbls.is_cuda:
+            if self._copy_stream is None:
+                self._copy_stream = torch.cuda.Stream(device=dev)
+            staged = StagedBatch(imgs, lbls, dev, group, self._copy_stream)
+            imgs, lbls = staged.x, staged.labels
+        else:
+            imgs = imgs.to(dev, non_blocking=True)
+            lbls = lbls.to(dev, non_blocking=True)
+        k = self.hparams.num_classes
+        tally = LossTally(k, dev) if tally is None else tally
+        bsz = imgs.shape[0]
+        rows = (torch.zeros(bsz, dtype=torch.float64, device=dev), torch.zeros(bsz, dtype=torch.int64, device=dev),
+                torch.zeros(bsz, k, k, dtype=torch.int64, device=dev)) if per_sample else None
+        labels = torch.empty(bsz, *imgs.shape[2:], dtype=torch.uint8, device=dev) if return_labels else None
+        core.engine.eval_step(imgs, lbls, tally, group=group, ignore_index=IGNORE_INDEX, per_sample=rows, labels_out=labels,
+                              staged=staged)
+        return {"loss": self._tally_loss(tally), "tally": tally, "per_sample": rows, "labels": labels}
+
+    def _tally_loss(self, tally: LossTally) -> torch.Tensor:
+        """ce_plus_macro_dice_loss from its statistics: CE over the valid voxels + 0.5 * (1 - hard macro Dice)."""
+        return tally.loss()
+
+    @torch.no_grad()
+    def evaluate(self, batches, sample_group: Optional[int] = None):
+        """`eval_step` over an iterable of batches into one tally: the validation / test loss and metrics of the whole
+        set. Under torch.distributed every rank passes its own batches and gets the result of all of them. Returns
+        {"loss": float, "metrics": per_class_metrics_3d's 9-tuple, "tally", "voxels"}."""
+        return _evaluate(self, batches, lambda b, t: self.eval_step(b, tally=t, sample_group=sample_group))
+
+
+def _eval_voxels(batch) -> int:
+    """Voxels of a batch as given, before any padding: ignored voxels count as true negatives in
+    `metrics_from_confusion`, padding voxels must not."""
+    lbls = batch[1] if isinstance(batch, (list, tuple)) else batch["label"]
+    return int(_pick_first_if_seq(lbls).numel())
+
+
+def _evaluate(lit, batches, step):
+    """Shared driver of the `evaluate` methods: one tally over the batches, ONE all-reduce of the tally (plus the voxel
+    count) under data parallelism, ONE device->host copy at the end."""
+    tally, voxels = None, 0
+    dev = next(lit.parameters()).device
+    for batch in batches:
+        tally = step(batch, tally)["tally"]
+        voxels += _eval_voxels(batch)
+    if tally is None:   # a rank without batches still joins the all-reduce
+        tally = LossTally(lit.hparams.num_classes, dev)
+    vox = torch.tensor([voxels], dtype=torch.int64, device=tally._buf.device)
+    if dp.world()[1] > 1:
+        dp.allreduce_tally(tally.nll, tally.count, tally.confusion)
+        torch.distributed.all_reduce(vox)
+    loss = lit._tally_loss(tally).double().reshape(1)
+    # one copy: [nll (fp64 bits), count, confusion..., voxels, loss (fp64 bits)]
+    host = torch.cat([tally._buf, vox, loss.view(torch.int64)]).cpu()
+    k = tally.k
+    cm = host[2:2 + k * k].view(k, k).numpy()
+    voxels = int(host[2 + k * k])
+    return {"loss": float(host[-1:].view(torch.float64)[0]), "metrics": metrics_from_confusion(cm, voxels),
+            "tally": tally, "voxels": voxels}
+
 
 def _next_mult(n: int, m: int = 16) -> int:
     return ((n + m - 1) // m) * m
@@ -697,19 +779,35 @@ class _LitSPCT_Base(BaseLitModel):
         x_pad, orig = _pad_to_mult16_3d(x.float(), self._pad_multiple)
         return _center_crop_3d(self.model(x_pad), orig)
 
-    def fit_step(self, batch, optimize: bool = True, sample_group: Optional[int] = None):
+    def _padded_batch(self, batch):
+        """(x_pad, labels, orig): the images padded as `forward` pads them, the labels placed at the crop and
+        ignore_index outside it (voxels outside the crop carry no loss and no tally), orig (D,H,W) or None."""
         imgs, lbls = batch if isinstance(batch, (list, tuple)) else (batch["image"], batch["label"])
         imgs, lbls = _pick_first_if_seq(imgs), _pick_first_if_seq(lbls)
         if imgs.ndim == 4:
             imgs = imgs.unsqueeze(1)
         x_pad, orig = _pad_to_mult16_3d(imgs.float(), self._pad_multiple)
-        if orig is not None:   # voxels outside the crop carry no loss: label them ignore_index
+        if orig is not None:
             D, H, W = orig
             full = torch.full((lbls.shape[0],) + tuple(x_pad.shape[2:]), IGNORE_INDEX, dtype=torch.int64, device=lbls.device)
             sd, sh, sw = (x_pad.shape[2] - D) // 2, (x_pad.shape[3] - H) // 2, (x_pad.shape[4] - W) // 2
             full[:, sd:sd + D, sh:sh + H, sw:sw + W] = lbls
             lbls = full
+        return x_pad, lbls, orig
+
+    def fit_step(self, batch, optimize: bool = True, sample_group: Optional[int] = None):
+        x_pad, lbls, _ = self._padded_batch(batch)
         return super().fit_step((x_pad, lbls), optimize=optimize, sample_group=sample_group)
+
+    def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False,
+                  sample_group: Optional[int] = None):
+        """BaseLitModel.eval_step on the padded batch; the returned label map is cropped back to the input's size."""
+        x_pad, lbls, orig = self._padded_batch(batch)
+        out = super().eval_step((x_pad, lbls), tally=tally, per_sample=per_sample, return_labels=return_labels,
+                                sample_group=sample_group)
+        if out["labels"] is not None and orig is not None:
+            out["labels"] = _center_crop_to_3d(out["labels"].unsqueeze(1), orig)[:, 0].contiguous()
+        return out
 
 
 class LitSPCT_SEspec(_LitSPCT_Base):
@@ -1029,6 +1127,41 @@ class LitCicek3DUNet_DepthAdapter_Published(pl.LightningModule):
 
     def fused_grads(self) -> Dict[str, torch.Tensor]:
         return self._fused["G"]
+
+    # -- B200-native fused evaluation step --------------------------------------------------------
+    @torch.no_grad()
+    def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False):
+        """`_loss_and_log`'s loss and per_class_metrics_3d's statistics without the logits, BatchNorm in the module's
+        mode (as `forward` under no_grad; BatchNorm couples the samples, so the batch runs whole). Batch forms,
+        accumulation and return value as BaseLitModel.eval_step; the loss is ce_weight * CE over max(#valid, 1)."""
+        x, y, _ = self._unpack(batch)
+        x, y = _pick_first_if_seq(x), _pick_first_if_seq(y)
+        net = self.backbone
+        if x.ndim == 4:
+            x = x.unsqueeze(1)
+        net.materialize()
+        dev = net._flat.device
+        y = _canonicalize_targets_3d(y) if y.dtype not in (torch.uint8, torch.int64) or y.ndim != 4 else y
+        x = x.to(dev, non_blocking=True)
+        y = y.to(dev, non_blocking=True)
+        k = self.hparams.num_classes
+        tally = LossTally(k, dev) if tally is None else tally
+        bsz = x.shape[0]
+        rows = (torch.zeros(bsz, dtype=torch.float64, device=dev), torch.zeros(bsz, dtype=torch.int64, device=dev),
+                torch.zeros(bsz, k, k, dtype=torch.int64, device=dev)) if per_sample else None
+        labels = torch.empty(bsz, *x.shape[2:], dtype=torch.uint8, device=dev) if return_labels else None
+        ign = -1 if self.ignore_index is None else int(self.ignore_index)
+        net.engine.eval_step(x, y, tally, self.target_depth, ignore_index=ign, training=net.training, per_sample=rows,
+                             labels_out=labels)
+        return {"loss": self._tally_loss(tally), "tally": tally, "per_sample": rows, "labels": labels}
+
+    def _tally_loss(self, tally: LossTally) -> torch.Tensor:
+        return (self.ce_weight * tally.nll[0] / tally.count[0].clamp(min=1).double()).float()
+
+    @torch.no_grad()
+    def evaluate(self, batches):
+        """BaseLitModel.evaluate for this variant (loss: ce_weight * CE, no Dice term)."""
+        return _evaluate(self, batches, lambda b, t: self.eval_step(b, tally=t))
 
     def fused_optimizer_state(self) -> Dict[str, object]:
         """Momentum buffer + step count of the fused SGD, for checkpoint / resume (save next to `state_dict()`)."""

@@ -358,6 +358,26 @@ class CicekEngine:
                             tally.count, tally.confusion, gh, G["out.weight"].view(-1, self.base), G["out.bias"], 1.0)
         self.backward(B, G, x, gh)
 
+    def eval_step(self, x: torch.Tensor, labels: torch.Tensor, tally: LossTally, target_depth: Optional[int],
+                  ignore_index: int = 255, training: bool = False,
+                  per_sample: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None,
+                  labels_out: Optional[torch.Tensor] = None):
+        """Forward + head + CE/confusion over the whole batch, with no gradient and no logits in memory: the tally of
+        `infer(x, target_depth, training)` accumulates (+=) into `tally` (BatchNorm as `training` selects, like infer).
+        per_sample / labels_out as in SpffEngine.eval_step."""
+        x = self._check_input(x)
+        n, _, d0, h, w = x.shape
+        if labels.shape != (n, d0, h, w):
+            raise ValueError(f"labels must be [B,D,H,W] = {(n, d0, h, w)}, got {tuple(labels.shape)}")
+        labels = labels.contiguous()
+        self.refresh_weights()
+        B = self.buffers(n, d0, target_depth or d0, h, w, x.device, train=False)
+        hx = self.forward(B, x, training)
+        p = self._params()
+        rows = per_sample if per_sample is not None else (None, None, None)
+        ops.head_eval(hx, p["out.weight"], p["out.bias"], labels, ignore_index, tally.nll, tally.count, tally.confusion,
+                      *rows, labels_out)
+
 
 def flat_names(named_params: List[Tuple[str, torch.Tensor]]):
     """16-byte aligned slots of a flat fp32 buffer holding the given parameters in order: name -> (offset, numel, shape)."""

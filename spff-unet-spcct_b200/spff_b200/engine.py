@@ -647,6 +647,33 @@ class SpffEngine:
             self.backward_group(B, T, G, None, stage_done=hook)
         T.finish(G)
 
+    def eval_step(self, x: torch.Tensor, labels: torch.Tensor, tally: "LossTally", group: int = 32,
+                  ignore_index: int = 255, per_sample: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None,
+                  labels_out: Optional[torch.Tensor] = None, staged: Optional["StagedBatch"] = None):
+        """Forward + head + CE/confusion over the batch in sample groups, with no gradient: the loss statistics of
+        `ce_plus_macro_dice_loss` / `per_class_metrics_3d` on `infer(x)` accumulate (+=) into `tally`, and the fp32 logits
+        never reach memory. per_sample = (nll fp64 [B], count int64 [B], confusion int64 [B,K,K]) receives the same
+        tally per sample (+=); labels_out (uint8 [B,F,H,W]) the arg-max the tally counts. `staged`: as in train_step."""
+        x = self._check_input(x)
+        bsz, _, d, h, w = x.shape
+        if labels.shape != (bsz, d, h, w):
+            raise ValueError(f"labels must be [B,F,H,W] = {(bsz, d, h, w)}, got {tuple(labels.shape)}")
+        labels = labels.contiguous()
+        self.refresh_weights()
+        group = self._fitted(min(group, bsz), d, h, w, x.device, train=False)
+        T = GateTables(self.cfg, self.params(), d, need_grad=False)
+        p = self.params()
+        for lo, hi in self._groups(bsz, group):
+            if staged is not None:
+                staged.wait_images(hi)
+            B = self.buffers(hi - lo, d, h, w, x.device, train=False)
+            self.forward_group(B, T, x[lo:hi], head="none")
+            if staged is not None:
+                staged.wait_labels(hi)
+            rows = tuple(t[lo:hi] for t in per_sample) if per_sample is not None else (None, None, None)
+            ops.head_eval(B.out["dec1"], p["out.weight"], p["out.bias"], labels[lo:hi], ignore_index, tally.nll,
+                          tally.count, tally.confusion, *rows, labels_out[lo:hi] if labels_out is not None else None)
+
 
 class StagedBatch:
     """Host -> device staging of one batch on a dedicated copy stream, group by group: the images of a group, then its

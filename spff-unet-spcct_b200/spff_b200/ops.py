@@ -361,6 +361,26 @@ def head_loss_fused(x, w, b, labels, ignore_index, n_valid, gscale, acc, counts,
          ptr(ws), ws.numel(), stream_ptr())
 
 
+def head_eval(x, w, b, labels, ignore_index, acc, counts, confusion, sample_acc=None, sample_counts=None,
+              sample_confusion=None, labels_out=None):
+    """Fused evaluation head (no logits in memory): the loss statistics of head_fwd + ce_confusion += into acc /
+    counts / confusion; optionally per sample (fp64 [n], int64 [n], int64 [n,K,K], +=) and the uint8 arg-max map
+    [n,d,h,w] the tally counts."""
+    k = w.shape[0]
+    s, ldx = _view(x, 32)
+    assert labels.is_contiguous() and labels.numel() == s.n * s.d * s.h * s.w
+    per = (sample_acc, sample_counts, sample_confusion)
+    if any(t is not None for t in per):
+        assert sample_acc.dtype == torch.float64 and sample_acc.numel() == s.n
+        assert sample_counts.dtype == torch.int64 and sample_counts.numel() == s.n
+        assert sample_confusion.dtype == torch.int64 and sample_confusion.is_contiguous()
+        assert sample_confusion.numel() == s.n * k * k
+    if labels_out is not None:
+        assert labels_out.dtype == torch.uint8 and labels_out.is_contiguous() and labels_out.numel() == s.n * s.d * s.h * s.w
+    call("spff_head_eval", ptr(x), ldx, 32, ptr(w), ptr(b), ptr(labels), _label_bytes(labels), int(ignore_index), k, s,
+         ptr(acc), ptr(counts), ptr(confusion), *(ptr(t) for t in per), ptr(labels_out), stream_ptr())
+
+
 def scale_by_count(g, count, factor: float = 1.0):
     """g (fp32, contiguous) *= factor / count[0]  (0 when the count is 0)."""
     assert g.dtype == torch.float32 and g.is_contiguous() and count.dtype == torch.int64
