@@ -253,6 +253,15 @@ int spff_head_eval(const void* x, long long ldx, int cin, const float* w, const 
                    int label_bytes, int ignore_index, int k, spff_shape s, double* acc, long long* counts,
                    long long* confusion, double* sample_acc, long long* sample_counts, long long* sample_confusion,
                    uint8_t* labels_out, void* stream);
+/* spff_head_eval plus the ranking statistics of the softmax: for every counted voxel (label in [0,K), not
+ * ignore_index) and every class c, p_c = e_c / sum(e) (fp32, IEEE division) falls in bin min(floor(p_c * bins),
+ * bins - 1); hist int64 [K][2][bins] receives (+=) the positives (label == c) in [c][0] and the negatives in [c][1],
+ * sample_hist [N][K][2][bins] the same per sample. bins in [16, 1024]; hist required; sample_hist is given exactly
+ * when the per-sample tallies are. Every other argument and output is that of spff_head_eval. */
+int spff_head_eval_hist(const void* x, long long ldx, int cin, const float* w, const float* b, const void* labels,
+                        int label_bytes, int ignore_index, int k, spff_shape s, double* acc, long long* counts,
+                        long long* confusion, double* sample_acc, long long* sample_counts, long long* sample_confusion,
+                        uint8_t* labels_out, int bins, long long* hist, long long* sample_hist, void* stream);
 
 /* ---- "3DUNet" control: Cicek3DUNet + depth adapter (models.py:718-777; config.py:283-311) ---------------
  * Its 3x3x3 convolutions, normalise + ReLU passes (slope 0), head and loss are the entry points above;

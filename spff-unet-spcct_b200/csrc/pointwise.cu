@@ -1319,23 +1319,36 @@ head_loss_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
 // only, so a block's tally belongs to one sample: it is kept in shared memory and flushed once per block to
 // the batch arrays and, when given, to the sample's row of the per-sample arrays. Optionally the arg-max map
 // (the one the tally counts) is written. Traffic: the 64 B of x + the label per voxel (+ 1 B of arg-max).
+//
+// HIST adds the ranking statistics: for every counted voxel (label in [0, K), not ignore_index) and every class c,
+// p_c = e_c / se (IEEE division) falls in bin min(floor(p_c * T), T - 1) of hist[c][label == c ? 0 : 1][T], a
+// sufficient statistic of the ROC and PR curves at the thresholds i / T. The block-private histogram is uint32
+// [K][2][T] in dynamic shared memory. The two bins almost every voxel lands in once the model is trained (a negative
+// in bin 0, a positive in bin T - 1) are counted in registers per lane and added at the flush, so that they do not
+// serialise the block on two shared addresses.
 // ---------------------------------------------------------------------------------------------
 constexpr int kHeBlocksPerSm = 3;
+constexpr int kHeMinBins = 16, kHeMaxBins = 1024;
 
-template <typename LabelT>
+template <typename LabelT, bool HIST>
 __global__ void __launch_bounds__(kHmWarps * 32, kHeBlocksPerSm)
 head_eval_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const void* __restrict__ labels, int ignore_index,
                      int K, long long dhw, double* __restrict__ acc, unsigned long long* __restrict__ counts,
                      unsigned long long* __restrict__ confusion, double* __restrict__ sample_acc,
                      unsigned long long* __restrict__ sample_counts, unsigned long long* __restrict__ sample_confusion,
-                     uint8_t* __restrict__ labels_out) {
+                     uint8_t* __restrict__ labels_out, int T, unsigned long long* __restrict__ hist,
+                     unsigned long long* __restrict__ sample_hist) {
   __shared__ __align__(16) __nv_bfloat16 xs[kHmWarps][16][kHmXPitch];
   __shared__ unsigned int s_conf[kMaxK * kMaxK];
   __shared__ float s_nll[kHmWarps];
   __shared__ unsigned int s_cnt[kHmWarps];
+  extern __shared__ unsigned int s_hist[];   // HIST: [K][2][T]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int g = lane >> 2, t = lane & 3;
   for (int i = threadIdx.x; i < K * K; i += blockDim.x) s_conf[i] = 0;
+  if constexpr (HIST)
+    for (int i = threadIdx.x; i < K * 2 * T; i += blockDim.x) s_hist[i] = 0;
+  unsigned int hot_neg[4] = {0, 0, 0, 0}, hot_pos[4] = {0, 0, 0, 0};   // HIST: bin 0 of negatives, bin T - 1 of positives
   __syncthreads();
   HmLogitW wl;
   hm_logit_weights(K, g, t, wl);
@@ -1376,6 +1389,23 @@ head_eval_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
           if (lab >= 0 && lab < K) atomicAdd(&s_conf[lab * K + arg], 1u);
         }
       }
+      if constexpr (HIST) {   // all four lanes of the quad: classes cls[0..3] of this row
+        if (inb && lab != ignore_index && lab >= 0 && lab < K) {
+#pragma unroll
+          for (int q = 0; q < 4; ++q)
+            if (cls[q] < K) {
+              const float p = __fdiv_rn(e[q], se);
+              const int bin = min(static_cast<int>(__fmul_rn(p, static_cast<float>(T))), T - 1);
+              const bool positive = cls[q] == lab;
+              if (positive && bin == T - 1)
+                ++hot_pos[q];
+              else if (!positive && bin == 0)
+                ++hot_neg[q];
+              else
+                atomicAdd(&s_hist[(cls[q] * 2 + (positive ? 0 : 1)) * T + bin], 1u);
+            }
+        }
+      }
     }
     __syncwarp();   // the tile is read before the next iteration overwrites it
   }
@@ -1386,6 +1416,21 @@ head_eval_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
   if (lane == 0) {
     s_nll[warp] = nll_sum;
     s_cnt[warp] = cnt;
+  }
+  if constexpr (HIST) {   // the register bins: sum over the 8 lanes holding the same classes, then one add per warp
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+#pragma unroll
+      for (int o = 4; o < 32; o <<= 1) {
+        hot_pos[q] += __shfl_xor_sync(0xffffffffu, hot_pos[q], o);
+        hot_neg[q] += __shfl_xor_sync(0xffffffffu, hot_neg[q], o);
+      }
+      const int c = 8 * (q >> 1) + 2 * t + (q & 1);
+      if (g == 0 && c < K) {
+        if (hot_pos[q]) atomicAdd(&s_hist[(c * 2 + 0) * T + T - 1], hot_pos[q]);
+        if (hot_neg[q]) atomicAdd(&s_hist[(c * 2 + 1) * T + 0], hot_neg[q]);
+      }
+    }
   }
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -1407,6 +1452,12 @@ head_eval_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
       atomicAdd(confusion + i, static_cast<unsigned long long>(s_conf[i]));
       if (sample_confusion) atomicAdd(sample_confusion + n * K * K + i, static_cast<unsigned long long>(s_conf[i]));
     }
+  if constexpr (HIST)
+    for (int i = threadIdx.x; i < K * 2 * T; i += blockDim.x)
+      if (s_hist[i]) {
+        atomicAdd(hist + i, static_cast<unsigned long long>(s_hist[i]));
+        if (sample_hist) atomicAdd(sample_hist + n * K * 2 * T + i, static_cast<unsigned long long>(s_hist[i]));
+      }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1458,6 +1509,76 @@ constexpr int kHeadBwdBlocksPerSm = 2;
   } while (0)
 
 typedef __nv_bfloat16 bf16;
+
+namespace {
+
+template <typename LabelT>
+int head_eval_hist_attr() {   // once per device: the [K][2][T] histogram may exceed the 48 KB default (128 KB at most)
+  static bool attr_set[spff::kMaxDevices] = {};
+  const int dev = spff::current_device();
+  if (!attr_set[dev]) {
+    SPFF_CUDA(cudaFuncSetAttribute(spff::head_eval_mma_kernel<LabelT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   static_cast<int>(sizeof(unsigned int) * spff::kMaxK * 2 * spff::kHeMaxBins)));
+    attr_set[dev] = true;
+  }
+  return 0;
+}
+
+// spff_head_eval and spff_head_eval_hist: bins = 0 and hist = NULL select the kernel without the histogram
+int head_eval_launch(const char* name, const void* x, long long ldx, int cin, const float* w, const float* b,
+                     const void* labels, int label_bytes, int ignore_index, int k, spff_shape s, double* acc,
+                     long long* counts, long long* confusion, double* sample_acc, long long* sample_counts,
+                     long long* sample_confusion, uint8_t* labels_out, int bins, long long* hist, long long* sample_hist,
+                     void* stream) {
+  SPFF_REQUIRE(x && w && b && labels && acc && counts && confusion, "%s: null pointer", name);
+  SPFF_REQUIRE((sample_acc != nullptr) == (sample_counts != nullptr) && (sample_acc != nullptr) == (sample_confusion != nullptr),
+               "%s: the per-sample arrays are given together or not at all", name);
+  SPFF_REQUIRE(label_bytes == 1 || label_bytes == 8, "%s: labels must be uint8 or int64", name);
+  SPFF_REQUIRE(ldx >= cin && ldx % 8 == 0, "%s: bad channel pitch", name);
+  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "%s: bad shape", name);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int e = spff::upload_head(w, b, k, cin, st);
+  if (e) return e;
+  const long long dhw = static_cast<long long>(s.d) * s.h * s.w;
+  // blocks never straddle samples (grid.y = sample); grid.x spreads a sample over enough blocks for ~4 waves of
+  // kHeBlocksPerSm resident blocks per SM, and no more blocks than the sample has warp tiles for
+  const long long warp_tiles = ((dhw + 15) / 16 + spff::kHmWarps - 1) / spff::kHmWarps;
+  long long per = (4LL * spff::kHeBlocksPerSm * spff::num_sms() + s.n - 1) / s.n;
+  if (per > warp_tiles) per = warp_tiles;
+  if (per < 1) per = 1;
+  const dim3 grid(static_cast<unsigned>(per), s.n);
+  auto cnt = reinterpret_cast<unsigned long long*>(counts);
+  auto conf = reinterpret_cast<unsigned long long*>(confusion);
+  auto scnt = reinterpret_cast<unsigned long long*>(sample_counts);
+  auto sconf = reinterpret_cast<unsigned long long*>(sample_confusion);
+  auto hst = reinterpret_cast<unsigned long long*>(hist);
+  auto shst = reinterpret_cast<unsigned long long*>(sample_hist);
+  const size_t hist_smem = sizeof(unsigned int) * k * 2 * bins;
+  if (hist) {
+    e = label_bytes == 1 ? head_eval_hist_attr<uint8_t>() : head_eval_hist_attr<long long>();
+    if (e) return e;
+  }
+  if (label_bytes == 1 && !hist)
+    spff::head_eval_mma_kernel<uint8_t, false><<<grid, spff::kHmWarps * 32, 0, st>>>(
+        static_cast<const bf16*>(x), ldx, labels, ignore_index, k, dhw, acc, cnt, conf, sample_acc, scnt, sconf, labels_out,
+        0, nullptr, nullptr);
+  else if (!hist)
+    spff::head_eval_mma_kernel<long long, false><<<grid, spff::kHmWarps * 32, 0, st>>>(
+        static_cast<const bf16*>(x), ldx, labels, ignore_index, k, dhw, acc, cnt, conf, sample_acc, scnt, sconf, labels_out,
+        0, nullptr, nullptr);
+  else if (label_bytes == 1)
+    spff::head_eval_mma_kernel<uint8_t, true><<<grid, spff::kHmWarps * 32, hist_smem, st>>>(
+        static_cast<const bf16*>(x), ldx, labels, ignore_index, k, dhw, acc, cnt, conf, sample_acc, scnt, sconf, labels_out,
+        bins, hst, shst);
+  else
+    spff::head_eval_mma_kernel<long long, true><<<grid, spff::kHmWarps * 32, hist_smem, st>>>(
+        static_cast<const bf16*>(x), ldx, labels, ignore_index, k, dhw, acc, cnt, conf, sample_acc, scnt, sconf, labels_out,
+        bins, hst, shst);
+  SPFF_CUDA(cudaGetLastError());
+  return 0;
+}
+
+}  // namespace
 
 extern "C" {
 
@@ -1689,35 +1810,23 @@ int spff_head_eval(const void* x, long long ldx, int cin, const float* w, const 
                    long long* confusion, double* sample_acc, long long* sample_counts, long long* sample_confusion,
                    uint8_t* labels_out, void* stream) {
   SPFF_ENTRY_CHECK();
-  SPFF_REQUIRE(x && w && b && labels && acc && counts && confusion, "head_eval: null pointer");
-  SPFF_REQUIRE((sample_acc != nullptr) == (sample_counts != nullptr) && (sample_acc != nullptr) == (sample_confusion != nullptr),
-               "head_eval: the per-sample arrays are given together or not at all");
-  SPFF_REQUIRE(label_bytes == 1 || label_bytes == 8, "head_eval: labels must be uint8 or int64");
-  SPFF_REQUIRE(ldx >= cin && ldx % 8 == 0, "head_eval: bad channel pitch");
-  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "head_eval: bad shape");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int e = spff::upload_head(w, b, k, cin, st);
-  if (e) return e;
-  const long long dhw = static_cast<long long>(s.d) * s.h * s.w;
-  // blocks never straddle samples (grid.y = sample); grid.x spreads a sample over enough blocks for ~4 waves of
-  // kHeBlocksPerSm resident blocks per SM, and no more blocks than the sample has warp tiles for
-  const long long warp_tiles = ((dhw + 15) / 16 + spff::kHmWarps - 1) / spff::kHmWarps;
-  long long per = (4LL * spff::kHeBlocksPerSm * spff::num_sms() + s.n - 1) / s.n;
-  if (per > warp_tiles) per = warp_tiles;
-  if (per < 1) per = 1;
-  const dim3 grid(static_cast<unsigned>(per), s.n);
-  auto cnt = reinterpret_cast<unsigned long long*>(counts);
-  auto conf = reinterpret_cast<unsigned long long*>(confusion);
-  auto scnt = reinterpret_cast<unsigned long long*>(sample_counts);
-  auto sconf = reinterpret_cast<unsigned long long*>(sample_confusion);
-  if (label_bytes == 1)
-    spff::head_eval_mma_kernel<uint8_t><<<grid, spff::kHmWarps * 32, 0, st>>>(
-        static_cast<const bf16*>(x), ldx, labels, ignore_index, k, dhw, acc, cnt, conf, sample_acc, scnt, sconf, labels_out);
-  else
-    spff::head_eval_mma_kernel<long long><<<grid, spff::kHmWarps * 32, 0, st>>>(
-        static_cast<const bf16*>(x), ldx, labels, ignore_index, k, dhw, acc, cnt, conf, sample_acc, scnt, sconf, labels_out);
-  SPFF_CUDA(cudaGetLastError());
-  return 0;
+  return head_eval_launch("head_eval", x, ldx, cin, w, b, labels, label_bytes, ignore_index, k, s, acc, counts, confusion,
+                          sample_acc, sample_counts, sample_confusion, labels_out, 0, nullptr, nullptr, stream);
+}
+
+int spff_head_eval_hist(const void* x, long long ldx, int cin, const float* w, const float* b, const void* labels,
+                        int label_bytes, int ignore_index, int k, spff_shape s, double* acc, long long* counts,
+                        long long* confusion, double* sample_acc, long long* sample_counts, long long* sample_confusion,
+                        uint8_t* labels_out, int bins, long long* hist, long long* sample_hist, void* stream) {
+  SPFF_ENTRY_CHECK();
+  SPFF_REQUIRE(bins >= spff::kHeMinBins && bins <= spff::kHeMaxBins, "head_eval_hist: bins must be in [%d, %d] (got %d)",
+               spff::kHeMinBins, spff::kHeMaxBins, bins);
+  SPFF_REQUIRE(hist, "head_eval_hist: null histogram");
+  SPFF_REQUIRE((sample_hist != nullptr) == (sample_acc != nullptr),
+               "head_eval_hist: the per-sample histogram is given exactly when the per-sample tallies are");
+  return head_eval_launch("head_eval_hist", x, ldx, cin, w, b, labels, label_bytes, ignore_index, k, s, acc, counts,
+                          confusion, sample_acc, sample_counts, sample_confusion, labels_out, bins, hist, sample_hist,
+                          stream);
 }
 
 int spff_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr,

@@ -182,6 +182,87 @@ def sample_metrics(per_sample, voxels_per_sample: int, smooth: float = 1e-6) -> 
     return [metrics_from_confusion(row, voxels_per_sample, smooth) for row in cm]
 
 
+def _nanmean_fg(v) -> float:
+    """per_class_metrics_3d's macro convention: the nanmean over classes 1..K-1 (NaN when none is defined)."""
+    vals = [float(x) for x in list(v)[1:] if not math.isnan(float(x))]
+    return float(np.mean(vals)) if vals else float("nan")
+
+
+def _ranking(hist: np.ndarray):
+    """(auroc [K], ap [K], auroc_tie_bound [K], tp [K,T+1], fp [K,T+1]) of one [K,2,T] histogram.
+    tp[:, i] / fp[:, i] count the positives / negatives in bins >= i (threshold i / T); column T is 0."""
+    h = np.asarray(hist, dtype=np.float64)
+    pos, neg = h[:, 0], h[:, 1]
+    k, bins = pos.shape
+    zero = np.zeros((k, 1))
+    tp = np.concatenate([np.cumsum(pos[:, ::-1], axis=1)[:, ::-1], zero], axis=1)
+    fp = np.concatenate([np.cumsum(neg[:, ::-1], axis=1)[:, ::-1], zero], axis=1)
+    P, N = tp[:, 0], fp[:, 0]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        # trapezoids between the ROC points of thresholds i + 1 and i: width neg_i / N, mean height (tp_{i+1} + pos_i / 2) / P
+        auroc = (neg * (tp[:, 1:] + 0.5 * pos)).sum(1) / (P * N)
+        # sklearn's step AP: recall steps pos_i / P at precision tp_i / (tp_i + fp_i); empty steps add nothing
+        prec = np.where(pos > 0, tp[:, :bins] / np.maximum(tp[:, :bins] + fp[:, :bins], 1), 0.0)
+        ap = (pos * prec).sum(1) / P
+        bound = 0.5 * (pos * neg).sum(1) / (P * N)
+    undefined = (P == 0) | (N == 0)
+    auroc[undefined] = np.nan
+    bound[undefined] = np.nan
+    ap[P == 0] = np.nan
+    return auroc, ap, bound, tp, fp
+
+
+def _as_numpy(t) -> np.ndarray:
+    return t.detach().cpu().numpy() if torch.is_tensor(t) else np.asarray(t)
+
+
+def curves_from_hist(hist) -> dict:
+    """Per-class ROC and precision-recall curves from the softmax histogram of `eval_step(curves=T)` / `evaluate`
+    (int64 [K,2,T]: hist[c,0,b] positives and hist[c,1,b] negatives of class c whose probability falls in bin b).
+
+    Thresholds are t_i = i / T, i = 0..T; TP_i / FP_i count the positives / negatives in bins >= i. Per class c:
+    ROC points (FP_i / N_c, TP_i / P_c) in order of falling threshold (`roc_thresholds` = t_T..t_0), PR points
+    (recall TP_i / P_c, precision TP_i / (TP_i + FP_i)) for the i with TP_i + FP_i > 0 in order of rising threshold
+    (`pr_thresholds`). `auroc` is the trapezoid area under the ROC points (NaN when P_c or N_c is 0), `ap` sklearn's
+    step average precision sum_i (R_i - R_{i+1}) * Prec_i (NaN when P_c is 0): both equal sklearn's roc_auc_score /
+    average_precision_score with the bin index as the score. Binning makes every positive-negative pair inside one
+    bin a tie worth 1/2, so the unbinned AUROC differs by at most `auroc_tie_bound` = 1/2 sum_b pos_b * neg_b /
+    (P_c * N_c). `macro_auroc` / `macro_ap` are the nanmeans over classes 1..K-1, as in per_class_metrics_3d."""
+    h = _as_numpy(hist)
+    if h.ndim != 3 or h.shape[1] != 2:
+        raise ValueError(f"expected a [K,2,T] histogram, got {h.shape}")
+    auroc, ap, bound, tp, fp = _ranking(h)
+    k, bins = h.shape[0], h.shape[2]
+    thr = np.arange(bins + 1, dtype=np.float64) / bins
+    out = {k_: [] for k_ in ("fpr", "tpr", "roc_thresholds", "precision", "recall", "pr_thresholds")}
+    for c in range(k):
+        P, N = tp[c, 0], fp[c, 0]
+        with np.errstate(invalid="ignore", divide="ignore"):
+            out["fpr"].append(fp[c, ::-1] / N)
+            out["tpr"].append(tp[c, ::-1] / P)
+            out["roc_thresholds"].append(thr[::-1].copy())
+            keep = (tp[c] + fp[c]) > 0
+            out["precision"].append(tp[c][keep] / (tp[c][keep] + fp[c][keep]))
+            out["recall"].append(tp[c][keep] / P)
+            out["pr_thresholds"].append(thr[keep])
+    out.update(auroc=auroc, ap=ap, auroc_tie_bound=bound, macro_auroc=_nanmean_fg(auroc), macro_ap=_nanmean_fg(ap))
+    return out
+
+
+def sample_curves(per_sample_hist) -> List[tuple]:
+    """Per-case ranking metrics: one (auroc [K], ap [K], macro_auroc, macro_ap) per sample from the per-sample
+    histograms of `eval_step(curves=T, per_sample=True)` ([B,K,2,T]), as curves_from_hist defines them. The ranking
+    counterpart of `sample_metrics`."""
+    h = _as_numpy(per_sample_hist)
+    if h.ndim != 4 or h.shape[2] != 2:
+        raise ValueError(f"expected a [B,K,2,T] histogram, got {h.shape}")
+    out = []
+    for row in h:
+        auroc, ap, _, _, _ = _ranking(row)
+        out.append((auroc, ap, _nanmean_fg(auroc), _nanmean_fg(ap)))
+    return out
+
+
 def per_class_metrics_2d(preds, labels, num_classes, smooth=1e-6, ignore_index=None):
     """2-D twin (helpers.py:728-779): same counting rules on [B,K,H,W] logits."""
     return per_class_metrics_3d(preds, labels, num_classes, smooth, ignore_index)

@@ -36,8 +36,8 @@ from spff_b200.engine import LossTally, NetConfig, SpffEngine, StagedBatch
 from spff_b200.sched import PlateauLR
 
 from .config import BEST_LR, IGNORE_INDEX, NUM_CLASSES, NUM_FRAMES
-from .helpers import (LOSS_REGISTRY, ce_plus_macro_dice_loss, metrics_from_confusion, per_class_metrics_2d,
-                      per_class_metrics_3d)
+from .helpers import (LOSS_REGISTRY, ce_plus_macro_dice_loss, curves_from_hist, metrics_from_confusion,
+                      per_class_metrics_2d, per_class_metrics_3d)
 
 LOG_PER_CLASS = os.getenv("LOG_PER_CLASS", "1") == "1"
 # samples per group of the engine's schedule (activations of one group live at a time in fit_step)
@@ -654,14 +654,19 @@ class BaseLitModel(pl.LightningModule):
     # -- B200-native fused evaluation step --------------------------------------------------------
     @torch.no_grad()
     def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False,
-                  sample_group: Optional[int] = None):
+                  sample_group: Optional[int] = None, curves=None):
         """The loss statistics of `ce_plus_macro_dice_loss(model(x), y)` and `per_class_metrics_3d` without the logits:
         forward, head, CE and confusion tally in the engine's sample-group schedule. Takes the batch forms `fit_step`
         takes (tuple or dict; host or device; uint8 or int64 labels) and accumulates into `tally` (a fresh LossTally when
         None). Touches no parameter, gradient or optimizer state and does not synchronise the host.
 
+        `curves`: None, a bin count T in [16, 1024], or an int64 [K,2,T] histogram to accumulate into (as `tally`): the
+        head also bins every class's softmax probability of the counted voxels, positives and negatives apart, which is
+        what `helpers.curves_from_hist` turns into ROC / PR curves, AUROC and AP.
+
         Returns {"loss": device scalar of the tally so far, "tally", "per_sample": (nll fp64 [B], count int64 [B],
-        confusion int64 [B,K,K]) or None, "labels": uint8 arg-max map [B,F,H,W] or None}."""
+        confusion int64 [B,K,K]) or None, "labels": uint8 arg-max map [B,F,H,W] or None, "hist": int64 [K,2,T] or None,
+        "per_sample_hist": int64 [B,K,2,T] with curves and per_sample, else None}."""
         imgs, lbls = batch if isinstance(batch, (list, tuple)) else (batch["image"], batch["label"])
         imgs, lbls = _pick_first_if_seq(imgs), _pick_first_if_seq(lbls)
         core: UNet3D_SpectralCore = self.model
@@ -687,20 +692,25 @@ class BaseLitModel(pl.LightningModule):
         rows = (torch.zeros(bsz, dtype=torch.float64, device=dev), torch.zeros(bsz, dtype=torch.int64, device=dev),
                 torch.zeros(bsz, k, k, dtype=torch.int64, device=dev)) if per_sample else None
         labels = torch.empty(bsz, *imgs.shape[2:], dtype=torch.uint8, device=dev) if return_labels else None
+        hist, sample_hist = _curve_buffers(curves, k, bsz, per_sample, dev)
         core.engine.eval_step(imgs, lbls, tally, group=group, ignore_index=IGNORE_INDEX, per_sample=rows, labels_out=labels,
-                              staged=staged)
-        return {"loss": self._tally_loss(tally), "tally": tally, "per_sample": rows, "labels": labels}
+                              staged=staged, hist=hist, sample_hist=sample_hist)
+        return {"loss": self._tally_loss(tally), "tally": tally, "per_sample": rows, "labels": labels, "hist": hist,
+                "per_sample_hist": sample_hist}
 
     def _tally_loss(self, tally: LossTally) -> torch.Tensor:
         """ce_plus_macro_dice_loss from its statistics: CE over the valid voxels + 0.5 * (1 - hard macro Dice)."""
         return tally.loss()
 
     @torch.no_grad()
-    def evaluate(self, batches, sample_group: Optional[int] = None):
+    def evaluate(self, batches, sample_group: Optional[int] = None, curves: Optional[int] = None):
         """`eval_step` over an iterable of batches into one tally: the validation / test loss and metrics of the whole
         set. Under torch.distributed every rank passes its own batches and gets the result of all of them. Returns
-        {"loss": float, "metrics": per_class_metrics_3d's 9-tuple, "tally", "voxels"}."""
-        return _evaluate(self, batches, lambda b, t: self.eval_step(b, tally=t, sample_group=sample_group))
+        {"loss": float, "metrics": per_class_metrics_3d's 9-tuple, "tally", "voxels"}; with `curves` = T bins also
+        "hist" (int64 [K,2,T] on the device) and "curves" (`helpers.curves_from_hist`: per-class ROC / PR curves, AUROC,
+        AP and their macro averages)."""
+        return _evaluate(self, batches, lambda b, t, h: self.eval_step(b, tally=t, sample_group=sample_group, curves=h),
+                         curves)
 
 
 def _eval_voxels(batch) -> int:
@@ -710,28 +720,57 @@ def _eval_voxels(batch) -> int:
     return int(_pick_first_if_seq(lbls).numel())
 
 
-def _evaluate(lit, batches, step):
-    """Shared driver of the `evaluate` methods: one tally over the batches, ONE all-reduce of the tally (plus the voxel
-    count) under data parallelism, ONE device->host copy at the end."""
+def _curve_buffers(curves, k: int, bsz: int, per_sample: bool, dev):
+    """(hist [K,2,T], per-sample hist [B,K,2,T] or None) for `eval_step(curves=...)`; (None, None) without curves.
+    `curves` is a bin count T (fresh zeros) or a [K,2,T] int64 histogram on `dev` to accumulate into."""
+    if curves is None:
+        return None, None
+    if torch.is_tensor(curves):
+        hist = curves
+        if hist.dtype != torch.int64 or hist.dim() != 3 or tuple(hist.shape[:2]) != (k, 2) or not hist.is_contiguous() \
+                or hist.device != torch.device(dev):
+            raise ValueError(f"curves must be a contiguous int64 [{k},2,T] histogram on {dev}, got {hist.dtype} "
+                             f"{tuple(hist.shape)} on {hist.device}")
+    else:
+        hist = torch.zeros(k, 2, int(curves), dtype=torch.int64, device=dev)
+    bins = hist.shape[-1]
+    if not 16 <= bins <= 1024:
+        raise ValueError(f"curves: the bin count must be in [16, 1024], got {bins}")
+    sample_hist = torch.zeros(bsz, k, 2, bins, dtype=torch.int64, device=dev) if per_sample else None
+    return hist, sample_hist
+
+
+def _evaluate(lit, batches, step, curves: Optional[int] = None):
+    """Shared driver of the `evaluate` methods: one tally (and, with `curves` = T, one [K,2,T] softmax histogram) over
+    the batches, ONE all-reduce of the tally (plus the voxel count and the histogram) under data parallelism, ONE
+    device->host copy at the end."""
     tally, voxels = None, 0
     dev = next(lit.parameters()).device
+    k = lit.hparams.num_classes
+    hist = _curve_buffers(curves, k, 0, False, dev)[0]
     for batch in batches:
-        tally = step(batch, tally)["tally"]
+        tally = step(batch, tally, hist)["tally"]
         voxels += _eval_voxels(batch)
     if tally is None:   # a rank without batches still joins the all-reduce
-        tally = LossTally(lit.hparams.num_classes, dev)
+        tally = LossTally(k, dev)
     vox = torch.tensor([voxels], dtype=torch.int64, device=tally._buf.device)
     if dp.world()[1] > 1:
         dp.allreduce_tally(tally.nll, tally.count, tally.confusion)
         torch.distributed.all_reduce(vox)
+        if hist is not None:
+            dp.allreduce_hist(hist)
     loss = lit._tally_loss(tally).double().reshape(1)
-    # one copy: [nll (fp64 bits), count, confusion..., voxels, loss (fp64 bits)]
-    host = torch.cat([tally._buf, vox, loss.view(torch.int64)]).cpu()
-    k = tally.k
+    # one copy: [nll (fp64 bits), count, confusion..., voxels, loss (fp64 bits), histogram...]
+    parts = [tally._buf, vox, loss.view(torch.int64)] + ([hist.view(-1)] if hist is not None else [])
+    host = torch.cat(parts).cpu()
     cm = host[2:2 + k * k].view(k, k).numpy()
     voxels = int(host[2 + k * k])
-    return {"loss": float(host[-1:].view(torch.float64)[0]), "metrics": metrics_from_confusion(cm, voxels),
-            "tally": tally, "voxels": voxels}
+    out = {"loss": float(host[3 + k * k:4 + k * k].view(torch.float64)[0]), "metrics": metrics_from_confusion(cm, voxels),
+           "tally": tally, "voxels": voxels}
+    if hist is not None:
+        out["hist"] = hist
+        out["curves"] = curves_from_hist(host[4 + k * k:].view(hist.shape).numpy())
+    return out
 
 
 def _next_mult(n: int, m: int = 16) -> int:
@@ -800,11 +839,12 @@ class _LitSPCT_Base(BaseLitModel):
         return super().fit_step((x_pad, lbls), optimize=optimize, sample_group=sample_group)
 
     def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False,
-                  sample_group: Optional[int] = None):
-        """BaseLitModel.eval_step on the padded batch; the returned label map is cropped back to the input's size."""
+                  sample_group: Optional[int] = None, curves=None):
+        """BaseLitModel.eval_step on the padded batch; the returned label map is cropped back to the input's size. The
+        padding carries ignore_index, so the histograms count the input's voxels only."""
         x_pad, lbls, orig = self._padded_batch(batch)
         out = super().eval_step((x_pad, lbls), tally=tally, per_sample=per_sample, return_labels=return_labels,
-                                sample_group=sample_group)
+                                sample_group=sample_group, curves=curves)
         if out["labels"] is not None and orig is not None:
             out["labels"] = _center_crop_to_3d(out["labels"].unsqueeze(1), orig)[:, 0].contiguous()
         return out
@@ -1130,10 +1170,12 @@ class LitCicek3DUNet_DepthAdapter_Published(pl.LightningModule):
 
     # -- B200-native fused evaluation step --------------------------------------------------------
     @torch.no_grad()
-    def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False):
+    def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False,
+                  curves=None):
         """`_loss_and_log`'s loss and per_class_metrics_3d's statistics without the logits, BatchNorm in the module's
         mode (as `forward` under no_grad; BatchNorm couples the samples, so the batch runs whole). Batch forms,
-        accumulation and return value as BaseLitModel.eval_step; the loss is ce_weight * CE over max(#valid, 1)."""
+        accumulation, `curves` and return value as BaseLitModel.eval_step; the loss is ce_weight * CE over
+        max(#valid, 1)."""
         x, y, _ = self._unpack(batch)
         x, y = _pick_first_if_seq(x), _pick_first_if_seq(y)
         net = self.backbone
@@ -1151,17 +1193,19 @@ class LitCicek3DUNet_DepthAdapter_Published(pl.LightningModule):
                 torch.zeros(bsz, k, k, dtype=torch.int64, device=dev)) if per_sample else None
         labels = torch.empty(bsz, *x.shape[2:], dtype=torch.uint8, device=dev) if return_labels else None
         ign = -1 if self.ignore_index is None else int(self.ignore_index)
+        hist, sample_hist = _curve_buffers(curves, k, bsz, per_sample, dev)
         net.engine.eval_step(x, y, tally, self.target_depth, ignore_index=ign, training=net.training, per_sample=rows,
-                             labels_out=labels)
-        return {"loss": self._tally_loss(tally), "tally": tally, "per_sample": rows, "labels": labels}
+                             labels_out=labels, hist=hist, sample_hist=sample_hist)
+        return {"loss": self._tally_loss(tally), "tally": tally, "per_sample": rows, "labels": labels, "hist": hist,
+                "per_sample_hist": sample_hist}
 
     def _tally_loss(self, tally: LossTally) -> torch.Tensor:
         return (self.ce_weight * tally.nll[0] / tally.count[0].clamp(min=1).double()).float()
 
     @torch.no_grad()
-    def evaluate(self, batches):
+    def evaluate(self, batches, curves: Optional[int] = None):
         """BaseLitModel.evaluate for this variant (loss: ce_weight * CE, no Dice term)."""
-        return _evaluate(self, batches, lambda b, t: self.eval_step(b, tally=t))
+        return _evaluate(self, batches, lambda b, t, h: self.eval_step(b, tally=t, curves=h), curves)
 
     def fused_optimizer_state(self) -> Dict[str, object]:
         """Momentum buffer + step count of the fused SGD, for checkpoint / resume (save next to `state_dict()`)."""

@@ -361,10 +361,11 @@ class CicekEngine:
     def eval_step(self, x: torch.Tensor, labels: torch.Tensor, tally: LossTally, target_depth: Optional[int],
                   ignore_index: int = 255, training: bool = False,
                   per_sample: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None,
-                  labels_out: Optional[torch.Tensor] = None):
+                  labels_out: Optional[torch.Tensor] = None, hist: Optional[torch.Tensor] = None,
+                  sample_hist: Optional[torch.Tensor] = None):
         """Forward + head + CE/confusion over the whole batch, with no gradient and no logits in memory: the tally of
         `infer(x, target_depth, training)` accumulates (+=) into `tally` (BatchNorm as `training` selects, like infer).
-        per_sample / labels_out as in SpffEngine.eval_step."""
+        per_sample / labels_out / hist / sample_hist as in SpffEngine.eval_step (at the original depth)."""
         x = self._check_input(x)
         n, _, d0, h, w = x.shape
         if labels.shape != (n, d0, h, w):
@@ -376,7 +377,7 @@ class CicekEngine:
         p = self._params()
         rows = per_sample if per_sample is not None else (None, None, None)
         ops.head_eval(hx, p["out.weight"], p["out.bias"], labels, ignore_index, tally.nll, tally.count, tally.confusion,
-                      *rows, labels_out)
+                      *rows, labels_out, hist=hist, sample_hist=sample_hist)
 
 
 def flat_names(named_params: List[Tuple[str, torch.Tensor]]):

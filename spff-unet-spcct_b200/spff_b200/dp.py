@@ -45,6 +45,14 @@ def allreduce_tally(nll: torch.Tensor, count: torch.Tensor, confusion: torch.Ten
             dist.all_reduce(t, op=dist.ReduceOp.SUM)
 
 
+def allreduce_hist(hist: torch.Tensor) -> None:
+    """Sum the softmax histograms of the evaluation step ([K,2,T] int64) over ranks in place, so that every rank
+    derives the same ROC / PR curves."""
+    _, n = world()
+    if n > 1:
+        dist.all_reduce(hist, op=dist.ReduceOp.SUM)
+
+
 def shard_range(total: int, rank: int | None = None, world_size: int | None = None) -> Tuple[int, int]:
     """[lo, hi) of the `total` independent units (slices / sliding-window tiles = whole z-slices)
     owned by `rank`: contiguous, sizes differ by at most one. No collective is involved."""

@@ -649,11 +649,14 @@ class SpffEngine:
 
     def eval_step(self, x: torch.Tensor, labels: torch.Tensor, tally: "LossTally", group: int = 32,
                   ignore_index: int = 255, per_sample: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None,
-                  labels_out: Optional[torch.Tensor] = None, staged: Optional["StagedBatch"] = None):
+                  labels_out: Optional[torch.Tensor] = None, staged: Optional["StagedBatch"] = None,
+                  hist: Optional[torch.Tensor] = None, sample_hist: Optional[torch.Tensor] = None):
         """Forward + head + CE/confusion over the batch in sample groups, with no gradient: the loss statistics of
         `ce_plus_macro_dice_loss` / `per_class_metrics_3d` on `infer(x)` accumulate (+=) into `tally`, and the fp32 logits
         never reach memory. per_sample = (nll fp64 [B], count int64 [B], confusion int64 [B,K,K]) receives the same
-        tally per sample (+=); labels_out (uint8 [B,F,H,W]) the arg-max the tally counts. `staged`: as in train_step."""
+        tally per sample (+=); labels_out (uint8 [B,F,H,W]) the arg-max the tally counts. `staged`: as in train_step.
+        hist (int64 [K,2,T]) / sample_hist (int64 [B,K,2,T], with per_sample) receive (+=) the softmax histograms of
+        ops.head_eval."""
         x = self._check_input(x)
         bsz, _, d, h, w = x.shape
         if labels.shape != (bsz, d, h, w):
@@ -672,7 +675,8 @@ class SpffEngine:
                 staged.wait_labels(hi)
             rows = tuple(t[lo:hi] for t in per_sample) if per_sample is not None else (None, None, None)
             ops.head_eval(B.out["dec1"], p["out.weight"], p["out.bias"], labels[lo:hi], ignore_index, tally.nll,
-                          tally.count, tally.confusion, *rows, labels_out[lo:hi] if labels_out is not None else None)
+                          tally.count, tally.confusion, *rows, labels_out[lo:hi] if labels_out is not None else None,
+                          hist=hist, sample_hist=sample_hist[lo:hi] if sample_hist is not None else None)
 
 
 class StagedBatch:

@@ -362,10 +362,21 @@ def head_loss_fused(x, w, b, labels, ignore_index, n_valid, gscale, acc, counts,
 
 
 def head_eval(x, w, b, labels, ignore_index, acc, counts, confusion, sample_acc=None, sample_counts=None,
-              sample_confusion=None, labels_out=None):
+              sample_confusion=None, labels_out=None, hist=None, sample_hist=None):
     """Fused evaluation head (no logits in memory): the loss statistics of head_fwd + ce_confusion += into acc /
     counts / confusion; optionally per sample (fp64 [n], int64 [n], int64 [n,K,K], +=) and the uint8 arg-max map
-    [n,d,h,w] the tally counts."""
+    [n,d,h,w] the tally counts. `hist` (int64 [K,2,T], +=) adds the per-class histogram of the softmax probability
+    over T = hist.shape[-1] bins, positives in [c,0] and negatives in [c,1] (spff_head_eval_hist); `sample_hist`
+    (int64 [n,K,2,T]) is the same per sample and goes with the per-sample tallies."""
+    if hist is not None:
+        k, bins = w.shape[0], hist.shape[-1]
+        assert hist.dtype == torch.int64 and hist.is_contiguous() and tuple(hist.shape) == (k, 2, bins)
+        if sample_hist is not None:
+            n = x.shape[0]
+            assert sample_hist.dtype == torch.int64 and sample_hist.is_contiguous()
+            assert tuple(sample_hist.shape) == (n, k, 2, bins)
+    else:
+        assert sample_hist is None, "sample_hist needs hist"
     k = w.shape[0]
     s, ldx = _view(x, 32)
     assert labels.is_contiguous() and labels.numel() == s.n * s.d * s.h * s.w
@@ -377,8 +388,13 @@ def head_eval(x, w, b, labels, ignore_index, acc, counts, confusion, sample_acc=
         assert sample_confusion.numel() == s.n * k * k
     if labels_out is not None:
         assert labels_out.dtype == torch.uint8 and labels_out.is_contiguous() and labels_out.numel() == s.n * s.d * s.h * s.w
-    call("spff_head_eval", ptr(x), ldx, 32, ptr(w), ptr(b), ptr(labels), _label_bytes(labels), int(ignore_index), k, s,
-         ptr(acc), ptr(counts), ptr(confusion), *(ptr(t) for t in per), ptr(labels_out), stream_ptr())
+    if hist is None:
+        call("spff_head_eval", ptr(x), ldx, 32, ptr(w), ptr(b), ptr(labels), _label_bytes(labels), int(ignore_index), k, s,
+             ptr(acc), ptr(counts), ptr(confusion), *(ptr(t) for t in per), ptr(labels_out), stream_ptr())
+    else:
+        call("spff_head_eval_hist", ptr(x), ldx, 32, ptr(w), ptr(b), ptr(labels), _label_bytes(labels), int(ignore_index),
+             k, s, ptr(acc), ptr(counts), ptr(confusion), *(ptr(t) for t in per), ptr(labels_out), int(hist.shape[-1]),
+             ptr(hist), ptr(sample_hist), stream_ptr())
 
 
 def scale_by_count(g, count, factor: float = 1.0):
