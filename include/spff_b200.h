@@ -263,6 +263,34 @@ int spff_head_eval_hist(const void* x, long long ldx, int cin, const float* w, c
                         long long* confusion, double* sample_acc, long long* sample_counts, long long* sample_confusion,
                         uint8_t* labels_out, int bins, long long* hist, long long* sample_hist, void* stream);
 
+/* ---- averaged softmax: ensembles and mirror test-time augmentation ------------------------------------------
+ * Head + softmax added into a probability accumulator: for every position (n,d,h,w) of the network output,
+ * p_c = e_c / sum(e) (fp32, IEEE division: the p of spff_head_eval_hist, from the same logits) and
+ *   acc[n][d][h'][w'][c] = beta * acc[...][c] + p_c,   h' = H-1-h when flip & 1, w' = W-1-w when flip & 2,
+ * i.e. the inverse of an input flip is folded into the store. acc: fp32 [N,D,H,W,16] (64 B per position, 16-byte
+ * aligned); classes >= K are written as 0 when beta = 0 and never touched when beta = 1. Each element is written by
+ * one thread per call (no atomics, deterministic); beta = 0 does not read acc. x as in spff_head_eval. k in [2,16],
+ * flip in [0,3], beta 0 or 1, N <= 65535. */
+int spff_head_prob_accum(const void* x, long long ldx, int cin, const float* w, const float* b, int k, spff_shape s,
+                         int flip, int beta, float* acc, void* stream);
+/* One pass over an accumulator of spff_head_prob_accum: p̄_c = scale * acc_c (fp32; scale = 1 / number of passes), the
+ * arg-max is the first maximum of acc_c over c < K (torch.argmax; taken on acc so that the scaling cannot create ties).
+ * Outputs, each optional:
+ *  - labels_out uint8 [N,D,H,W]: the arg-max;
+ *  - proba_out fp16 [N,K,D,H,W] (class-major, the layout of softmax(model(x), 1)): p̄_c rounded to nearest;
+ *  - with labels (uint8 or int64 [N,D,H,W]; NULL = no tally, and then no tally output may be given) the tally of
+ *    spff_head_eval (+=): a label equal to ignore_index is not counted; a label y in [0,K) counts in counts, adds
+ *    -log(max(p̄_y, FLT_MIN)) to nll and one to confusion[y][arg]; any other label counts in counts only.
+ *    sample_acc / sample_counts / sample_confusion: the same per sample (together or not at all);
+ *  - hist int64 [K][2][bins] (+=, needs labels): for every voxel with a label in [0,K) and every class c, p̄_c falls in
+ *    bin min(floor(p̄_c * bins), bins - 1) of [c][0] (label == c) or [c][1]; bins in [16, 1024]; sample_hist
+ *    [N][K][2][bins] is given exactly when the per-sample tallies are.
+ * k in [2,16], acc 16-byte aligned, N <= 65535. */
+int spff_prob_finalize(const float* acc, int k, spff_shape s, float scale, const void* labels, int label_bytes,
+                       int ignore_index, double* nll, long long* counts, long long* confusion, double* sample_acc,
+                       long long* sample_counts, long long* sample_confusion, uint8_t* labels_out, int bins,
+                       long long* hist, long long* sample_hist, void* proba_out, void* stream);
+
 /* ---- "3DUNet" control: Cicek3DUNet + depth adapter (models.py:718-777; config.py:283-311) ---------------
  * Its 3x3x3 convolutions, normalise + ReLU passes (slope 0), head and loss are the entry points above;
  * the ones below are what only this variant needs. */

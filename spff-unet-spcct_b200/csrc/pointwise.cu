@@ -6,13 +6,17 @@
 //     and backward, fused with the loss for training and, forward only, for evaluation;
 //   * cross-entropy with ignore_index + the hard confusion tally that macro_dice_loss and
 //     per_class_metrics_3d derive all their counts from (innovative3D/helpers.py:668-725, 782-803);
+//   * the averaged softmax of ensembles and mirror test-time augmentation: the head's softmax added into
+//     an fp32 probability accumulator, and one finishing pass to arg-max / probabilities / tallies;
 //   * Adam (BaseLitModel.configure_optimizers, models.py:591-594).
 // All are bandwidth-bound: one thread per voxel (or per 16-byte channel vector), coalesced
 // accesses, weights broadcast from constant / shared memory.
 #include "common.h"
 #include "ptx.cuh"
 
+#include <cfloat>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 namespace spff {
 namespace {
@@ -1461,6 +1465,231 @@ head_eval_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
 }
 
 // ---------------------------------------------------------------------------------------------
+// Averaged softmax (ensembles, mirror TTA). head_prob_accum_kernel: the logits / softmax of head_eval_mma_kernel
+// (same functions, so the same numbers), p_c = e_c / se with the IEEE division the histogram uses, added into the
+// fp32 accumulator acc [n][d][h][w][16] at the position mirrored back by `flip` (1 = H, 2 = W). Within one (n, d)
+// plane the flip is a bijection, so every accumulator element has exactly one writer per launch: plain
+// load-add-store, deterministic. beta = 0 stores p (and 0 for classes >= K) without reading acc.
+// ---------------------------------------------------------------------------------------------
+constexpr int kPaBlocksPerSm = 3;
+
+// x rows (two 16-byte halves per lane) of `tile`; zeros past `total` (hm_fetch without labels)
+__device__ __forceinline__ void hm_fetch_x(const __nv_bfloat16* __restrict__ x, long long ldx, long long total,
+                                           long long ntiles, long long tile, int lane, uint4& nx0, uint4& nx1) {
+  nx0 = nx1 = make_uint4(0, 0, 0, 0);
+  if (tile >= ntiles) return;
+  const long long q0 = tile * 16;
+  const int pos = lane >> 1, half = lane & 1;
+  if (q0 + pos < total) {
+    const uint4* src = reinterpret_cast<const uint4*>(x + (q0 + pos) * ldx + half * 16);
+    nx0 = __ldg(src);
+    nx1 = __ldg(src + 1);
+  }
+}
+
+__global__ void __launch_bounds__(kHmWarps * 32, kPaBlocksPerSm)
+head_prob_accum_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, int K, int H, int W, long long dhw, int flip,
+                       int beta, float* __restrict__ acc) {
+  __shared__ __align__(16) __nv_bfloat16 xs[kHmWarps][16][kHmXPitch];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int g = lane >> 2, t = lane & 3;
+  HmLogitW wl;
+  hm_logit_weights(K, g, t, wl);
+  const long long n = blockIdx.y;
+  x += n * dhw * ldx;
+  acc += n * dhw * kMaxK;
+  const long long hw = static_cast<long long>(H) * W;
+  const long long ntiles = (dhw + 15) / 16;
+  const long long tstep = static_cast<long long>(gridDim.x) * kHmWarps;
+  uint4 nx0, nx1;
+  hm_fetch_x(x, ldx, dhw, ntiles, static_cast<long long>(blockIdx.x) * kHmWarps + warp, lane, nx0, nx1);
+  for (long long tile = static_cast<long long>(blockIdx.x) * kHmWarps + warp; tile < ntiles; tile += tstep) {
+    const long long p0 = tile * 16;
+    hm_stage(xs[warp], lane, nx0, nx1);
+    hm_fetch_x(x, ldx, dhw, ntiles, tile + tstep, lane, nx0, nx1);
+    __syncwarp();
+    float l[2][4];
+    hm_logits(xs[warp], lane, wl, l);
+#pragma unroll
+    for (int rr = 0; rr < 2; ++rr) {
+      const long long pos = p0 + g + 8 * rr;
+      float v[4], mx, e[4], se, ll;
+      int cls[4], arg;
+      hm_row_softmax(l, rr, t, K, -1, v, cls, mx, arg, e, se, ll);
+      if (pos < dhw) {
+        const long long plane = pos / hw, rem = pos - plane * hw;
+        int hh = static_cast<int>(rem / W), ww = static_cast<int>(rem - static_cast<long long>(hh) * W);
+        if (flip & 1) hh = H - 1 - hh;
+        if (flip & 2) ww = W - 1 - ww;
+        float* dst = acc + (plane * hw + static_cast<long long>(hh) * W + ww) * kMaxK;
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {   // this lane's classes 8j + 2t, 8j + 2t + 1 (e[2j], e[2j + 1])
+          const int c0 = 8 * j + 2 * t;
+          const float2 p = make_float2(c0 < K ? __fdiv_rn(e[2 * j], se) : 0.f, c0 + 1 < K ? __fdiv_rn(e[2 * j + 1], se) : 0.f);
+          float2* d2 = reinterpret_cast<float2*>(dst + c0);
+          if (!beta) {
+            *d2 = p;
+          } else if (c0 + 1 < K) {
+            float2 o = *d2;
+            o.x = __fadd_rn(o.x, p.x);
+            o.y = __fadd_rn(o.y, p.y);
+            *d2 = o;
+          } else if (c0 < K) {
+            dst[c0] = __fadd_rn(dst[c0], p.x);
+          }
+        }
+      }
+    }
+    __syncwarp();   // the tile is read before the next iteration overwrites it
+  }
+}
+
+// prob_finalize_kernel: one thread per position of sample blockIdx.y. p̄_c = scale * acc_c; the arg-max is the first
+// maximum of acc_c over c < K (on acc, so that the scaling cannot create ties). With labels: a label equal to
+// ignore_index is not counted; a label in [0, K) counts, adds -log(max(p̄_y, FLT_MIN)) to the nll and one to
+// confusion[y][arg] (and, with HIST, every class's p̄_c to bin min(floor(p̄_c * T), T - 1) of hist[c][y == c ? 0 : 1]);
+// any other label counts only. Tallies are block-private in shared memory and flushed once per block, as in
+// head_eval_mma_kernel (the register bins too).
+constexpr int kPfThreads = 256;
+
+template <typename LabelT, bool HIST>
+__global__ void __launch_bounds__(kPfThreads)
+prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float scale, const void* __restrict__ labels,
+                     int ignore_index, double* __restrict__ nll, unsigned long long* __restrict__ counts,
+                     unsigned long long* __restrict__ confusion, double* __restrict__ sample_acc,
+                     unsigned long long* __restrict__ sample_counts, unsigned long long* __restrict__ sample_confusion,
+                     uint8_t* __restrict__ labels_out, __half* __restrict__ proba_out, int T,
+                     unsigned long long* __restrict__ hist, unsigned long long* __restrict__ sample_hist) {
+  __shared__ unsigned int s_conf[kMaxK * kMaxK];
+  __shared__ float s_nll[kPfThreads / 32];
+  __shared__ unsigned int s_cnt[kPfThreads / 32];
+  extern __shared__ unsigned int s_hist[];   // HIST: [K][2][T]
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int i = threadIdx.x; i < K * K; i += blockDim.x) s_conf[i] = 0;
+  if constexpr (HIST)
+    for (int i = threadIdx.x; i < K * 2 * T; i += blockDim.x) s_hist[i] = 0;
+  unsigned int hot_neg[kMaxK], hot_pos[kMaxK];   // HIST: bin 0 of negatives, bin T - 1 of positives
+#pragma unroll
+  for (int c = 0; c < kMaxK; ++c) hot_neg[c] = hot_pos[c] = 0;
+  __syncthreads();
+  const long long n = blockIdx.y;
+  acc += n * dhw * kMaxK;
+  const LabelT* lab_in = labels ? static_cast<const LabelT*>(labels) + n * dhw : nullptr;
+  if (labels_out) labels_out += n * dhw;
+  if (proba_out) proba_out += n * K * dhw;
+  float nll_sum = 0.f;
+  unsigned int cnt = 0;
+  for (long long pos = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; pos < dhw;
+       pos += static_cast<long long>(gridDim.x) * blockDim.x) {
+    float a[kMaxK];
+    const float4* src = reinterpret_cast<const float4*>(acc + pos * kMaxK);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float4 q = __ldg(src + j);
+      a[4 * j] = q.x;
+      a[4 * j + 1] = q.y;
+      a[4 * j + 2] = q.z;
+      a[4 * j + 3] = q.w;
+    }
+    int arg = 0;
+    float mx = a[0];
+#pragma unroll
+    for (int c = 1; c < kMaxK; ++c)
+      if (c < K && a[c] > mx) {   // ascending class order: strict > keeps the first maximum
+        mx = a[c];
+        arg = c;
+      }
+    float p[kMaxK];
+#pragma unroll
+    for (int c = 0; c < kMaxK; ++c) p[c] = __fmul_rn(scale, a[c]);
+    if (labels_out) labels_out[pos] = static_cast<uint8_t>(arg);
+    if (proba_out) {
+#pragma unroll
+      for (int c = 0; c < kMaxK; ++c)
+        if (c < K) proba_out[c * dhw + pos] = __float2half_rn(p[c]);
+    }
+    if (lab_in) {
+      const int lab = static_cast<int>(lab_in[pos]);
+      if (lab != ignore_index) {
+        ++cnt;
+        if (lab >= 0 && lab < K) {
+          float py = p[0];
+#pragma unroll
+          for (int c = 1; c < kMaxK; ++c)
+            if (c == lab) py = p[c];
+          nll_sum += -logf(fmaxf(py, FLT_MIN));
+          atomicAdd(&s_conf[lab * K + arg], 1u);
+          if constexpr (HIST) {
+#pragma unroll
+            for (int c = 0; c < kMaxK; ++c)
+              if (c < K) {
+                const int bin = min(static_cast<int>(__fmul_rn(p[c], static_cast<float>(T))), T - 1);
+                const bool positive = c == lab;
+                if (positive && bin == T - 1)
+                  ++hot_pos[c];
+                else if (!positive && bin == 0)
+                  ++hot_neg[c];
+                else
+                  atomicAdd(&s_hist[(c * 2 + (positive ? 0 : 1)) * T + bin], 1u);
+              }
+          }
+        }
+      }
+    }
+  }
+  if (!lab_in) return;
+  for (int o = 16; o > 0; o >>= 1) {
+    nll_sum += __shfl_xor_sync(0xffffffffu, nll_sum, o);
+    cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+  }
+  if (lane == 0) {
+    s_nll[warp] = nll_sum;
+    s_cnt[warp] = cnt;
+  }
+  if constexpr (HIST) {   // the register bins: a warp sum, then one shared add per warp and class
+#pragma unroll
+    for (int c = 0; c < kMaxK; ++c) {
+      if (c >= K) break;
+      unsigned int hp = hot_pos[c], hn = hot_neg[c];
+      for (int o = 16; o > 0; o >>= 1) {
+        hp += __shfl_xor_sync(0xffffffffu, hp, o);
+        hn += __shfl_xor_sync(0xffffffffu, hn, o);
+      }
+      if (lane == 0) {
+        if (hp) atomicAdd(&s_hist[(c * 2 + 0) * T + T - 1], hp);
+        if (hn) atomicAdd(&s_hist[(c * 2 + 1) * T + 0], hn);
+      }
+    }
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double tt = 0;
+    unsigned long long c = 0;
+    for (int wv = 0; wv < kPfThreads / 32; ++wv) {
+      tt += s_nll[wv];
+      c += s_cnt[wv];
+    }
+    atomicAdd(nll, tt);
+    atomicAdd(counts, c);
+    if (sample_acc) {
+      atomicAdd(sample_acc + n, tt);
+      atomicAdd(sample_counts + n, c);
+    }
+  }
+  for (int i = threadIdx.x; i < K * K; i += blockDim.x)
+    if (s_conf[i]) {
+      atomicAdd(confusion + i, static_cast<unsigned long long>(s_conf[i]));
+      if (sample_confusion) atomicAdd(sample_confusion + n * K * K + i, static_cast<unsigned long long>(s_conf[i]));
+    }
+  if constexpr (HIST)
+    for (int i = threadIdx.x; i < K * 2 * T; i += blockDim.x)
+      if (s_hist[i]) {
+        atomicAdd(hist + i, static_cast<unsigned long long>(s_hist[i]));
+        if (sample_hist) atomicAdd(sample_hist + n * K * 2 * T + i, static_cast<unsigned long long>(s_hist[i]));
+      }
+}
+
+// ---------------------------------------------------------------------------------------------
 // Adam (torch.optim.Adam semantics, no weight decay / amsgrad)
 // ---------------------------------------------------------------------------------------------
 __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
@@ -1575,6 +1804,18 @@ int head_eval_launch(const char* name, const void* x, long long ldx, int cin, co
         static_cast<const bf16*>(x), ldx, labels, ignore_index, k, dhw, acc, cnt, conf, sample_acc, scnt, sconf, labels_out,
         bins, hst, shst);
   SPFF_CUDA(cudaGetLastError());
+  return 0;
+}
+
+template <typename LabelT>
+int prob_finalize_hist_attr() {   // once per device, as head_eval_hist_attr
+  static bool attr_set[spff::kMaxDevices] = {};
+  const int dev = spff::current_device();
+  if (!attr_set[dev]) {
+    SPFF_CUDA(cudaFuncSetAttribute(spff::prob_finalize_kernel<LabelT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   static_cast<int>(sizeof(unsigned int) * spff::kMaxK * 2 * spff::kHeMaxBins)));
+    attr_set[dev] = true;
+  }
   return 0;
 }
 
@@ -1827,6 +2068,88 @@ int spff_head_eval_hist(const void* x, long long ldx, int cin, const float* w, c
   return head_eval_launch("head_eval_hist", x, ldx, cin, w, b, labels, label_bytes, ignore_index, k, s, acc, counts,
                           confusion, sample_acc, sample_counts, sample_confusion, labels_out, bins, hist, sample_hist,
                           stream);
+}
+
+int spff_head_prob_accum(const void* x, long long ldx, int cin, const float* w, const float* b, int k, spff_shape s,
+                         int flip, int beta, float* acc, void* stream) {
+  SPFF_ENTRY_CHECK();
+  SPFF_REQUIRE(x && w && b && acc, "head_prob_accum: null pointer");
+  SPFF_REQUIRE(k >= 2 && k <= spff::kMaxK, "head_prob_accum: classes must be in [2, %d] (got %d)", spff::kMaxK, k);
+  SPFF_REQUIRE(flip >= 0 && flip <= 3, "head_prob_accum: flip is a bit set of 1 (H) and 2 (W) (got %d)", flip);
+  SPFF_REQUIRE(beta == 0 || beta == 1, "head_prob_accum: beta must be 0 or 1 (got %d)", beta);
+  SPFF_REQUIRE((reinterpret_cast<uintptr_t>(acc) & 15) == 0, "head_prob_accum: acc must be 16-byte aligned");
+  SPFF_REQUIRE(ldx >= cin && ldx % 8 == 0, "head_prob_accum: bad channel pitch");
+  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "head_prob_accum: bad shape (N must be <= 65535)");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int e = spff::upload_head(w, b, k, cin, st);
+  if (e) return e;
+  const long long dhw = static_cast<long long>(s.d) * s.h * s.w;
+  // the grid of head_eval: one block row per sample, ~4 waves of resident blocks, no more blocks than warp tiles
+  const long long warp_tiles = ((dhw + 15) / 16 + spff::kHmWarps - 1) / spff::kHmWarps;
+  long long per = (4LL * spff::kPaBlocksPerSm * spff::num_sms() + s.n - 1) / s.n;
+  if (per > warp_tiles) per = warp_tiles;
+  if (per < 1) per = 1;
+  const dim3 grid(static_cast<unsigned>(per), s.n);
+  spff::head_prob_accum_kernel<<<grid, spff::kHmWarps * 32, 0, st>>>(static_cast<const bf16*>(x), ldx, k, s.h, s.w, dhw,
+                                                                      flip, beta, acc);
+  SPFF_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int spff_prob_finalize(const float* acc, int k, spff_shape s, float scale, const void* labels, int label_bytes,
+                       int ignore_index, double* nll, long long* counts, long long* confusion, double* sample_acc,
+                       long long* sample_counts, long long* sample_confusion, uint8_t* labels_out, int bins,
+                       long long* hist, long long* sample_hist, void* proba_out, void* stream) {
+  SPFF_ENTRY_CHECK();
+  SPFF_REQUIRE(acc, "prob_finalize: null accumulator");
+  SPFF_REQUIRE(k >= 2 && k <= spff::kMaxK, "prob_finalize: classes must be in [2, %d] (got %d)", spff::kMaxK, k);
+  SPFF_REQUIRE((reinterpret_cast<uintptr_t>(acc) & 15) == 0, "prob_finalize: acc must be 16-byte aligned");
+  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "prob_finalize: bad shape (N must be <= 65535)");
+  SPFF_REQUIRE(scale > 0.f, "prob_finalize: scale must be positive");
+  SPFF_REQUIRE(!labels || label_bytes == 1 || label_bytes == 8, "prob_finalize: labels must be uint8 or int64");
+  SPFF_REQUIRE(labels ? (nll && counts && confusion) : !(nll || counts || confusion || sample_acc || hist),
+               "prob_finalize: the tally (nll, counts, confusion) is given exactly when the labels are");
+  SPFF_REQUIRE((sample_acc != nullptr) == (sample_counts != nullptr) && (sample_acc != nullptr) == (sample_confusion != nullptr),
+               "prob_finalize: the per-sample arrays are given together or not at all");
+  SPFF_REQUIRE(!hist || (bins >= spff::kHeMinBins && bins <= spff::kHeMaxBins),
+               "prob_finalize: bins must be in [%d, %d] (got %d)", spff::kHeMinBins, spff::kHeMaxBins, bins);
+  SPFF_REQUIRE(hist || !sample_hist, "prob_finalize: sample_hist needs hist");
+  SPFF_REQUIRE(!hist || (sample_hist != nullptr) == (sample_acc != nullptr),
+               "prob_finalize: the per-sample histogram is given exactly when the per-sample tallies are");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long dhw = static_cast<long long>(s.d) * s.h * s.w;
+  const long long blocks_needed = (dhw + spff::kPfThreads - 1) / spff::kPfThreads;
+  long long per = (16LL * spff::num_sms() + s.n - 1) / s.n;   // ~2 waves of 8 resident blocks per SM
+  if (per > blocks_needed) per = blocks_needed;
+  if (per < 1) per = 1;
+  const dim3 grid(static_cast<unsigned>(per), s.n);
+  auto cnt = reinterpret_cast<unsigned long long*>(counts);
+  auto conf = reinterpret_cast<unsigned long long*>(confusion);
+  auto scnt = reinterpret_cast<unsigned long long*>(sample_counts);
+  auto sconf = reinterpret_cast<unsigned long long*>(sample_confusion);
+  auto hst = reinterpret_cast<unsigned long long*>(hist);
+  auto shst = reinterpret_cast<unsigned long long*>(sample_hist);
+  auto pout = static_cast<__half*>(proba_out);
+  const size_t hist_smem = hist ? sizeof(unsigned int) * k * 2 * bins : 0;
+  if (hist) {
+    const int e = label_bytes == 1 ? prob_finalize_hist_attr<uint8_t>() : prob_finalize_hist_attr<long long>();
+    if (e) return e;
+  }
+  const int T = hist ? bins : 0;
+  if (label_bytes != 8 && !hist)
+    spff::prob_finalize_kernel<uint8_t, false><<<grid, spff::kPfThreads, 0, st>>>(
+        acc, k, dhw, scale, labels, ignore_index, nll, cnt, conf, sample_acc, scnt, sconf, labels_out, pout, T, hst, shst);
+  else if (!hist)
+    spff::prob_finalize_kernel<long long, false><<<grid, spff::kPfThreads, 0, st>>>(
+        acc, k, dhw, scale, labels, ignore_index, nll, cnt, conf, sample_acc, scnt, sconf, labels_out, pout, T, hst, shst);
+  else if (label_bytes == 1)
+    spff::prob_finalize_kernel<uint8_t, true><<<grid, spff::kPfThreads, hist_smem, st>>>(
+        acc, k, dhw, scale, labels, ignore_index, nll, cnt, conf, sample_acc, scnt, sconf, labels_out, pout, T, hst, shst);
+  else
+    spff::prob_finalize_kernel<long long, true><<<grid, spff::kPfThreads, hist_smem, st>>>(
+        acc, k, dhw, scale, labels, ignore_index, nll, cnt, conf, sample_acc, scnt, sconf, labels_out, pout, T, hst, shst);
+  SPFF_CUDA(cudaGetLastError());
+  return 0;
 }
 
 int spff_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr,

@@ -20,6 +20,7 @@ LitSPCT_SEspec ("SP_UNet", depth padded 5 -> 16), LitSPCT_ControlUNet ("PlainCor
 from __future__ import annotations
 
 import copy
+import dataclasses
 import os
 from typing import Dict, List, Optional
 
@@ -32,7 +33,7 @@ except ImportError:  # not in this image: a minimal stand-in with the same metho
     from ._lightning import pl
 
 from spff_b200 import dp, ops
-from spff_b200.engine import LossTally, NetConfig, SpffEngine, StagedBatch
+from spff_b200.engine import LossTally, NetConfig, SpffEngine, StagedBatch, run_ensemble
 from spff_b200.sched import PlateauLR
 
 from .config import BEST_LR, IGNORE_INDEX, NUM_CLASSES, NUM_FRAMES
@@ -709,8 +710,8 @@ class BaseLitModel(pl.LightningModule):
         {"loss": float, "metrics": per_class_metrics_3d's 9-tuple, "tally", "voxels"}; with `curves` = T bins also
         "hist" (int64 [K,2,T] on the device) and "curves" (`helpers.curves_from_hist`: per-class ROC / PR curves, AUROC,
         AP and their macro averages)."""
-        return _evaluate(self, batches, lambda b, t, h: self.eval_step(b, tally=t, sample_group=sample_group, curves=h),
-                         curves)
+        return _evaluate(self.hparams.num_classes, next(self.parameters()).device, self._tally_loss, batches,
+                         lambda b, t, h: self.eval_step(b, tally=t, sample_group=sample_group, curves=h), curves)
 
 
 def _eval_voxels(batch) -> int:
@@ -740,13 +741,11 @@ def _curve_buffers(curves, k: int, bsz: int, per_sample: bool, dev):
     return hist, sample_hist
 
 
-def _evaluate(lit, batches, step, curves: Optional[int] = None):
+def _evaluate(k: int, dev, loss_fn, batches, step, curves: Optional[int] = None):
     """Shared driver of the `evaluate` methods: one tally (and, with `curves` = T, one [K,2,T] softmax histogram) over
     the batches, ONE all-reduce of the tally (plus the voxel count and the histogram) under data parallelism, ONE
-    device->host copy at the end."""
+    device->host copy at the end. k classes, `dev` the device of the tallies, loss_fn(tally) -> device scalar."""
     tally, voxels = None, 0
-    dev = next(lit.parameters()).device
-    k = lit.hparams.num_classes
     hist = _curve_buffers(curves, k, 0, False, dev)[0]
     for batch in batches:
         tally = step(batch, tally, hist)["tally"]
@@ -759,7 +758,7 @@ def _evaluate(lit, batches, step, curves: Optional[int] = None):
         torch.distributed.all_reduce(vox)
         if hist is not None:
             dp.allreduce_hist(hist)
-    loss = lit._tally_loss(tally).double().reshape(1)
+    loss = loss_fn(tally).double().reshape(1)
     # one copy: [nll (fp64 bits), count, confusion..., voxels, loss (fp64 bits), histogram...]
     parts = [tally._buf, vox, loss.view(torch.int64)] + ([hist.view(-1)] if hist is not None else [])
     host = torch.cat(parts).cpu()
@@ -1205,7 +1204,8 @@ class LitCicek3DUNet_DepthAdapter_Published(pl.LightningModule):
     @torch.no_grad()
     def evaluate(self, batches, curves: Optional[int] = None):
         """BaseLitModel.evaluate for this variant (loss: ce_weight * CE, no Dice term)."""
-        return _evaluate(self, batches, lambda b, t, h: self.eval_step(b, tally=t, curves=h), curves)
+        return _evaluate(self.hparams.num_classes, next(self.parameters()).device, self._tally_loss, batches,
+                         lambda b, t, h: self.eval_step(b, tally=t, curves=h), curves)
 
     def fused_optimizer_state(self) -> Dict[str, object]:
         """Momentum buffer + step count of the fused SGD, for checkpoint / resume (save next to `state_dict()`)."""
@@ -1237,6 +1237,126 @@ class LitCicek3DUNet_DepthAdapter_Published(pl.LightningModule):
         net = self.backbone
         net.materialize()
         return net.engine.infer(x.to(net._flat.device), self.target_depth, training=net.training, argmax=True)
+
+
+class SpctEnsemble:
+    """Seed ensembles and mirror test-time augmentation of the depth-preserving SPCT family: the softmax averaged over
+    members and input flips, on the device, with no logits in memory.
+
+    `members`: Lightning wrappers whose `.model` is a UNet3D_SpectralCore (SPFF-UNet, E_SP_UNet, FG_SP_UNet,
+    PlainCore_UNet) or such cores themselves, of one `net_config()` and one device; the ensemble holds references to
+    them (no copies of weights) and touches no optimizer or fused-step state. `tta`: None (the input as given) or
+    "flip" (identity, H, W and H+W mirrors; the depth axis holds the energy bins and is not a symmetry).
+
+    Every pass runs the member on the (flipped) input and adds its softmax, mirrored back, into an fp32 accumulator of
+    one sample group; p̄ = the mean over members x flips. `predict_labels` / `predict_proba` give its arg-max / p̄,
+    `eval_step` / `evaluate` the loss, metrics and curves of BaseLitModel's on p̄: the loss is ce_plus_macro_dice_loss on
+    the averaged probabilities (CE of p̄ + 0.5 * (1 - hard macro Dice of its arg-max))."""
+
+    def __init__(self, members, tta: Optional[str] = None):
+        if tta not in (None, "flip"):
+            raise ValueError(f"tta must be None or 'flip', got {tta!r}")
+        members = list(members)
+        if not members:
+            raise ValueError("an ensemble needs at least one member")
+        cores = []
+        for i, m in enumerate(members):
+            if isinstance(m, _LitSPCT_Base):
+                raise NotImplementedError(f"member {i}: SP_UNet pads the depth to 16 planes and crops its logits back; the "
+                                          "ensemble averages the softmax of depth-preserving cores only")
+            if isinstance(m, (LitCicek3DUNet_DepthAdapter_Published, Cicek3DUNet)):
+                raise NotImplementedError(f"member {i}: the 3DUNet's BatchNorm couples the samples of a batch, so its "
+                                          "output cannot be computed sample group by sample group like the SPCT family's")
+            core = m if isinstance(m, UNet3D_SpectralCore) else getattr(m, "model", None)
+            if not isinstance(core, UNet3D_SpectralCore):
+                raise TypeError(f"member {i}: expected a UNet3D_SpectralCore or a Lightning wrapper of one, got "
+                                f"{type(m).__name__}")
+            cores.append(core)
+        cfg0, dev0 = cores[0].net_config(), cores[0].out.weight.device
+        for i, core in enumerate(cores[1:], 1):
+            cfg = core.net_config()
+            for f in dataclasses.fields(cfg):
+                if getattr(cfg, f.name) != getattr(cfg0, f.name):
+                    raise ValueError(f"member {i}: net_config field {f.name!r} is {getattr(cfg, f.name)!r}, member 0 has "
+                                     f"{getattr(cfg0, f.name)!r}")
+            if core.out.weight.device != dev0:
+                raise ValueError(f"member {i} lives on {core.out.weight.device}, member 0 on {dev0}")
+        self.members, self.cores, self.tta = members, cores, tta
+        self.num_classes = cfg0.num_classes
+        self.flips = (0, 1, 2, 3) if tta == "flip" else (0,)
+        self._copy_stream = None
+
+    @property
+    def device(self) -> torch.device:
+        return self.cores[0].out.weight.device
+
+    def _engines(self, frames: int):
+        for core in self.cores:
+            core.materialize(frames)
+        return [core.engine for core in self.cores]
+
+    def _images(self, x) -> torch.Tensor:
+        x = _pick_first_if_seq(x)
+        return x.unsqueeze(1) if x.ndim == 4 else x
+
+    @torch.no_grad()
+    def predict_labels(self, x, sample_group: Optional[int] = None) -> torch.Tensor:
+        """uint8 label map [B,F,H,W]: the arg-max (first maximum) of the averaged softmax."""
+        x = self._images(x)
+        engines = self._engines(x.shape[2])
+        b, _, d, h, w = x.shape
+        out = torch.empty(b, d, h, w, dtype=torch.uint8, device=self.device)
+        run_ensemble(engines, x.to(self.device), self.flips, sample_group or self.cores[0].sample_group, labels_out=out)
+        return out
+
+    @torch.no_grad()
+    def predict_proba(self, x, sample_group: Optional[int] = None) -> torch.Tensor:
+        """float16 [B,K,F,H,W]: the averaged softmax (the layout of softmax(model(x), 1))."""
+        x = self._images(x)
+        engines = self._engines(x.shape[2])
+        b, _, d, h, w = x.shape
+        out = torch.empty(b, self.num_classes, d, h, w, dtype=torch.float16, device=self.device)
+        run_ensemble(engines, x.to(self.device), self.flips, sample_group or self.cores[0].sample_group, proba_out=out)
+        return out
+
+    @torch.no_grad()
+    def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False,
+                  sample_group: Optional[int] = None, curves=None):
+        """BaseLitModel.eval_step for the ensemble: the tally, per-sample rows, arg-max map and histograms of the
+        averaged softmax p̄ (same arguments, batch forms and return dict)."""
+        imgs, lbls = batch if isinstance(batch, (list, tuple)) else (batch["image"], batch["label"])
+        imgs, lbls = self._images(imgs), _pick_first_if_seq(lbls)
+        engines = self._engines(imgs.shape[2])
+        dev = self.device
+        if lbls.dtype not in (torch.uint8, torch.int64):
+            lbls = lbls.long()
+        group = sample_group or self.cores[0].sample_group
+        staged = None
+        if not imgs.is_cuda and not lbls.is_cuda:
+            if self._copy_stream is None:
+                self._copy_stream = torch.cuda.Stream(device=dev)
+            staged = StagedBatch(imgs, lbls, dev, group, self._copy_stream)
+            imgs, lbls = staged.x, staged.labels
+        else:
+            imgs = imgs.to(dev, non_blocking=True)
+            lbls = lbls.to(dev, non_blocking=True)
+        k = self.num_classes
+        tally = LossTally(k, dev) if tally is None else tally
+        bsz = imgs.shape[0]
+        rows = (torch.zeros(bsz, dtype=torch.float64, device=dev), torch.zeros(bsz, dtype=torch.int64, device=dev),
+                torch.zeros(bsz, k, k, dtype=torch.int64, device=dev)) if per_sample else None
+        labels = torch.empty(bsz, *imgs.shape[2:], dtype=torch.uint8, device=dev) if return_labels else None
+        hist, sample_hist = _curve_buffers(curves, k, bsz, per_sample, dev)
+        run_ensemble(engines, imgs, self.flips, group, labels=lbls, tally=tally, ignore_index=IGNORE_INDEX,
+                     per_sample=rows, labels_out=labels, hist=hist, sample_hist=sample_hist, staged=staged)
+        return {"loss": tally.loss(), "tally": tally, "per_sample": rows, "labels": labels, "hist": hist,
+                "per_sample_hist": sample_hist}
+
+    @torch.no_grad()
+    def evaluate(self, batches, sample_group: Optional[int] = None, curves: Optional[int] = None):
+        """BaseLitModel.evaluate for the ensemble: {"loss", "metrics", "tally", "voxels"} (+ "hist", "curves")."""
+        return _evaluate(self.num_classes, self.device, lambda t: t.loss(), batches,
+                         lambda b, t, h: self.eval_step(b, tally=t, sample_group=sample_group, curves=h), curves)
 
 
 # Model families outside the hot path (UNETR / SwinUNETR wrappers, R2U-Net, ResUNet++, their helper blocks and losses:

@@ -88,6 +88,8 @@ _PROTOTYPES = {
     "spff_head_eval": [_P, _LL, c_int, _P, _P, _P, c_int, c_int, c_int, Shape, _P, _P, _P, _P, _P, _P, _P, _P],
     "spff_head_eval_hist": [_P, _LL, c_int, _P, _P, _P, c_int, c_int, c_int, Shape, _P, _P, _P, _P, _P, _P, _P, c_int, _P,
                             _P, _P],
+    "spff_head_prob_accum": [_P, _LL, c_int, _P, _P, c_int, Shape, c_int, c_int, _P, _P],
+    "spff_prob_finalize": [_P, c_int, Shape, c_float, _P, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, c_int, _P, _P, _P, _P],
     "spff_count_valid": [_P, c_int, _LL, c_int, _P, _P],
     "spff_scale_by_count": [_P, _LL, _P, c_float, _P],
     "spff_loss_from_tally": [_P, _P, _P, c_int, c_double, _P, _P],

@@ -488,25 +488,26 @@ class SpffEngine:
         return x.float().contiguous()
 
     @staticmethod
-    def fit_group(group: int, d: int, h: int, w: int, device, train: bool) -> int:
+    def fit_group(group: int, d: int, h: int, w: int, device, train: bool, extra: float = 0.0) -> int:
         """Largest sample group <= `group` whose buffers fit in ~45 % of the free HBM. One sample holds, in units of
         one level-1 32-channel bf16 tensor (d*h*w*64 bytes): x1/a1/x2/out per block, the concat and pooled buffers
-        (16.7 units forward) plus the gradient scratch (26.5 units for a training step)."""
-        per = (26.5 if train else 16.7) * d * h * w * 64
+        (16.7 units forward) plus the gradient scratch (26.5 units for a training step). `extra`: further units per
+        sample that a caller keeps beside the buffers (ENSEMBLE_UNITS for run_ensemble)."""
+        per = ((26.5 if train else 16.7) + extra) * d * h * w * 64
         try:
             free, _ = torch.cuda.mem_get_info(device)
         except Exception:
             return max(1, group)
         return max(1, min(group, int(0.45 * free / per)))
 
-    def _fitted(self, group: int, d: int, h: int, w: int, device, train: bool) -> int:
-        """fit_group, decided once per (shape, mode, requested group) — before that shape's buffers exist, when the
-        free-memory reading still describes what is available to them."""
-        key = (group, d, h, w, str(device), train)
+    def _fitted(self, group: int, d: int, h: int, w: int, device, train: bool, extra: float = 0.0) -> int:
+        """fit_group, decided once per (shape, mode, requested group, extra) — before that shape's buffers exist, when
+        the free-memory reading still describes what is available to them."""
+        key = (group, d, h, w, str(device), train) + ((extra,) if extra else ())
         if key not in self._fit:
             if not any(k[1:4] == (d, h, w) for k in self._bufs):
                 self._bufs.clear()          # buffers of another slice size would otherwise count as unavailable
-            self._fit[key] = self.fit_group(group, d, h, w, device, train)
+            self._fit[key] = self.fit_group(group, d, h, w, device, train, extra)
         return self._fit[key]
 
     @staticmethod
@@ -677,6 +678,99 @@ class SpffEngine:
             ops.head_eval(B.out["dec1"], p["out.weight"], p["out.bias"], labels[lo:hi], ignore_index, tally.nll,
                           tally.count, tally.confusion, *rows, labels_out[lo:hi] if labels_out is not None else None,
                           hist=hist, sample_hist=sample_hist[lo:hi] if sample_hist is not None else None)
+
+
+# per sample, in fit_group's units, of run_ensemble beside the inference buffers: the fp32 probability accumulator
+# (16 classes x 4 B = 64 B per position, one unit) and the fp32 flipped input (4 B per position)
+ENSEMBLE_UNITS = 1.0 + 1.0 / 16
+
+
+def flip_tables(n: int, h: int, w: int, flip: int, device="cpu"):
+    """(amap int32 [n,h], bmap int32 [n,w]) that make spff_grid_aug's gather x[., ., amap[u], bmap[v]] torch.flip over H
+    (flip & 1) and / or W (flip & 2)."""
+    a = torch.arange(h, dtype=torch.int32)
+    b = torch.arange(w, dtype=torch.int32)
+    if flip & 1:
+        a = a.flip(0)
+    if flip & 2:
+        b = b.flip(0)
+    return a.to(device).expand(n, h).contiguous(), b.to(device).expand(n, w).contiguous()
+
+
+class _FlipGather:
+    """spff_grid_aug as a pure gather (not transposed, scale 1, shift 0, no noise or stamp): torch.flip of an fp32
+    [n,1,d,h,w] group over H / W, for up to `n` samples."""
+
+    def __init__(self, n: int, h: int, w: int, device):
+        self.maps = {f: flip_tables(n, h, w, f, device) for f in (1, 2, 3)}
+        self.zi = torch.zeros(n, dtype=torch.int32, device=device)
+        self.one = torch.ones(n, device=device)
+        self.zf = torch.zeros(n, device=device)
+        self.seed = torch.zeros(n, dtype=torch.int64, device=device)
+
+    def __call__(self, x: torch.Tensor, out: torch.Tensor, flip: int):
+        n, _, d, h, w = x.shape
+        a, b = self.maps[flip]
+        ops.grid_aug(x.view(n, d, h, w), None, out.view(n, d, h, w), None, a[:n], b[:n], self.zi[:n], self.one[:n],
+                     self.zf[:n], self.zf[:n], self.seed[:n], self.zi[:n], 0, 0)
+
+
+def run_ensemble(engines: List[SpffEngine], x: torch.Tensor, flips: Tuple[int, ...], group: int = 32,
+                 labels: Optional[torch.Tensor] = None, tally: Optional["LossTally"] = None, ignore_index: int = 255,
+                 per_sample: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None,
+                 labels_out: Optional[torch.Tensor] = None, proba_out: Optional[torch.Tensor] = None,
+                 hist: Optional[torch.Tensor] = None, sample_hist: Optional[torch.Tensor] = None,
+                 staged: Optional["StagedBatch"] = None):
+    """Averaged softmax of several networks of one NetConfig over input flips (1 = H, 2 = W, 0 = none), sample group by
+    sample group, with no logits in memory. Every member runs on the FIRST engine's inference buffers; for each group
+    and member (outer) and flip (inner): flip the input (spff_grid_aug), forward, and add the head's softmax, mirrored
+    back, into an fp32 [group,d,h,w,16] accumulator (ops.head_prob_accum). One ops.prob_finalize per group then writes
+    p̄ = mean over the passes: labels_out (uint8 [B,F,H,W], arg-max), proba_out (fp16 [B,K,F,H,W]) and, with labels,
+    the tally, per-sample rows and histograms of SpffEngine.eval_step computed on p̄. `staged`: as in train_step."""
+    first = engines[0]
+    x = first._check_input(x)
+    bsz, _, d, h, w = x.shape
+    if labels is not None:
+        if labels.shape != (bsz, d, h, w):
+            raise ValueError(f"labels must be [B,F,H,W] = {(bsz, d, h, w)}, got {tuple(labels.shape)}")
+        labels = labels.contiguous()
+    tables = []
+    for e in engines:   # once per call, not per group
+        e.refresh_weights()
+        tables.append(GateTables(e.cfg, e.params(), d, need_grad=False))
+    group = first._fitted(min(group, bsz), d, h, w, x.device, train=False, extra=ENSEMBLE_UNITS)
+    acc = torch.empty(group, d, h, w, 16, device=x.device)
+    flipped = any(flips)
+    xf = torch.empty(group, 1, d, h, w, device=x.device) if flipped else None
+    gather = _FlipGather(group, h, w, x.device) if flipped else None
+    scale = 1.0 / (len(engines) * len(flips))
+    tl = (tally.nll, tally.count, tally.confusion) if tally is not None else None
+
+    def rows(t, lo, hi):
+        return t[lo:hi] if t is not None else None
+    for lo, hi in first._groups(bsz, group):
+        n = hi - lo
+        if staged is not None:
+            staged.wait_images(hi)
+        B = first.buffers(n, d, h, w, x.device, train=False)
+        a = acc[:n]
+        beta = 0
+        for e, T in zip(engines, tables):
+            p = e.params()
+            for f in flips:
+                xin = x[lo:hi]
+                if f:
+                    gather(xin, xf[:n], f)
+                    xin = xf[:n]
+                e.forward_group(B, T, xin, head="none")
+                ops.head_prob_accum(B.out["dec1"], p["out.weight"], p["out.bias"], a, flip=f, beta=beta)
+                beta = 1
+        if staged is not None:
+            staged.wait_labels(hi)
+        ops.prob_finalize(a, first.cfg.num_classes, scale, labels=rows(labels, lo, hi), ignore_index=ignore_index,
+                          tally=tl, per_sample=tuple(t[lo:hi] for t in per_sample) if per_sample is not None else None,
+                          labels_out=rows(labels_out, lo, hi), hist=hist, sample_hist=rows(sample_hist, lo, hi),
+                          proba_out=rows(proba_out, lo, hi))
 
 
 class StagedBatch:

@@ -397,6 +397,55 @@ def head_eval(x, w, b, labels, ignore_index, acc, counts, confusion, sample_acc=
              ptr(hist), ptr(sample_hist), stream_ptr())
 
 
+def head_prob_accum(x, w, b, acc, flip: int = 0, beta: int = 0):
+    """Head + softmax added into the probability accumulator acc (fp32 [n,d,h,w,16], contiguous, 16-byte aligned):
+    acc[n,d,h',w',c] = beta * acc + p_c, with h' / w' mirrored back when bit 1 / 2 of `flip` is set (the inverse of an
+    input flip). Classes >= K are written as 0 when beta = 0 and left alone when beta = 1 (spff_head_prob_accum)."""
+    s, ldx = _view(x, 32)
+    assert acc.dtype == torch.float32 and acc.is_contiguous() and acc.numel() == s.n * s.d * s.h * s.w * 16
+    call("spff_head_prob_accum", ptr(x), ldx, 32, ptr(w), ptr(b), w.shape[0], s, int(flip), int(beta), ptr(acc),
+         stream_ptr())
+
+
+def prob_finalize(acc, k: int, scale: float, labels=None, ignore_index: int = 255, tally=None, per_sample=None,
+                  labels_out=None, hist=None, sample_hist=None, proba_out=None):
+    """One pass over a spff_head_prob_accum accumulator acc (fp32 [n,d,h,w,16]): p̄ = scale * acc. Optional outputs:
+    labels_out (uint8 [n,d,h,w], the first arg-max of acc over classes < k), proba_out (fp16 [n,k,d,h,w], p̄), and with
+    labels (uint8 / int64 [n,d,h,w]) the tally (nll fp64 [1], count int64 [1], confusion int64 [k,k], +=) of
+    head_eval on p̄, per_sample rows (fp64 [n], int64 [n], int64 [n,k,k]), hist (int64 [k,2,T]) and sample_hist
+    (int64 [n,k,2,T]) of p̄ (spff_prob_finalize)."""
+    assert acc.dtype == torch.float32 and acc.dim() == 5 and acc.shape[-1] == 16 and acc.is_contiguous()
+    n, d, h, w, _ = acc.shape
+    vox = n * d * h * w
+    s = Shape(n, d, h, w)
+    lb = 0
+    if labels is not None:
+        assert labels.is_contiguous() and labels.numel() == vox
+        lb = _label_bytes(labels)
+    nll, cnt, conf = tally if tally is not None else (None, None, None)
+    per = per_sample if per_sample is not None else (None, None, None)
+    if per_sample is not None:
+        assert per[0].dtype == torch.float64 and per[0].numel() == n
+        assert per[1].dtype == torch.int64 and per[1].numel() == n
+        assert per[2].dtype == torch.int64 and per[2].is_contiguous() and per[2].numel() == n * k * k
+    if conf is not None:
+        assert conf.dtype == torch.int64 and conf.is_contiguous() and conf.numel() == k * k
+    bins = 0
+    if hist is not None:
+        bins = hist.shape[-1]
+        assert hist.dtype == torch.int64 and hist.is_contiguous() and tuple(hist.shape) == (k, 2, bins)
+        if sample_hist is not None:
+            assert sample_hist.dtype == torch.int64 and sample_hist.is_contiguous()
+            assert tuple(sample_hist.shape) == (n, k, 2, bins)
+    if labels_out is not None:
+        assert labels_out.dtype == torch.uint8 and labels_out.is_contiguous() and labels_out.numel() == vox
+    if proba_out is not None:
+        assert proba_out.dtype == torch.float16 and proba_out.is_contiguous() and tuple(proba_out.shape) == (n, k, d, h, w)
+    call("spff_prob_finalize", ptr(acc), int(k), s, float(scale), ptr(labels), lb, int(ignore_index), ptr(nll), ptr(cnt),
+         ptr(conf), *(ptr(t) for t in per), ptr(labels_out), int(bins), ptr(hist), ptr(sample_hist), ptr(proba_out),
+         stream_ptr())
+
+
 def scale_by_count(g, count, factor: float = 1.0):
     """g (fp32, contiguous) *= factor / count[0]  (0 when the count is 0)."""
     assert g.dtype == torch.float32 and g.is_contiguous() and count.dtype == torch.int64
