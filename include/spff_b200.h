@@ -291,6 +291,38 @@ int spff_prob_finalize(const float* acc, int k, spff_shape s, float scale, const
                        long long* sample_counts, long long* sample_confusion, uint8_t* labels_out, int bins,
                        long long* hist, long long* sample_hist, void* proba_out, void* stream);
 
+/* ---- uncertainty and calibration of the averaged softmax ----------------------------------------------------
+ * spff_head_prob_accum plus the expected-entropy plane: acc is written exactly as spff_head_prob_accum writes it, and
+ *   ent[n][d][h'][w'] = beta * ent[...] + H(p),   H(p) = -sum_{c<K} p_c log p_c (nats, fp32),
+ * at the same mirrored position. ent: fp32 [N,D,H,W], 4-byte aligned; one writer per element per call. */
+int spff_head_prob_accum_ent(const void* x, long long ldx, int cin, const float* w, const float* b, int k, spff_shape s,
+                             int flip, int beta, float* acc, float* ent, void* stream);
+
+/* Outputs of spff_prob_finalize_unc; every pointer may be NULL unless a rule below needs it. A voxel is counted when its
+ * label is in [0,K) and not ignore_index. Sums of real quantities (all but brier) are rounded per voxel to the fixed
+ * point 2^-24 and summed in integers, so they are bit-reproducible. */
+typedef struct spff_unc_out {
+  const float* ent;         /* expected-entropy plane of spff_head_prob_accum_ent (sum over passes), or NULL          */
+  void* entropy_out;        /* fp16 [N,D,H,W]: H[p̄] = -sum_c p̄_c log p̄_c (0 log 0 = 0), nats                         */
+  void* mi_out;             /* fp16 [N,D,H,W]: max(H[p̄] - scale * ent, 0), the mutual information; needs ent           */
+  long long* unc;           /* int64 [2] (+=): sum of H[p̄], sum of MI over all positions (MI: 0 without ent), 2^-24 */
+  long long* sample_unc;    /* int64 [N][2] (+=): the same per sample; needs unc                                      */
+  int cal_bins;             /* T in [2, 1024], when calib is given                                                    */
+  long long* calib;         /* int64 [3][T] (+=), needs labels: per confidence bin min(floor(conf * T), T - 1),        */
+                            /* conf = p̄_arg, the counted voxels, the correct ones (arg == label), sum conf in 2^-24   */
+  long long* sample_calib;  /* int64 [N][3][T]; given exactly when the per-sample tallies are (with calib)           */
+  double* brier;            /* (+=) sum over counted voxels of sum_c (p̄_c - [c == y])^2; given exactly when calib is */
+  double* sample_brier;     /* [N]; given exactly when sample_calib is                                               */
+} spff_unc_out;
+
+/* spff_prob_finalize (same arguments, same outputs, bit for bit) plus the uncertainty maps, sums and calibration
+ * histogram of `unc` (not NULL). */
+int spff_prob_finalize_unc(const float* acc, int k, spff_shape s, float scale, const void* labels, int label_bytes,
+                           int ignore_index, double* nll, long long* counts, long long* confusion, double* sample_acc,
+                           long long* sample_counts, long long* sample_confusion, uint8_t* labels_out, int bins,
+                           long long* hist, long long* sample_hist, void* proba_out, const spff_unc_out* unc,
+                           void* stream);
+
 /* ---- "3DUNet" control: Cicek3DUNet + depth adapter (models.py:718-777; config.py:283-311) ---------------
  * Its 3x3x3 convolutions, normalise + ReLU passes (slope 0), head and loss are the entry points above;
  * the ones below are what only this variant needs. */

@@ -1470,6 +1470,10 @@ head_eval_mma_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, const v
 // fp32 accumulator acc [n][d][h][w][16] at the position mirrored back by `flip` (1 = H, 2 = W). Within one (n, d)
 // plane the flip is a bijection, so every accumulator element has exactly one writer per launch: plain
 // load-add-store, deterministic. beta = 0 stores p (and 0 for classes >= K) without reading acc.
+// ENT: also ent [n][d][h'][w'] = beta * ent + H(p), the entropy of this pass's softmax, at the same mirrored position
+// (the expected-entropy plane of the mutual information). From the row's softmax statistics:
+// H = log(se) - sum_{c<K} e_c (v_c - mx) / se, the quad's partial sums reduced with two shuffles; lane t = 0 of the
+// row writes it (one writer per element per launch, as for acc).
 // ---------------------------------------------------------------------------------------------
 constexpr int kPaBlocksPerSm = 3;
 
@@ -1487,9 +1491,10 @@ __device__ __forceinline__ void hm_fetch_x(const __nv_bfloat16* __restrict__ x, 
   }
 }
 
+template <bool ENT>
 __global__ void __launch_bounds__(kHmWarps * 32, kPaBlocksPerSm)
 head_prob_accum_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, int K, int H, int W, long long dhw, int flip,
-                       int beta, float* __restrict__ acc) {
+                       int beta, float* __restrict__ acc, float* __restrict__ ent) {
   __shared__ __align__(16) __nv_bfloat16 xs[kHmWarps][16][kHmXPitch];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int g = lane >> 2, t = lane & 3;
@@ -1498,6 +1503,7 @@ head_prob_accum_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, int K
   const long long n = blockIdx.y;
   x += n * dhw * ldx;
   acc += n * dhw * kMaxK;
+  if constexpr (ENT) ent += n * dhw;
   const long long hw = static_cast<long long>(H) * W;
   const long long ntiles = (dhw + 15) / 16;
   const long long tstep = static_cast<long long>(gridDim.x) * kHmWarps;
@@ -1516,6 +1522,16 @@ head_prob_accum_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, int K
       float v[4], mx, e[4], se, ll;
       int cls[4], arg;
       hm_row_softmax(l, rr, t, K, -1, v, cls, mx, arg, e, se, ll);
+      float h_p = 0.f;
+      if constexpr (ENT) {
+        float ev = 0.f;
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+          if (cls[q] < K) ev = fmaf(e[q], v[q] - mx, ev);   // classes >= K: v = -inf, e = 0, and 0 * -inf is NaN
+#pragma unroll
+        for (int o = 1; o <= 2; o <<= 1) ev += __shfl_xor_sync(0xffffffffu, ev, o);
+        h_p = __logf(se) - __fdividef(ev, se);
+      }
       if (pos < dhw) {
         const long long plane = pos / hw, rem = pos - plane * hw;
         int hh = static_cast<int>(rem / W), ww = static_cast<int>(rem - static_cast<long long>(hh) * W);
@@ -1538,6 +1554,12 @@ head_prob_accum_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, int K
             dst[c0] = __fadd_rn(dst[c0], p.x);
           }
         }
+        if constexpr (ENT) {
+          if (t == 0) {
+            float* de = ent + plane * hw + static_cast<long long>(hh) * W + ww;
+            *de = beta ? __fadd_rn(*de, h_p) : h_p;
+          }
+        }
       }
     }
     __syncwarp();   // the tile is read before the next iteration overwrites it
@@ -1550,16 +1572,37 @@ head_prob_accum_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, int K
 // confusion[y][arg] (and, with HIST, every class's p̄_c to bin min(floor(p̄_c * T), T - 1) of hist[c][y == c ? 0 : 1]);
 // any other label counts only. Tallies are block-private in shared memory and flushed once per block, as in
 // head_eval_mma_kernel (the register bins too).
+// UNC (spff_prob_finalize_unc, outputs in `u`): per position H[p̄] = -sum_{c<K} p̄_c log p̄_c (0 log 0 = 0) and, with the
+// expected-entropy plane u.ent, MI = max(H[p̄] - scale * ent, 0); optional fp16 maps, and both rounded per position to
+// the 2^-24 fixed point and summed in integers (bit-reproducible whatever the launch order). With u.calib (needs labels),
+// every counted voxel (label in [0, K)) adds to confidence bin min(floor(conf * Tc), Tc - 1), conf = p̄_arg: one count,
+// one if arg == label, and conf in units of 2^-24; its Brier term sum_c (p̄_c - [c == y])^2 is reduced like the nll.
+// The top bin is counted in registers (a trained model puts most voxels there); the UNC tallies live in dynamic shared
+// memory behind the HIST histogram: ull [2] uncertainty sums, ull [Tc] confidence sums, u32 [2][Tc] counts, float [8].
 constexpr int kPfThreads = 256;
+constexpr float kFix24 = 16777216.f;   // 2^24
 
-template <typename LabelT, bool HIST>
+// the block's uncertainty sums into unc[2] and its sample's row of sample_unc [N][2]
+__device__ __forceinline__ void prob_finalize_flush_unc(const spff_unc_out& u, long long n, const unsigned long long* s_u) {
+  auto unc = reinterpret_cast<unsigned long long*>(u.unc);
+  auto sunc = reinterpret_cast<unsigned long long*>(u.sample_unc);
+  atomicAdd(unc, s_u[0]);
+  atomicAdd(unc + 1, s_u[1]);
+  if (sunc) {
+    atomicAdd(sunc + 2 * n, s_u[0]);
+    atomicAdd(sunc + 2 * n + 1, s_u[1]);
+  }
+}
+
+template <typename LabelT, bool HIST, bool UNC = false>
 __global__ void __launch_bounds__(kPfThreads)
 prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float scale, const void* __restrict__ labels,
                      int ignore_index, double* __restrict__ nll, unsigned long long* __restrict__ counts,
                      unsigned long long* __restrict__ confusion, double* __restrict__ sample_acc,
                      unsigned long long* __restrict__ sample_counts, unsigned long long* __restrict__ sample_confusion,
                      uint8_t* __restrict__ labels_out, __half* __restrict__ proba_out, int T,
-                     unsigned long long* __restrict__ hist, unsigned long long* __restrict__ sample_hist) {
+                     unsigned long long* __restrict__ hist, unsigned long long* __restrict__ sample_hist,
+                     spff_unc_out u) {
   __shared__ unsigned int s_conf[kMaxK * kMaxK];
   __shared__ float s_nll[kPfThreads / 32];
   __shared__ unsigned int s_cnt[kPfThreads / 32];
@@ -1571,6 +1614,21 @@ prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float 
   unsigned int hot_neg[kMaxK], hot_pos[kMaxK];   // HIST: bin 0 of negatives, bin T - 1 of positives
 #pragma unroll
   for (int c = 0; c < kMaxK; ++c) hot_neg[c] = hot_pos[c] = 0;
+  [[maybe_unused]] unsigned long long* s_u = nullptr;   // UNC: [0] sum H, [1] sum MI, [2, 2 + Tc) confidence sums
+  [[maybe_unused]] unsigned int* s_cal = nullptr;       // UNC: [0][Tc] counted, [1][Tc] correct
+  [[maybe_unused]] float* s_brier = nullptr;            // UNC: per warp
+  [[maybe_unused]] const int Tc = UNC && u.calib ? u.cal_bins : 0;
+  [[maybe_unused]] long long h_sum = 0, mi_sum = 0, top_conf = 0;
+  [[maybe_unused]] unsigned int top_cnt = 0, top_cor = 0;
+  [[maybe_unused]] float brier_sum = 0.f;
+  if constexpr (UNC) {
+    extern __shared__ unsigned long long s_dyn64[];
+    s_u = s_dyn64 + (HIST ? K * T : 0);
+    s_cal = reinterpret_cast<unsigned int*>(s_u + 2 + Tc);
+    s_brier = reinterpret_cast<float*>(s_cal + 2 * Tc);
+    for (int i = threadIdx.x; i < 2 + Tc; i += blockDim.x) s_u[i] = 0;
+    for (int i = threadIdx.x; i < 2 * Tc; i += blockDim.x) s_cal[i] = 0;
+  }
   __syncthreads();
   const long long n = blockIdx.y;
   acc += n * dhw * kMaxK;
@@ -1608,6 +1666,19 @@ prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float 
       for (int c = 0; c < kMaxK; ++c)
         if (c < K) proba_out[c * dhw + pos] = __float2half_rn(p[c]);
     }
+    if constexpr (UNC) {
+      float hb = 0.f;
+#pragma unroll
+      for (int c = 0; c < kMaxK; ++c)
+        if (c < K && p[c] > 0.f) hb = fmaf(-p[c], logf(p[c]), hb);
+      hb = fmaxf(hb, 0.f);   // p̄_c may exceed 1 by an ulp
+      float mi = 0.f;
+      if (u.ent) mi = fmaxf(hb - __fmul_rn(scale, __ldg(u.ent + n * dhw + pos)), 0.f);
+      if (u.entropy_out) static_cast<__half*>(u.entropy_out)[n * dhw + pos] = __float2half_rn(hb);
+      if (u.mi_out) static_cast<__half*>(u.mi_out)[n * dhw + pos] = __float2half_rn(mi);
+      h_sum += __float2ll_rn(hb * kFix24);
+      mi_sum += __float2ll_rn(mi * kFix24);
+    }
     if (lab_in) {
       const int lab = static_cast<int>(lab_in[pos]);
       if (lab != ignore_index) {
@@ -1633,6 +1704,62 @@ prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float 
                   atomicAdd(&s_hist[(c * 2 + (positive ? 0 : 1)) * T + bin], 1u);
               }
           }
+          if constexpr (UNC) {
+            if (Tc) {
+              const float conf = __fmul_rn(scale, mx);   // p̄_arg
+              const int bin = min(static_cast<int>(__fmul_rn(conf, static_cast<float>(Tc))), Tc - 1);
+              const long long cfix = __float2ll_rn(conf * kFix24);
+              const unsigned int correct = arg == lab ? 1u : 0u;
+              if (bin == Tc - 1) {
+                ++top_cnt;
+                top_cor += correct;
+                top_conf += cfix;
+              } else {
+                atomicAdd(&s_cal[bin], 1u);
+                if (correct) atomicAdd(&s_cal[Tc + bin], 1u);
+                atomicAdd(&s_u[2 + bin], static_cast<unsigned long long>(cfix));
+              }
+              float b = 0.f;
+#pragma unroll
+              for (int c = 0; c < kMaxK; ++c)
+                if (c < K) {
+                  const float dlt = c == lab ? p[c] - 1.f : p[c];
+                  b = fmaf(dlt, dlt, b);
+                }
+              brier_sum += b;
+            }
+          }
+        }
+      }
+    }
+  }
+  if constexpr (UNC) {
+    for (int o = 16; o > 0; o >>= 1) {
+      h_sum += __shfl_xor_sync(0xffffffffu, h_sum, o);
+      mi_sum += __shfl_xor_sync(0xffffffffu, mi_sum, o);
+    }
+    if (lane == 0) {
+      atomicAdd(&s_u[0], static_cast<unsigned long long>(h_sum));
+      atomicAdd(&s_u[1], static_cast<unsigned long long>(mi_sum));
+    }
+    if (!lab_in) {
+      __syncthreads();
+      if (threadIdx.x == 0 && u.unc) prob_finalize_flush_unc(u, n, s_u);
+      return;
+    }
+    if (Tc) {
+      for (int o = 16; o > 0; o >>= 1) {
+        top_cnt += __shfl_xor_sync(0xffffffffu, top_cnt, o);
+        top_cor += __shfl_xor_sync(0xffffffffu, top_cor, o);
+        top_conf += __shfl_xor_sync(0xffffffffu, top_conf, o);
+        brier_sum += __shfl_xor_sync(0xffffffffu, brier_sum, o);
+      }
+      if (lane == 0) {
+        s_brier[warp] = brier_sum;
+        if (top_cnt) {
+          atomicAdd(&s_cal[Tc - 1], top_cnt);
+          if (top_cor) atomicAdd(&s_cal[2 * Tc - 1], top_cor);
+          atomicAdd(&s_u[2 + Tc - 1], static_cast<unsigned long long>(top_conf));
         }
       }
     }
@@ -1687,6 +1814,28 @@ prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float 
         atomicAdd(hist + i, static_cast<unsigned long long>(s_hist[i]));
         if (sample_hist) atomicAdd(sample_hist + n * K * 2 * T + i, static_cast<unsigned long long>(s_hist[i]));
       }
+  if constexpr (UNC) {
+    if (threadIdx.x == 0) {
+      if (u.unc) prob_finalize_flush_unc(u, n, s_u);
+      if (Tc) {
+        double bt = 0;
+        for (int wv = 0; wv < kPfThreads / 32; ++wv) bt += s_brier[wv];
+        atomicAdd(u.brier, bt);
+        if (u.sample_brier) atomicAdd(u.sample_brier + n, bt);
+      }
+    }
+    auto cal = reinterpret_cast<unsigned long long*>(u.calib);
+    auto scal = reinterpret_cast<unsigned long long*>(u.sample_calib);
+    for (int i = threadIdx.x; i < Tc; i += blockDim.x) {
+      const unsigned long long v[3] = {s_cal[i], s_cal[Tc + i], s_u[2 + i]};
+#pragma unroll
+      for (int r = 0; r < 3; ++r)
+        if (v[r]) {
+          atomicAdd(cal + r * Tc + i, v[r]);
+          if (scal) atomicAdd(scal + (n * 3 + r) * Tc + i, v[r]);
+        }
+    }
+  }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1817,6 +1966,145 @@ int prob_finalize_hist_attr() {   // once per device, as head_eval_hist_attr
     attr_set[dev] = true;
   }
   return 0;
+}
+
+// spff_head_prob_accum (with_ent = false) and spff_head_prob_accum_ent (with_ent = true, ent required)
+int head_prob_accum_launch(const char* name, bool with_ent, const void* x, long long ldx, int cin, const float* w,
+                           const float* b, int k, spff_shape s, int flip, int beta, float* acc, float* ent, void* stream) {
+  SPFF_REQUIRE(x && w && b && acc && (ent || !with_ent), "%s: null pointer", name);
+  SPFF_REQUIRE(k >= 2 && k <= spff::kMaxK, "%s: classes must be in [2, %d] (got %d)", name, spff::kMaxK, k);
+  SPFF_REQUIRE(flip >= 0 && flip <= 3, "%s: flip is a bit set of 1 (H) and 2 (W) (got %d)", name, flip);
+  SPFF_REQUIRE(beta == 0 || beta == 1, "%s: beta must be 0 or 1 (got %d)", name, beta);
+  SPFF_REQUIRE((reinterpret_cast<uintptr_t>(acc) & 15) == 0, "%s: acc must be 16-byte aligned", name);
+  SPFF_REQUIRE(!with_ent || (reinterpret_cast<uintptr_t>(ent) & 3) == 0, "%s: ent must be 4-byte aligned", name);
+  SPFF_REQUIRE(ldx >= cin && ldx % 8 == 0, "%s: bad channel pitch", name);
+  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "%s: bad shape (N must be <= 65535)", name);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int e = spff::upload_head(w, b, k, cin, st);
+  if (e) return e;
+  const long long dhw = static_cast<long long>(s.d) * s.h * s.w;
+  // the grid of head_eval: one block row per sample, ~4 waves of resident blocks, no more blocks than warp tiles
+  const long long warp_tiles = ((dhw + 15) / 16 + spff::kHmWarps - 1) / spff::kHmWarps;
+  long long per = (4LL * spff::kPaBlocksPerSm * spff::num_sms() + s.n - 1) / s.n;
+  if (per > warp_tiles) per = warp_tiles;
+  if (per < 1) per = 1;
+  const dim3 grid(static_cast<unsigned>(per), s.n);
+  if (with_ent)
+    spff::head_prob_accum_kernel<true><<<grid, spff::kHmWarps * 32, 0, st>>>(static_cast<const bf16*>(x), ldx, k, s.h, s.w,
+                                                                            dhw, flip, beta, acc, ent);
+  else
+    spff::head_prob_accum_kernel<false><<<grid, spff::kHmWarps * 32, 0, st>>>(static_cast<const bf16*>(x), ldx, k, s.h, s.w,
+                                                                             dhw, flip, beta, acc, nullptr);
+  SPFF_CUDA(cudaGetLastError());
+  return 0;
+}
+
+constexpr int kUncMinBins = 2, kUncMaxBins = 1024;
+
+// dynamic shared memory of prob_finalize_kernel: the HIST histogram, then the UNC tallies (see the kernel)
+size_t prob_finalize_smem(bool unc, int k, int bins, int cal_bins) {
+  return sizeof(unsigned int) * k * 2 * bins +
+         (unc ? sizeof(unsigned long long) * (2 + cal_bins) + sizeof(unsigned int) * 2 * cal_bins +
+                    sizeof(float) * (spff::kPfThreads / 32)
+              : 0);
+}
+
+template <typename LabelT, bool HIST>
+int prob_finalize_unc_attr() {   // once per device, as head_eval_hist_attr
+  static bool attr_set[spff::kMaxDevices] = {};
+  const int dev = spff::current_device();
+  if (!attr_set[dev]) {
+    SPFF_CUDA(cudaFuncSetAttribute(spff::prob_finalize_kernel<LabelT, HIST, true>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   static_cast<int>(prob_finalize_smem(true, spff::kMaxK, HIST ? spff::kHeMaxBins : 0,
+                                                                       kUncMaxBins))));
+    attr_set[dev] = true;
+  }
+  return 0;
+}
+
+template <typename LabelT, bool HIST, bool UNC>
+int prob_finalize_run(dim3 grid, size_t smem, cudaStream_t st, const float* acc, int k, long long dhw, float scale,
+                      const void* labels, int ignore_index, double* nll, long long* counts, long long* confusion,
+                      double* sample_acc, long long* sample_counts, long long* sample_confusion, uint8_t* labels_out,
+                      int T, long long* hist, long long* sample_hist, void* proba_out, const spff_unc_out& u) {
+  if constexpr (HIST && !UNC) {
+    const int e = prob_finalize_hist_attr<LabelT>();
+    if (e) return e;
+  }
+  if constexpr (UNC) {
+    const int e = prob_finalize_unc_attr<LabelT, HIST>();
+    if (e) return e;
+  }
+  spff::prob_finalize_kernel<LabelT, HIST, UNC><<<grid, spff::kPfThreads, smem, st>>>(
+      acc, k, dhw, scale, labels, ignore_index, nll, reinterpret_cast<unsigned long long*>(counts),
+      reinterpret_cast<unsigned long long*>(confusion), sample_acc, reinterpret_cast<unsigned long long*>(sample_counts),
+      reinterpret_cast<unsigned long long*>(sample_confusion), labels_out, static_cast<__half*>(proba_out), T,
+      reinterpret_cast<unsigned long long*>(hist), reinterpret_cast<unsigned long long*>(sample_hist), u);
+  SPFF_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// spff_prob_finalize (with_unc = false) and spff_prob_finalize_unc (with_unc = true, unc required)
+int prob_finalize_launch(const char* name, bool with_unc, const float* acc, int k, spff_shape s, float scale,
+                         const void* labels, int label_bytes, int ignore_index, double* nll, long long* counts,
+                         long long* confusion, double* sample_acc, long long* sample_counts, long long* sample_confusion,
+                         uint8_t* labels_out, int bins, long long* hist, long long* sample_hist, void* proba_out,
+                         const spff_unc_out* unc, void* stream) {
+  SPFF_REQUIRE(acc, "%s: null accumulator", name);
+  SPFF_REQUIRE(k >= 2 && k <= spff::kMaxK, "%s: classes must be in [2, %d] (got %d)", name, spff::kMaxK, k);
+  SPFF_REQUIRE((reinterpret_cast<uintptr_t>(acc) & 15) == 0, "%s: acc must be 16-byte aligned", name);
+  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "%s: bad shape (N must be <= 65535)", name);
+  SPFF_REQUIRE(scale > 0.f, "%s: scale must be positive", name);
+  SPFF_REQUIRE(!labels || label_bytes == 1 || label_bytes == 8, "%s: labels must be uint8 or int64", name);
+  SPFF_REQUIRE(labels ? (nll && counts && confusion) : !(nll || counts || confusion || sample_acc || hist),
+               "%s: the tally (nll, counts, confusion) is given exactly when the labels are", name);
+  SPFF_REQUIRE((sample_acc != nullptr) == (sample_counts != nullptr) && (sample_acc != nullptr) == (sample_confusion != nullptr),
+               "%s: the per-sample arrays are given together or not at all", name);
+  SPFF_REQUIRE(!hist || (bins >= spff::kHeMinBins && bins <= spff::kHeMaxBins),
+               "%s: bins must be in [%d, %d] (got %d)", name, spff::kHeMinBins, spff::kHeMaxBins, bins);
+  SPFF_REQUIRE(hist || !sample_hist, "%s: sample_hist needs hist", name);
+  SPFF_REQUIRE(!hist || (sample_hist != nullptr) == (sample_acc != nullptr),
+               "%s: the per-sample histogram is given exactly when the per-sample tallies are", name);
+  spff_unc_out u = {};
+  if (with_unc) {
+    SPFF_REQUIRE(unc, "%s: null output struct", name);
+    u = *unc;
+    SPFF_REQUIRE(!u.calib || (u.cal_bins >= kUncMinBins && u.cal_bins <= kUncMaxBins),
+                 "%s: cal_bins must be in [%d, %d] (got %d)", name, kUncMinBins, kUncMaxBins, u.cal_bins);
+    SPFF_REQUIRE(!u.calib || labels, "%s: calib needs labels", name);
+    SPFF_REQUIRE(!u.sample_calib || (u.calib && sample_acc), "%s: sample_calib needs calib and the per-sample tallies",
+                 name);
+    SPFF_REQUIRE(!(u.calib && sample_acc) || u.sample_calib,
+                 "%s: with calib, sample_calib is given exactly when the per-sample tallies are", name);
+    SPFF_REQUIRE((u.brier != nullptr) == (u.calib != nullptr), "%s: brier is given exactly when calib is", name);
+    SPFF_REQUIRE((u.sample_brier != nullptr) == (u.sample_calib != nullptr),
+                 "%s: sample_brier is given exactly when sample_calib is", name);
+    SPFF_REQUIRE(!u.mi_out || u.ent, "%s: mi_out needs ent", name);
+    SPFF_REQUIRE(!u.sample_unc || u.unc, "%s: sample_unc needs unc", name);
+    SPFF_REQUIRE((reinterpret_cast<uintptr_t>(u.ent) & 3) == 0, "%s: ent must be 4-byte aligned", name);
+    if (!u.calib) u.cal_bins = 0;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long dhw = static_cast<long long>(s.d) * s.h * s.w;
+  const long long blocks_needed = (dhw + spff::kPfThreads - 1) / spff::kPfThreads;
+  long long per = (16LL * spff::num_sms() + s.n - 1) / s.n;   // ~2 waves of 8 resident blocks per SM
+  if (per > blocks_needed) per = blocks_needed;
+  if (per < 1) per = 1;
+  const dim3 grid(static_cast<unsigned>(per), s.n);
+  const int T = hist ? bins : 0;
+  const size_t smem = prob_finalize_smem(with_unc, k, T, u.cal_bins);
+  const bool wide = label_bytes == 8;
+#define SPFF_PF_RUN(L, H, U)                                                                                              \
+  prob_finalize_run<L, H, U>(grid, smem, st, acc, k, dhw, scale, labels, ignore_index, nll, counts, confusion, sample_acc, \
+                             sample_counts, sample_confusion, labels_out, T, hist, sample_hist, proba_out, u)
+  if (!with_unc) {
+    if (!hist) return wide ? SPFF_PF_RUN(long long, false, false) : SPFF_PF_RUN(uint8_t, false, false);
+    return wide ? SPFF_PF_RUN(long long, true, false) : SPFF_PF_RUN(uint8_t, true, false);
+  }
+  if (!hist) return wide ? SPFF_PF_RUN(long long, false, true) : SPFF_PF_RUN(uint8_t, false, true);
+  return wide ? SPFF_PF_RUN(long long, true, true) : SPFF_PF_RUN(uint8_t, true, true);
+#undef SPFF_PF_RUN
 }
 
 }  // namespace
@@ -2073,27 +2361,13 @@ int spff_head_eval_hist(const void* x, long long ldx, int cin, const float* w, c
 int spff_head_prob_accum(const void* x, long long ldx, int cin, const float* w, const float* b, int k, spff_shape s,
                          int flip, int beta, float* acc, void* stream) {
   SPFF_ENTRY_CHECK();
-  SPFF_REQUIRE(x && w && b && acc, "head_prob_accum: null pointer");
-  SPFF_REQUIRE(k >= 2 && k <= spff::kMaxK, "head_prob_accum: classes must be in [2, %d] (got %d)", spff::kMaxK, k);
-  SPFF_REQUIRE(flip >= 0 && flip <= 3, "head_prob_accum: flip is a bit set of 1 (H) and 2 (W) (got %d)", flip);
-  SPFF_REQUIRE(beta == 0 || beta == 1, "head_prob_accum: beta must be 0 or 1 (got %d)", beta);
-  SPFF_REQUIRE((reinterpret_cast<uintptr_t>(acc) & 15) == 0, "head_prob_accum: acc must be 16-byte aligned");
-  SPFF_REQUIRE(ldx >= cin && ldx % 8 == 0, "head_prob_accum: bad channel pitch");
-  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "head_prob_accum: bad shape (N must be <= 65535)");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int e = spff::upload_head(w, b, k, cin, st);
-  if (e) return e;
-  const long long dhw = static_cast<long long>(s.d) * s.h * s.w;
-  // the grid of head_eval: one block row per sample, ~4 waves of resident blocks, no more blocks than warp tiles
-  const long long warp_tiles = ((dhw + 15) / 16 + spff::kHmWarps - 1) / spff::kHmWarps;
-  long long per = (4LL * spff::kPaBlocksPerSm * spff::num_sms() + s.n - 1) / s.n;
-  if (per > warp_tiles) per = warp_tiles;
-  if (per < 1) per = 1;
-  const dim3 grid(static_cast<unsigned>(per), s.n);
-  spff::head_prob_accum_kernel<<<grid, spff::kHmWarps * 32, 0, st>>>(static_cast<const bf16*>(x), ldx, k, s.h, s.w, dhw,
-                                                                      flip, beta, acc);
-  SPFF_CUDA(cudaGetLastError());
-  return 0;
+  return head_prob_accum_launch("head_prob_accum", false, x, ldx, cin, w, b, k, s, flip, beta, acc, nullptr, stream);
+}
+
+int spff_head_prob_accum_ent(const void* x, long long ldx, int cin, const float* w, const float* b, int k, spff_shape s,
+                             int flip, int beta, float* acc, float* ent, void* stream) {
+  SPFF_ENTRY_CHECK();
+  return head_prob_accum_launch("head_prob_accum_ent", true, x, ldx, cin, w, b, k, s, flip, beta, acc, ent, stream);
 }
 
 int spff_prob_finalize(const float* acc, int k, spff_shape s, float scale, const void* labels, int label_bytes,
@@ -2101,55 +2375,20 @@ int spff_prob_finalize(const float* acc, int k, spff_shape s, float scale, const
                        long long* sample_counts, long long* sample_confusion, uint8_t* labels_out, int bins,
                        long long* hist, long long* sample_hist, void* proba_out, void* stream) {
   SPFF_ENTRY_CHECK();
-  SPFF_REQUIRE(acc, "prob_finalize: null accumulator");
-  SPFF_REQUIRE(k >= 2 && k <= spff::kMaxK, "prob_finalize: classes must be in [2, %d] (got %d)", spff::kMaxK, k);
-  SPFF_REQUIRE((reinterpret_cast<uintptr_t>(acc) & 15) == 0, "prob_finalize: acc must be 16-byte aligned");
-  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "prob_finalize: bad shape (N must be <= 65535)");
-  SPFF_REQUIRE(scale > 0.f, "prob_finalize: scale must be positive");
-  SPFF_REQUIRE(!labels || label_bytes == 1 || label_bytes == 8, "prob_finalize: labels must be uint8 or int64");
-  SPFF_REQUIRE(labels ? (nll && counts && confusion) : !(nll || counts || confusion || sample_acc || hist),
-               "prob_finalize: the tally (nll, counts, confusion) is given exactly when the labels are");
-  SPFF_REQUIRE((sample_acc != nullptr) == (sample_counts != nullptr) && (sample_acc != nullptr) == (sample_confusion != nullptr),
-               "prob_finalize: the per-sample arrays are given together or not at all");
-  SPFF_REQUIRE(!hist || (bins >= spff::kHeMinBins && bins <= spff::kHeMaxBins),
-               "prob_finalize: bins must be in [%d, %d] (got %d)", spff::kHeMinBins, spff::kHeMaxBins, bins);
-  SPFF_REQUIRE(hist || !sample_hist, "prob_finalize: sample_hist needs hist");
-  SPFF_REQUIRE(!hist || (sample_hist != nullptr) == (sample_acc != nullptr),
-               "prob_finalize: the per-sample histogram is given exactly when the per-sample tallies are");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const long long dhw = static_cast<long long>(s.d) * s.h * s.w;
-  const long long blocks_needed = (dhw + spff::kPfThreads - 1) / spff::kPfThreads;
-  long long per = (16LL * spff::num_sms() + s.n - 1) / s.n;   // ~2 waves of 8 resident blocks per SM
-  if (per > blocks_needed) per = blocks_needed;
-  if (per < 1) per = 1;
-  const dim3 grid(static_cast<unsigned>(per), s.n);
-  auto cnt = reinterpret_cast<unsigned long long*>(counts);
-  auto conf = reinterpret_cast<unsigned long long*>(confusion);
-  auto scnt = reinterpret_cast<unsigned long long*>(sample_counts);
-  auto sconf = reinterpret_cast<unsigned long long*>(sample_confusion);
-  auto hst = reinterpret_cast<unsigned long long*>(hist);
-  auto shst = reinterpret_cast<unsigned long long*>(sample_hist);
-  auto pout = static_cast<__half*>(proba_out);
-  const size_t hist_smem = hist ? sizeof(unsigned int) * k * 2 * bins : 0;
-  if (hist) {
-    const int e = label_bytes == 1 ? prob_finalize_hist_attr<uint8_t>() : prob_finalize_hist_attr<long long>();
-    if (e) return e;
-  }
-  const int T = hist ? bins : 0;
-  if (label_bytes != 8 && !hist)
-    spff::prob_finalize_kernel<uint8_t, false><<<grid, spff::kPfThreads, 0, st>>>(
-        acc, k, dhw, scale, labels, ignore_index, nll, cnt, conf, sample_acc, scnt, sconf, labels_out, pout, T, hst, shst);
-  else if (!hist)
-    spff::prob_finalize_kernel<long long, false><<<grid, spff::kPfThreads, 0, st>>>(
-        acc, k, dhw, scale, labels, ignore_index, nll, cnt, conf, sample_acc, scnt, sconf, labels_out, pout, T, hst, shst);
-  else if (label_bytes == 1)
-    spff::prob_finalize_kernel<uint8_t, true><<<grid, spff::kPfThreads, hist_smem, st>>>(
-        acc, k, dhw, scale, labels, ignore_index, nll, cnt, conf, sample_acc, scnt, sconf, labels_out, pout, T, hst, shst);
-  else
-    spff::prob_finalize_kernel<long long, true><<<grid, spff::kPfThreads, hist_smem, st>>>(
-        acc, k, dhw, scale, labels, ignore_index, nll, cnt, conf, sample_acc, scnt, sconf, labels_out, pout, T, hst, shst);
-  SPFF_CUDA(cudaGetLastError());
-  return 0;
+  return prob_finalize_launch("prob_finalize", false, acc, k, s, scale, labels, label_bytes, ignore_index, nll, counts,
+                              confusion, sample_acc, sample_counts, sample_confusion, labels_out, bins, hist, sample_hist,
+                              proba_out, nullptr, stream);
+}
+
+int spff_prob_finalize_unc(const float* acc, int k, spff_shape s, float scale, const void* labels, int label_bytes,
+                           int ignore_index, double* nll, long long* counts, long long* confusion, double* sample_acc,
+                           long long* sample_counts, long long* sample_confusion, uint8_t* labels_out, int bins,
+                           long long* hist, long long* sample_hist, void* proba_out, const spff_unc_out* unc,
+                           void* stream) {
+  SPFF_ENTRY_CHECK();
+  return prob_finalize_launch("prob_finalize_unc", true, acc, k, s, scale, labels, label_bytes, ignore_index, nll, counts,
+                              confusion, sample_acc, sample_counts, sample_confusion, labels_out, bins, hist, sample_hist,
+                              proba_out, unc, stream);
 }
 
 int spff_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr,

@@ -263,6 +263,85 @@ def sample_curves(per_sample_hist) -> List[tuple]:
     return out
 
 
+FIX24 = 2.0 ** -24   # unit of the fixed-point sums of the ensemble's confidence and uncertainty
+
+
+def calibration_from_hist(calib, brier_sum=None, ece_bins: int = 15, unc=None, voxels=None) -> dict:
+    """Calibration of the top-label confidence from the histogram of `SpctEnsemble.eval_step(calibration=T)` /
+    `evaluate` (int64 [3,T]: per confidence bin b, i.e. conf in [b/T, (b+1)/T), the counted voxels n_b, the correct
+    ones k_b (arg-max == label) and the summed confidence s_b in units of 2^-24; conf = max_c p̄_c).
+
+    - `ece` / `mce`: expected / maximum calibration error over `ece_bins` equal-width bins, sum_B |k_B - s_B| / N and
+      max_B |k_B / n_B - s_B / n_B| over non-empty B. The fine bins carry the confidence sum, so merging T / ece_bins
+      of them is exact; T % ece_bins must be 0 (ValueError otherwise). calibration=960 gives the standard 15-bin ECE.
+    - `reliability`: {"confidence", "accuracy", "count"} per coarse bin (NaN for empty bins).
+    - `brier`: brier_sum / N, the mean over counted voxels of sum_c (p̄_c - [c == y])^2 (NaN without brier_sum).
+    - `error_auroc` / `error_ap` / `error_auroc_tie_bound`: detecting errors (positives) by 1 - confidence, as
+      curves_from_hist ranks (equal to sklearn's roc_auc_score / average_precision_score with the reversed bin index as
+      the score; voxels of one bin are ties).
+    - `coverage` / `risk` / `aurc`: keeping the voxels of bins >= i (most confident first) covers C_i / N of them at
+      risk E_i / C_i (errors / kept), points in order of rising coverage for the non-empty prefixes; `aurc` is the
+      trapezoid area under them from coverage 0, the first point's risk held down to 0.
+    - `mean_entropy` / `mean_mutual_info`: the uncertainty sums `unc` (int64 [2], 2^-24 nats) over `voxels` positions
+      (NaN without them).
+    - `counted`, `errors`, `ece_bins`: N, its errors and the number of ECE bins.
+
+    NaN rules: with no counted voxel every statistic above is NaN; with no error error_auroc is NaN (and error_ap, no
+    positive); with no correct voxel error_auroc is NaN and error_ap is 1."""
+    h = np.asarray(_as_numpy(calib), dtype=np.float64)
+    if h.ndim != 2 or h.shape[0] != 3:
+        raise ValueError(f"expected a [3,T] calibration histogram, got {h.shape}")
+    bins = h.shape[1]
+    if ece_bins < 1 or bins % ece_bins:
+        raise ValueError(f"the {bins} confidence bins cannot be merged exactly into {ece_bins} (T % ece_bins != 0)")
+    cnt, cor, csum = h[0], h[1], h[2] * FIX24
+    n = cnt.sum()
+    err = cnt - cor
+    g = bins // ece_bins
+    cn, kn, sn = (v.reshape(ece_bins, g).sum(1) for v in (cnt, cor, csum))
+    with np.errstate(invalid="ignore", divide="ignore"):
+        acc_b, conf_b = kn / cn, sn / cn
+        gap = np.abs(kn - sn)
+        ece = gap.sum() / n if n else float("nan")
+        mce = float(np.max(np.abs(acc_b - conf_b)[cn > 0])) if n else float("nan")
+        brier = float(brier_sum) / n if (brier_sum is not None and n) else float("nan")
+    # error detection: score 1 - confidence, i.e. the bins in reverse order
+    auroc, ap, bound, _, _ = _ranking(np.stack([err[::-1], cor[::-1]])[None])
+    kept = np.cumsum(cnt[::-1])
+    kept_err = np.cumsum(err[::-1])
+    nz = kept > 0
+    coverage = kept[nz] / n if n else np.zeros(0)
+    risk = kept_err[nz] / kept[nz]
+    if n:
+        aurc = float(risk[0] * coverage[0] + np.sum(0.5 * (risk[1:] + risk[:-1]) * np.diff(coverage)))
+    else:
+        aurc = float("nan")
+    mean_ent = mean_mi = float("nan")
+    if unc is not None and voxels:
+        u = np.asarray(_as_numpy(unc), dtype=np.float64) * FIX24
+        mean_ent, mean_mi = float(u[0] / voxels), float(u[1] / voxels)
+    return {"ece": float(ece), "mce": mce, "reliability": {"confidence": conf_b, "accuracy": acc_b, "count": cn},
+            "brier": brier, "error_auroc": float(auroc[0]), "error_ap": float(ap[0]),
+            "error_auroc_tie_bound": float(bound[0]), "coverage": coverage, "risk": risk, "aurc": aurc,
+            "mean_entropy": mean_ent, "mean_mutual_info": mean_mi, "counted": int(n), "errors": int(err.sum()),
+            "ece_bins": ece_bins}
+
+
+def sample_calibration(per_sample_calib, per_sample_brier=None, ece_bins: int = 15) -> List[tuple]:
+    """Per-case calibration: one (ece, brier, error_auroc) per sample from the per-sample histograms of
+    `SpctEnsemble.eval_step(calibration=T, per_sample=True)` ([B,3,T]) and its per-sample Brier sums ([B]), as
+    calibration_from_hist defines them. The calibration counterpart of `sample_curves`."""
+    h = _as_numpy(per_sample_calib)
+    if h.ndim != 3 or h.shape[1] != 3:
+        raise ValueError(f"expected a [B,3,T] calibration histogram, got {h.shape}")
+    b = _as_numpy(per_sample_brier) if per_sample_brier is not None else [None] * len(h)
+    out = []
+    for row, br in zip(h, b):
+        c = calibration_from_hist(row, br, ece_bins)
+        out.append((c["ece"], c["brier"], c["error_auroc"]))
+    return out
+
+
 def per_class_metrics_2d(preds, labels, num_classes, smooth=1e-6, ignore_index=None):
     """2-D twin (helpers.py:728-779): same counting rules on [B,K,H,W] logits."""
     return per_class_metrics_3d(preds, labels, num_classes, smooth, ignore_index)

@@ -37,8 +37,8 @@ from spff_b200.engine import LossTally, NetConfig, SpffEngine, StagedBatch, run_
 from spff_b200.sched import PlateauLR
 
 from .config import BEST_LR, IGNORE_INDEX, NUM_CLASSES, NUM_FRAMES
-from .helpers import (LOSS_REGISTRY, ce_plus_macro_dice_loss, curves_from_hist, metrics_from_confusion,
-                      per_class_metrics_2d, per_class_metrics_3d)
+from .helpers import (LOSS_REGISTRY, calibration_from_hist, ce_plus_macro_dice_loss, curves_from_hist,
+                      metrics_from_confusion, per_class_metrics_2d, per_class_metrics_3d)
 
 LOG_PER_CLASS = os.getenv("LOG_PER_CLASS", "1") == "1"
 # samples per group of the engine's schedule (activations of one group live at a time in fit_step)
@@ -741,14 +741,39 @@ def _curve_buffers(curves, k: int, bsz: int, per_sample: bool, dev):
     return hist, sample_hist
 
 
-def _evaluate(k: int, dev, loss_fn, batches, step, curves: Optional[int] = None):
+def _calib_buffers(calibration, dev):
+    """[3,T] int64 confidence histogram for `eval_step(calibration=...)`, or None: `calibration` is a bin count T (fresh
+    zeros) or a contiguous int64 [3,T] histogram on `dev` to accumulate into, T in [2, 1024]."""
+    if calibration is None:
+        return None
+    if torch.is_tensor(calibration):
+        calib = calibration
+        if calib.dtype != torch.int64 or calib.dim() != 2 or calib.shape[0] != 3 or not calib.is_contiguous() \
+                or calib.device != torch.device(dev):
+            raise ValueError(f"calibration must be a contiguous int64 [3,T] histogram on {dev}, got {calib.dtype} "
+                             f"{tuple(calib.shape)} on {calib.device}")
+    else:
+        calib = torch.zeros(3, int(calibration), dtype=torch.int64, device=dev)
+    if not 2 <= calib.shape[1] <= 1024:
+        raise ValueError(f"calibration: the bin count must be in [2, 1024], got {calib.shape[1]}")
+    return calib
+
+
+def _evaluate(k: int, dev, loss_fn, batches, step, curves: Optional[int] = None, calibration: Optional[int] = None):
     """Shared driver of the `evaluate` methods: one tally (and, with `curves` = T, one [K,2,T] softmax histogram) over
     the batches, ONE all-reduce of the tally (plus the voxel count and the histogram) under data parallelism, ONE
-    device->host copy at the end. k classes, `dev` the device of the tallies, loss_fn(tally) -> device scalar."""
+    device->host copy at the end. k classes, `dev` the device of the tallies, loss_fn(tally) -> device scalar.
+    `calibration` = T (ensembles only: step(batch, tally, hist, cal) takes a fourth argument, the dict of
+    SpctEnsemble.eval_step's calibration outputs) adds a [3,T] confidence histogram, the Brier sum and the uncertainty
+    sums to the all-reduce and the copy, and "calibration" (helpers.calibration_from_hist) to the result."""
     tally, voxels = None, 0
     hist = _curve_buffers(curves, k, 0, False, dev)[0]
+    cal = None
+    if calibration is not None:
+        cal = {"calib": _calib_buffers(calibration, dev), "brier": torch.zeros(1, dtype=torch.float64, device=dev),
+               "unc": torch.zeros(2, dtype=torch.int64, device=dev)}
     for batch in batches:
-        tally = step(batch, tally, hist)["tally"]
+        tally = (step(batch, tally, hist) if cal is None else step(batch, tally, hist, cal))["tally"]
         voxels += _eval_voxels(batch)
     if tally is None:   # a rank without batches still joins the all-reduce
         tally = LossTally(k, dev)
@@ -758,9 +783,13 @@ def _evaluate(k: int, dev, loss_fn, batches, step, curves: Optional[int] = None)
         torch.distributed.all_reduce(vox)
         if hist is not None:
             dp.allreduce_hist(hist)
+        if cal is not None:
+            dp.allreduce_calibration(cal["calib"], cal["brier"], cal["unc"])
     loss = loss_fn(tally).double().reshape(1)
-    # one copy: [nll (fp64 bits), count, confusion..., voxels, loss (fp64 bits), histogram...]
+    # one copy: [nll (fp64 bits), count, confusion..., voxels, loss (fp64 bits), histogram..., calibration...]
     parts = [tally._buf, vox, loss.view(torch.int64)] + ([hist.view(-1)] if hist is not None else [])
+    if cal is not None:
+        parts += [cal["calib"].view(-1), cal["brier"].view(torch.int64), cal["unc"]]
     host = torch.cat(parts).cpu()
     cm = host[2:2 + k * k].view(k, k).numpy()
     voxels = int(host[2 + k * k])
@@ -768,7 +797,16 @@ def _evaluate(k: int, dev, loss_fn, batches, step, curves: Optional[int] = None)
            "tally": tally, "voxels": voxels}
     if hist is not None:
         out["hist"] = hist
-        out["curves"] = curves_from_hist(host[4 + k * k:].view(hist.shape).numpy())
+        out["curves"] = curves_from_hist(host[4 + k * k:4 + k * k + hist.numel()].view(hist.shape).numpy())
+    if cal is not None:
+        c0 = 4 + k * k + (hist.numel() if hist is not None else 0)
+        ch = host[c0:c0 + cal["calib"].numel()].view(cal["calib"].shape)
+        rest = host[c0 + ch.numel():]
+        out["calib"] = cal["calib"]
+        bins = ch.shape[1]
+        out["calibration"] = calibration_from_hist(ch.numpy(), float(rest[:1].view(torch.float64)[0]),
+                                                   ece_bins=15 if bins % 15 == 0 else bins, unc=rest[1:3].numpy(),
+                                                   voxels=voxels)
     return out
 
 
@@ -1251,7 +1289,12 @@ class SpctEnsemble:
     Every pass runs the member on the (flipped) input and adds its softmax, mirrored back, into an fp32 accumulator of
     one sample group; p̄ = the mean over members x flips. `predict_labels` / `predict_proba` give its arg-max / p̄,
     `eval_step` / `evaluate` the loss, metrics and curves of BaseLitModel's on p̄: the loss is ce_plus_macro_dice_loss on
-    the averaged probabilities (CE of p̄ + 0.5 * (1 - hard macro Dice of its arg-max))."""
+    the averaged probabilities (CE of p̄ + 0.5 * (1 - hard macro Dice of its arg-max)).
+
+    `predict_uncertainty` gives per-voxel uncertainty maps (the predictive entropy H[p̄] and the mutual information
+    between prediction and pass, H[p̄] - mean over passes of H[p]), and `eval_step` / `evaluate(calibration=T)` the
+    calibration statistics of p̄ (helpers.calibration_from_hist). For one model, use SpctEnsemble([lit]): its MI is 0
+    and its entropy and calibration are the single model's."""
 
     def __init__(self, members, tta: Optional[str] = None):
         if tta not in (None, "flip"):
@@ -1320,10 +1363,39 @@ class SpctEnsemble:
         return out
 
     @torch.no_grad()
+    def predict_uncertainty(self, x, sample_group: Optional[int] = None) -> Dict[str, torch.Tensor]:
+        """One pass over members x flips: {"labels": uint8 [B,F,H,W] (predict_labels), "entropy": float16 [B,F,H,W]
+        (H[p̄] = -sum_c p̄_c log p̄_c, nats), "mutual_info": float16 [B,F,H,W] (H[p̄] - mean over passes of H[p], clamped
+        at 0: the members' / flips' disagreement), "case_entropy", "case_mutual_info": float64 [B] (their means over
+        the voxels of each case, from sums of the per-voxel values rounded to 2^-24)}."""
+        x = self._images(x)
+        engines = self._engines(x.shape[2])
+        b, _, d, h, w = x.shape
+        dev = self.device
+        labels = torch.empty(b, d, h, w, dtype=torch.uint8, device=dev)
+        ent = torch.empty(b, d, h, w, dtype=torch.float16, device=dev)
+        mi = torch.empty_like(ent)
+        sums = torch.zeros(2, dtype=torch.int64, device=dev)
+        rows = torch.zeros(b, 2, dtype=torch.int64, device=dev)
+        run_ensemble(engines, x.to(dev), self.flips, sample_group or self.cores[0].sample_group, labels_out=labels,
+                     entropy_out=ent, mi_out=mi, unc=sums, sample_unc=rows)
+        case = rows.double() * (2.0 ** -24) / (d * h * w)
+        return {"labels": labels, "entropy": ent, "mutual_info": mi, "case_entropy": case[:, 0],
+                "case_mutual_info": case[:, 1]}
+
+    @torch.no_grad()
     def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False,
-                  sample_group: Optional[int] = None, curves=None):
+                  sample_group: Optional[int] = None, curves=None, calibration=None):
         """BaseLitModel.eval_step for the ensemble: the tally, per-sample rows, arg-max map and histograms of the
-        averaged softmax p̄ (same arguments, batch forms and return dict)."""
+        averaged softmax p̄ (same arguments, batch forms and return dict).
+
+        `calibration`: a bin count T in [2, 1024] (fresh zeros) or a contiguous int64 [3,T] histogram on the device to
+        accumulate into (as `curves`); adds "calib" ([3,T]: per confidence bin min(floor(conf * T), T - 1), conf = the
+        largest p̄_c, the counted voxels, the correct ones and the summed confidence in units of 2^-24), "brier" (fp64
+        [1], the summed Brier score) and "uncertainty" (int64 [2], the summed H[p̄] and mutual information in units of
+        2^-24 nats); with per_sample=True also "per_sample_calib" [B,3,T], "per_sample_brier" [B] and
+        "per_sample_uncertainty" (float64 [B,2], the mean H[p̄] and MI per case). helpers.calibration_from_hist /
+        sample_calibration turn them into ECE, reliability diagrams and error detection."""
         imgs, lbls = batch if isinstance(batch, (list, tuple)) else (batch["image"], batch["label"])
         imgs, lbls = self._images(imgs), _pick_first_if_seq(lbls)
         engines = self._engines(imgs.shape[2])
@@ -1347,16 +1419,50 @@ class SpctEnsemble:
                 torch.zeros(bsz, k, k, dtype=torch.int64, device=dev)) if per_sample else None
         labels = torch.empty(bsz, *imgs.shape[2:], dtype=torch.uint8, device=dev) if return_labels else None
         hist, sample_hist = _curve_buffers(curves, k, bsz, per_sample, dev)
+        cal = {}
+        if calibration is not None:
+            calib = _calib_buffers(calibration, dev)
+            bins = calib.shape[1]
+            cal = dict(calib=calib, brier=torch.zeros(1, dtype=torch.float64, device=dev),
+                       unc=torch.zeros(2, dtype=torch.int64, device=dev))
+            if per_sample:
+                cal.update(sample_calib=torch.zeros(bsz, 3, bins, dtype=torch.int64, device=dev),
+                           sample_brier=torch.zeros(bsz, dtype=torch.float64, device=dev),
+                           sample_unc=torch.zeros(bsz, 2, dtype=torch.int64, device=dev))
         run_ensemble(engines, imgs, self.flips, group, labels=lbls, tally=tally, ignore_index=IGNORE_INDEX,
-                     per_sample=rows, labels_out=labels, hist=hist, sample_hist=sample_hist, staged=staged)
-        return {"loss": tally.loss(), "tally": tally, "per_sample": rows, "labels": labels, "hist": hist,
-                "per_sample_hist": sample_hist}
+                     per_sample=rows, labels_out=labels, hist=hist, sample_hist=sample_hist, staged=staged,
+                     unc=cal.get("unc"), sample_unc=cal.get("sample_unc"), calib=cal.get("calib"),
+                     sample_calib=cal.get("sample_calib"), brier=cal.get("brier"), sample_brier=cal.get("sample_brier"))
+        out = {"loss": tally.loss(), "tally": tally, "per_sample": rows, "labels": labels, "hist": hist,
+               "per_sample_hist": sample_hist}
+        if calibration is not None:
+            out.update(calib=cal["calib"], brier=cal["brier"], uncertainty=cal["unc"])
+            if per_sample:
+                vox = imgs.shape[2] * imgs.shape[3] * imgs.shape[4]
+                out.update(per_sample_calib=cal["sample_calib"], per_sample_brier=cal["sample_brier"],
+                           per_sample_uncertainty=cal["sample_unc"].double() * (2.0 ** -24) / vox)
+        return out
 
     @torch.no_grad()
-    def evaluate(self, batches, sample_group: Optional[int] = None, curves: Optional[int] = None):
-        """BaseLitModel.evaluate for the ensemble: {"loss", "metrics", "tally", "voxels"} (+ "hist", "curves")."""
-        return _evaluate(self.num_classes, self.device, lambda t: t.loss(), batches,
-                         lambda b, t, h: self.eval_step(b, tally=t, sample_group=sample_group, curves=h), curves)
+    def evaluate(self, batches, sample_group: Optional[int] = None, curves: Optional[int] = None,
+                 calibration: Optional[int] = None):
+        """BaseLitModel.evaluate for the ensemble: {"loss", "metrics", "tally", "voxels"} (+ "hist", "curves"). With
+        `calibration` = T confidence bins also "calib" (int64 [3,T] on the device) and "calibration"
+        (helpers.calibration_from_hist: ECE / MCE, reliability diagram, Brier score, error-detection AUROC / AP,
+        risk-coverage and the mean entropy and mutual information). The ECE is over 15 bins when T is a multiple of 15
+        and over the T bins otherwise ("ece_bins" says which): calibration=960 gives the standard 15-bin ECE exactly
+        (960 = 15 * 64)."""
+        k, dev = self.num_classes, self.device
+        if calibration is None:
+            return _evaluate(k, dev, lambda t: t.loss(), batches,
+                             lambda b, t, h: self.eval_step(b, tally=t, sample_group=sample_group, curves=h), curves)
+
+        def step(b, t, h, cal):
+            out = self.eval_step(b, tally=t, sample_group=sample_group, curves=h, calibration=cal["calib"])
+            cal["brier"] += out["brier"]
+            cal["unc"] += out["uncertainty"]
+            return out
+        return _evaluate(k, dev, lambda t: t.loss(), batches, step, curves, calibration)
 
 
 # Model families outside the hot path (UNETR / SwinUNETR wrappers, R2U-Net, ResUNet++, their helper blocks and losses:

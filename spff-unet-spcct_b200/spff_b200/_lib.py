@@ -21,6 +21,15 @@ class Shape(Structure):
     _fields_ = [("n", c_int), ("d", c_int), ("h", c_int), ("w", c_int)]
 
 
+class UncOut(Structure):
+    """spff_unc_out: the uncertainty / calibration outputs of spff_prob_finalize_unc (device pointers, NULL = not
+    wanted)."""
+
+    _fields_ = [("ent", c_void_p), ("entropy_out", c_void_p), ("mi_out", c_void_p), ("unc", c_void_p),
+                ("sample_unc", c_void_p), ("cal_bins", c_int), ("calib", c_void_p), ("sample_calib", c_void_p),
+                ("brier", c_void_p), ("sample_brier", c_void_p)]
+
+
 def _load() -> ctypes.CDLL:
     if not os.path.exists(LIB_PATH):
         raise RuntimeError(
@@ -90,6 +99,9 @@ _PROTOTYPES = {
                             _P, _P],
     "spff_head_prob_accum": [_P, _LL, c_int, _P, _P, c_int, Shape, c_int, c_int, _P, _P],
     "spff_prob_finalize": [_P, c_int, Shape, c_float, _P, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, c_int, _P, _P, _P, _P],
+    "spff_head_prob_accum_ent": [_P, _LL, c_int, _P, _P, c_int, Shape, c_int, c_int, _P, _P, _P],
+    "spff_prob_finalize_unc": [_P, c_int, Shape, c_float, _P, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, c_int, _P, _P, _P,
+                               POINTER(UncOut), _P],
     "spff_count_valid": [_P, c_int, _LL, c_int, _P, _P],
     "spff_scale_by_count": [_P, _LL, _P, c_float, _P],
     "spff_loss_from_tally": [_P, _P, _P, c_int, c_double, _P, _P],

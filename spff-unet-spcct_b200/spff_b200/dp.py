@@ -53,6 +53,15 @@ def allreduce_hist(hist: torch.Tensor) -> None:
         dist.all_reduce(hist, op=dist.ReduceOp.SUM)
 
 
+def allreduce_calibration(calib: torch.Tensor, brier: torch.Tensor, unc: torch.Tensor) -> None:
+    """Sum the ensemble's calibration statistics over ranks in place: the [3,T] int64 confidence histogram, the fp64
+    Brier sum and the int64 [2] uncertainty sums (fixed point, so the sum does not depend on the rank order)."""
+    _, n = world()
+    if n > 1:
+        for t in (calib, brier, unc):
+            dist.all_reduce(t, op=dist.ReduceOp.SUM)
+
+
 def shard_range(total: int, rank: int | None = None, world_size: int | None = None) -> Tuple[int, int]:
     """[lo, hi) of the `total` independent units (slices / sliding-window tiles = whole z-slices)
     owned by `rank`: contiguous, sizes differ by at most one. No collective is involved."""

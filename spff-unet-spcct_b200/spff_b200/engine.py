@@ -683,6 +683,13 @@ class SpffEngine:
 # per sample, in fit_group's units, of run_ensemble beside the inference buffers: the fp32 probability accumulator
 # (16 classes x 4 B = 64 B per position, one unit) and the fp32 flipped input (4 B per position)
 ENSEMBLE_UNITS = 1.0 + 1.0 / 16
+# and, when the mutual information is wanted, the fp32 expected-entropy plane (4 B per position)
+ENTROPY_UNITS = 1.0 / 16
+
+
+def ensemble_units(entropy: bool) -> float:
+    """fit_group's `extra` for run_ensemble: ENSEMBLE_UNITS, plus ENTROPY_UNITS when the entropy plane is allocated."""
+    return ENSEMBLE_UNITS + (ENTROPY_UNITS if entropy else 0.0)
 
 
 def flip_tables(n: int, h: int, w: int, flip: int, device="cpu"):
@@ -720,13 +727,23 @@ def run_ensemble(engines: List[SpffEngine], x: torch.Tensor, flips: Tuple[int, .
                  per_sample: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None,
                  labels_out: Optional[torch.Tensor] = None, proba_out: Optional[torch.Tensor] = None,
                  hist: Optional[torch.Tensor] = None, sample_hist: Optional[torch.Tensor] = None,
-                 staged: Optional["StagedBatch"] = None):
+                 staged: Optional["StagedBatch"] = None, entropy_out: Optional[torch.Tensor] = None,
+                 mi_out: Optional[torch.Tensor] = None, unc: Optional[torch.Tensor] = None,
+                 sample_unc: Optional[torch.Tensor] = None, calib: Optional[torch.Tensor] = None,
+                 sample_calib: Optional[torch.Tensor] = None, brier: Optional[torch.Tensor] = None,
+                 sample_brier: Optional[torch.Tensor] = None):
     """Averaged softmax of several networks of one NetConfig over input flips (1 = H, 2 = W, 0 = none), sample group by
     sample group, with no logits in memory. Every member runs on the FIRST engine's inference buffers; for each group
     and member (outer) and flip (inner): flip the input (spff_grid_aug), forward, and add the head's softmax, mirrored
     back, into an fp32 [group,d,h,w,16] accumulator (ops.head_prob_accum). One ops.prob_finalize per group then writes
     p̄ = mean over the passes: labels_out (uint8 [B,F,H,W], arg-max), proba_out (fp16 [B,K,F,H,W]) and, with labels,
-    the tally, per-sample rows and histograms of SpffEngine.eval_step computed on p̄. `staged`: as in train_step."""
+    the tally, per-sample rows and histograms of SpffEngine.eval_step computed on p̄. `staged`: as in train_step.
+
+    Uncertainty and calibration (ops.Uncertainty): entropy_out / mi_out fp16 [B,F,H,W] maps of H[p̄] and of the mutual
+    information H[p̄] - mean over passes of H[p]; unc int64 [2] / sample_unc int64 [B,2] (+=) their sums in units of
+    2^-24 nats; with labels calib int64 [3,T] / sample_calib [B,3,T] and brier fp64 [1] / sample_brier fp64 [B] (+=).
+    The fp32 [group,d,h,w] expected-entropy plane rides the member x flip loop only when mi_out, unc or sample_unc is
+    given (the mutual information needs it); it is counted in the group size only then."""
     first = engines[0]
     x = first._check_input(x)
     bsz, _, d, h, w = x.shape
@@ -738,8 +755,11 @@ def run_ensemble(engines: List[SpffEngine], x: torch.Tensor, flips: Tuple[int, .
     for e in engines:   # once per call, not per group
         e.refresh_weights()
         tables.append(GateTables(e.cfg, e.params(), d, need_grad=False))
-    group = first._fitted(min(group, bsz), d, h, w, x.device, train=False, extra=ENSEMBLE_UNITS)
+    want_mi = mi_out is not None or unc is not None or sample_unc is not None
+    want_unc = want_mi or entropy_out is not None or calib is not None
+    group = first._fitted(min(group, bsz), d, h, w, x.device, train=False, extra=ensemble_units(want_mi))
     acc = torch.empty(group, d, h, w, 16, device=x.device)
+    ent = torch.empty(group, d, h, w, device=x.device) if want_mi else None
     flipped = any(flips)
     xf = torch.empty(group, 1, d, h, w, device=x.device) if flipped else None
     gather = _FlipGather(group, h, w, x.device) if flipped else None
@@ -763,14 +783,19 @@ def run_ensemble(engines: List[SpffEngine], x: torch.Tensor, flips: Tuple[int, .
                     gather(xin, xf[:n], f)
                     xin = xf[:n]
                 e.forward_group(B, T, xin, head="none")
-                ops.head_prob_accum(B.out["dec1"], p["out.weight"], p["out.bias"], a, flip=f, beta=beta)
+                ops.head_prob_accum(B.out["dec1"], p["out.weight"], p["out.bias"], a, flip=f, beta=beta,
+                                    ent=ent[:n] if ent is not None else None)
                 beta = 1
         if staged is not None:
             staged.wait_labels(hi)
+        u = ops.Uncertainty(ent=ent[:n] if ent is not None else None, entropy_out=rows(entropy_out, lo, hi),
+                            mi_out=rows(mi_out, lo, hi), unc=unc, sample_unc=rows(sample_unc, lo, hi), calib=calib,
+                            sample_calib=rows(sample_calib, lo, hi), brier=brier,
+                            sample_brier=rows(sample_brier, lo, hi)) if want_unc else None
         ops.prob_finalize(a, first.cfg.num_classes, scale, labels=rows(labels, lo, hi), ignore_index=ignore_index,
                           tally=tl, per_sample=tuple(t[lo:hi] for t in per_sample) if per_sample is not None else None,
                           labels_out=rows(labels_out, lo, hi), hist=hist, sample_hist=rows(sample_hist, lo, hi),
-                          proba_out=rows(proba_out, lo, hi))
+                          proba_out=rows(proba_out, lo, hi), unc=u)
 
 
 class StagedBatch:

@@ -7,10 +7,14 @@ enqueue on the current CUDA stream.
 """
 from __future__ import annotations
 
+import ctypes
+import dataclasses
+from typing import Optional
+
 import torch
 
 from . import _lib
-from ._lib import Shape, call, ptr, stream_ptr
+from ._lib import Shape, UncOut, call, ptr, stream_ptr
 
 
 def _view(t: torch.Tensor, c: int):
@@ -397,23 +401,72 @@ def head_eval(x, w, b, labels, ignore_index, acc, counts, confusion, sample_acc=
              ptr(hist), ptr(sample_hist), stream_ptr())
 
 
-def head_prob_accum(x, w, b, acc, flip: int = 0, beta: int = 0):
+def head_prob_accum(x, w, b, acc, flip: int = 0, beta: int = 0, ent=None):
     """Head + softmax added into the probability accumulator acc (fp32 [n,d,h,w,16], contiguous, 16-byte aligned):
     acc[n,d,h',w',c] = beta * acc + p_c, with h' / w' mirrored back when bit 1 / 2 of `flip` is set (the inverse of an
-    input flip). Classes >= K are written as 0 when beta = 0 and left alone when beta = 1 (spff_head_prob_accum)."""
+    input flip). Classes >= K are written as 0 when beta = 0 and left alone when beta = 1 (spff_head_prob_accum).
+    With `ent` (fp32 [n,d,h,w], contiguous) also ent[n,d,h',w'] = beta * ent + H(p), the entropy of this pass's
+    softmax in nats (spff_head_prob_accum_ent)."""
     s, ldx = _view(x, 32)
     assert acc.dtype == torch.float32 and acc.is_contiguous() and acc.numel() == s.n * s.d * s.h * s.w * 16
-    call("spff_head_prob_accum", ptr(x), ldx, 32, ptr(w), ptr(b), w.shape[0], s, int(flip), int(beta), ptr(acc),
-         stream_ptr())
+    if ent is None:
+        call("spff_head_prob_accum", ptr(x), ldx, 32, ptr(w), ptr(b), w.shape[0], s, int(flip), int(beta), ptr(acc),
+             stream_ptr())
+        return
+    assert ent.dtype == torch.float32 and ent.is_contiguous() and ent.numel() == s.n * s.d * s.h * s.w
+    call("spff_head_prob_accum_ent", ptr(x), ldx, 32, ptr(w), ptr(b), w.shape[0], s, int(flip), int(beta), ptr(acc),
+         ptr(ent), stream_ptr())
+
+
+@dataclasses.dataclass
+class Uncertainty:
+    """Outputs of prob_finalize(unc=...) (spff_unc_out); every field is optional. Per position of an accumulator of n
+    samples: `ent` the expected-entropy plane of head_prob_accum(ent=...) (fp32 [n,d,h,w], the sum over the passes),
+    `entropy_out` / `mi_out` fp16 [n,d,h,w] maps of H[p̄] and of the mutual information max(H[p̄] - scale * ent, 0)
+    (needs ent); `unc` int64 [2] (+=) and `sample_unc` int64 [n,2] (+=) their sums in units of 2^-24 nats. With labels:
+    `calib` int64 [3,T] (+=: per confidence bin the counted voxels, the correct ones and the summed confidence in
+    units of 2^-24), `sample_calib` [n,3,T] (exactly when the per-sample tallies are given), `brier` fp64 [1] and
+    `sample_brier` fp64 [n] (exactly with calib / sample_calib) the summed Brier score."""
+    ent: Optional[torch.Tensor] = None
+    entropy_out: Optional[torch.Tensor] = None
+    mi_out: Optional[torch.Tensor] = None
+    unc: Optional[torch.Tensor] = None
+    sample_unc: Optional[torch.Tensor] = None
+    calib: Optional[torch.Tensor] = None
+    sample_calib: Optional[torch.Tensor] = None
+    brier: Optional[torch.Tensor] = None
+    sample_brier: Optional[torch.Tensor] = None
+
+
+def _unc_struct(u: Uncertainty, n: int, vox: int) -> UncOut:
+    def check(t, dtype, numel, name):
+        if t is not None:
+            assert t.dtype == dtype and t.is_contiguous() and t.numel() == numel, \
+                f"{name}: expected contiguous {dtype} with {numel} elements, got {t.dtype} {tuple(t.shape)}"
+    check(u.ent, torch.float32, vox, "ent")
+    check(u.entropy_out, torch.float16, vox, "entropy_out")
+    check(u.mi_out, torch.float16, vox, "mi_out")
+    check(u.unc, torch.int64, 2, "unc")
+    check(u.sample_unc, torch.int64, 2 * n, "sample_unc")
+    bins = 0
+    if u.calib is not None:
+        bins = u.calib.shape[-1]
+        check(u.calib, torch.int64, 3 * bins, "calib")
+        check(u.sample_calib, torch.int64, n * 3 * bins, "sample_calib")
+    check(u.brier, torch.float64, 1, "brier")
+    check(u.sample_brier, torch.float64, n, "sample_brier")
+    return UncOut(ptr(u.ent), ptr(u.entropy_out), ptr(u.mi_out), ptr(u.unc), ptr(u.sample_unc), int(bins), ptr(u.calib),
+                  ptr(u.sample_calib), ptr(u.brier), ptr(u.sample_brier))
 
 
 def prob_finalize(acc, k: int, scale: float, labels=None, ignore_index: int = 255, tally=None, per_sample=None,
-                  labels_out=None, hist=None, sample_hist=None, proba_out=None):
+                  labels_out=None, hist=None, sample_hist=None, proba_out=None, unc: Optional[Uncertainty] = None):
     """One pass over a spff_head_prob_accum accumulator acc (fp32 [n,d,h,w,16]): p̄ = scale * acc. Optional outputs:
     labels_out (uint8 [n,d,h,w], the first arg-max of acc over classes < k), proba_out (fp16 [n,k,d,h,w], p̄), and with
     labels (uint8 / int64 [n,d,h,w]) the tally (nll fp64 [1], count int64 [1], confusion int64 [k,k], +=) of
     head_eval on p̄, per_sample rows (fp64 [n], int64 [n], int64 [n,k,k]), hist (int64 [k,2,T]) and sample_hist
-    (int64 [n,k,2,T]) of p̄ (spff_prob_finalize)."""
+    (int64 [n,k,2,T]) of p̄ (spff_prob_finalize). With `unc` (an Uncertainty) also its maps, sums and calibration
+    histogram (spff_prob_finalize_unc); every other output is the same, bit for bit."""
     assert acc.dtype == torch.float32 and acc.dim() == 5 and acc.shape[-1] == 16 and acc.is_contiguous()
     n, d, h, w, _ = acc.shape
     vox = n * d * h * w
@@ -441,9 +494,15 @@ def prob_finalize(acc, k: int, scale: float, labels=None, ignore_index: int = 25
         assert labels_out.dtype == torch.uint8 and labels_out.is_contiguous() and labels_out.numel() == vox
     if proba_out is not None:
         assert proba_out.dtype == torch.float16 and proba_out.is_contiguous() and tuple(proba_out.shape) == (n, k, d, h, w)
-    call("spff_prob_finalize", ptr(acc), int(k), s, float(scale), ptr(labels), lb, int(ignore_index), ptr(nll), ptr(cnt),
-         ptr(conf), *(ptr(t) for t in per), ptr(labels_out), int(bins), ptr(hist), ptr(sample_hist), ptr(proba_out),
-         stream_ptr())
+    if unc is None:
+        call("spff_prob_finalize", ptr(acc), int(k), s, float(scale), ptr(labels), lb, int(ignore_index), ptr(nll),
+             ptr(cnt), ptr(conf), *(ptr(t) for t in per), ptr(labels_out), int(bins), ptr(hist), ptr(sample_hist),
+             ptr(proba_out), stream_ptr())
+        return
+    u = _unc_struct(unc, n, vox)
+    call("spff_prob_finalize_unc", ptr(acc), int(k), s, float(scale), ptr(labels), lb, int(ignore_index), ptr(nll),
+         ptr(cnt), ptr(conf), *(ptr(t) for t in per), ptr(labels_out), int(bins), ptr(hist), ptr(sample_hist),
+         ptr(proba_out), ctypes.byref(u), stream_ptr())
 
 
 def scale_by_count(g, count, factor: float = 1.0):
