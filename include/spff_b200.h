@@ -323,6 +323,33 @@ int spff_prob_finalize_unc(const float* acc, int k, spff_shape s, float scale, c
                            long long* hist, long long* sample_hist, void* proba_out, const spff_unc_out* unc,
                            void* stream);
 
+/* ---- temperature scaling of the averaged softmax -------------------------------------------------------------
+ * spff_prob_finalize_unc with the pooled distribution tempered: with β = inv_temperature (positive, finite),
+ *   p̃_c = p̄_c^β / sum_{c'<K} p̄_c'^β        (p̄_c = 0 stays 0),
+ * replaces p̄ in every output: proba_out, nll, hist, H[p̃] (entropy_out and unc[0]), the confidence p̃_arg and brier
+ * of `unc`. The arg-max (labels_out, confusion) is unchanged, and the mutual information (mi_out, unc[1]) stays
+ * H[p̄] - mean H[p] of the untempered passes, bit for bit. unc may be NULL (the outputs of spff_prob_finalize only).
+ * Every other argument is that of spff_prob_finalize_unc. */
+int spff_prob_finalize_tempered(const float* acc, int k, spff_shape s, float scale, const void* labels, int label_bytes,
+                                int ignore_index, double* nll, long long* counts, long long* confusion,
+                                double* sample_acc, long long* sample_counts, long long* sample_confusion,
+                                uint8_t* labels_out, int bins, long long* hist, long long* sample_hist, void* proba_out,
+                                const spff_unc_out* unc, float inv_temperature, void* stream);
+/* Bytes of the workspace of spff_prob_temp_fit for k classes, shape s and g grid points (0 when they are invalid). */
+size_t spff_prob_temp_fit_workspace(int k, spff_shape s, int g);
+/* Statistics of the temperature fit on an accumulator of spff_head_prob_accum (p̄_c = scale * acc_c): for every voxel
+ * whose label y (uint8 or int64 [N,D,H,W]) is in [0,K) and not ignore_index, and each grid value β_g (betas: fp32 [g]
+ * on the device, each positive and finite; not checked, as the host does not read device memory),
+ *   f(β)  = log sum_{c: p̄_c > 0} exp(β log p̄_c) - β log p̄_y   (the tempered nll; -log FLT_MIN when p̄_y = 0)
+ *   f'(β) = sum_c p̃_c log p̄_c - log p̄_y                        (0 when p̄_y = 0)
+ * sums fp64 [2][g] (+=) receives sum f(β_g) in [0][g] and sum f'(β_g) in [1][g], counted (+=) the voxels. f is convex
+ * in β. Per-block fp64 partials in the workspace are added in a fixed order: bit-reproducible, no float atomics.
+ * k in [2,16], g in [1,64], acc 16-byte aligned, N <= 65535; workspace of spff_prob_temp_fit_workspace(k, s, g) bytes
+ * (SPFF_ERR_WORKSPACE otherwise). Compute-bound: g x k exponentials per voxel. */
+int spff_prob_temp_fit(const float* acc, int k, spff_shape s, float scale, const void* labels, int label_bytes,
+                       int ignore_index, const float* betas, int g, double* sums, long long* counted, void* workspace,
+                       size_t workspace_bytes, void* stream);
+
 /* ---- "3DUNet" control: Cicek3DUNet + depth adapter (models.py:718-777; config.py:283-311) ---------------
  * Its 3x3x3 convolutions, normalise + ReLU passes (slope 0), head and loss are the entry points above;
  * the ones below are what only this variant needs. */

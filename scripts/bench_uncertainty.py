@@ -39,9 +39,9 @@ CONFIGS = (("1xnone", 1, None), ("3xflip", 3, "flip"))
 KERNELS = {
     "accumulate": ("head_prob_accum_kernel<false>", "head_prob_accum_kernelILb0EE"),
     "accumulate_ent": ("head_prob_accum_kernel<true>", "head_prob_accum_kernelILb1EE"),
-    "finalize": tuple(f"prob_finalize_kernel<{t}, {h}, false>" for t in ("unsigned char", "long long")
+    "finalize": tuple(f"prob_finalize_kernel<{t}, {h}, false, false>" for t in ("unsigned char", "long long")
                       for h in ("false", "true")),
-    "finalize_unc": tuple(f"prob_finalize_kernel<{t}, {h}, true>" for t in ("unsigned char", "long long")
+    "finalize_unc": tuple(f"prob_finalize_kernel<{t}, {h}, true, false>" for t in ("unsigned char", "long long")
                           for h in ("false", "true")),
 }
 

@@ -7,14 +7,17 @@
 //   * cross-entropy with ignore_index + the hard confusion tally that macro_dice_loss and
 //     per_class_metrics_3d derive all their counts from (innovative3D/helpers.py:668-725, 782-803);
 //   * the averaged softmax of ensembles and mirror test-time augmentation: the head's softmax added into
-//     an fp32 probability accumulator, and one finishing pass to arg-max / probabilities / tallies;
+//     an fp32 probability accumulator, and one finishing pass to arg-max / probabilities / tallies, optionally
+//     temperature-scaled; the statistics of the temperature fit on that accumulator;
 //   * Adam (BaseLitModel.configure_optimizers, models.py:591-594).
 // All are bandwidth-bound: one thread per voxel (or per 16-byte channel vector), coalesced
-// accesses, weights broadcast from constant / shared memory.
+// accesses, weights broadcast from constant / shared memory. The exception is the temperature fit, which evaluates
+// G x K exponentials per voxel and is compute-bound.
 #include "common.h"
 #include "ptx.cuh"
 
 #include <cfloat>
+#include <cmath>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -1579,6 +1582,10 @@ head_prob_accum_kernel(const __nv_bfloat16* __restrict__ x, long long ldx, int K
 // one if arg == label, and conf in units of 2^-24; its Brier term sum_c (p̄_c - [c == y])^2 is reduced like the nll.
 // The top bin is counted in registers (a trained model puts most voxels there); the UNC tallies live in dynamic shared
 // memory behind the HIST histogram: ull [2] uncertainty sums, ull [Tc] confidence sums, u32 [2][Tc] counts, float [8].
+// TEMP (spff_prob_finalize_tempered, inv_t = β = 1/T): p̃_c = p̄_c^β / sum_{c'<K} p̄_c'^β, computed as
+// e_c = exp(β (log p̄_c - log p̄_arg)) / sum e (accurate logf / expf; p̄_c = 0 stays 0), replaces p̄ everywhere below:
+// proba_out, nll, HIST, H[p̃] (entropy_out and the H sum), the confidence p̃_arg and Brier. The arg-max is still taken
+// on acc (p̃ is a monotone map of p̄) and the mutual information keeps H[p̄], the untempered passes' disagreement.
 constexpr int kPfThreads = 256;
 constexpr float kFix24 = 16777216.f;   // 2^24
 
@@ -1594,7 +1601,7 @@ __device__ __forceinline__ void prob_finalize_flush_unc(const spff_unc_out& u, l
   }
 }
 
-template <typename LabelT, bool HIST, bool UNC = false>
+template <typename LabelT, bool HIST, bool UNC = false, bool TEMP = false>
 __global__ void __launch_bounds__(kPfThreads)
 prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float scale, const void* __restrict__ labels,
                      int ignore_index, double* __restrict__ nll, unsigned long long* __restrict__ counts,
@@ -1602,7 +1609,7 @@ prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float 
                      unsigned long long* __restrict__ sample_counts, unsigned long long* __restrict__ sample_confusion,
                      uint8_t* __restrict__ labels_out, __half* __restrict__ proba_out, int T,
                      unsigned long long* __restrict__ hist, unsigned long long* __restrict__ sample_hist,
-                     spff_unc_out u) {
+                     spff_unc_out u, float inv_t) {
   __shared__ unsigned int s_conf[kMaxK * kMaxK];
   __shared__ float s_nll[kPfThreads / 32];
   __shared__ unsigned int s_cnt[kPfThreads / 32];
@@ -1660,6 +1667,28 @@ prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float 
     float p[kMaxK];
 #pragma unroll
     for (int c = 0; c < kMaxK; ++c) p[c] = __fmul_rn(scale, a[c]);
+    [[maybe_unused]] float hb_bar = 0.f;   // TEMP: H[p̄] for the mutual information, as the untempered pass sums it
+    [[maybe_unused]] float p_arg = 0.f;    // TEMP: p̃_arg
+    if constexpr (TEMP) {
+      const float l_arg = logf(__fmul_rn(scale, mx));
+      float se = 0.f;
+#pragma unroll
+      for (int c = 0; c < kMaxK; ++c) {
+        float e = 0.f;
+        if (c < K && p[c] > 0.f) {
+          const float l = logf(p[c]);
+          if constexpr (UNC) hb_bar = fmaf(-p[c], l, hb_bar);
+          e = expf(inv_t * (l - l_arg));
+        }
+        p[c] = e;
+        se += e;
+      }
+#pragma unroll
+      for (int c = 0; c < kMaxK; ++c) {
+        if (se > 0.f) p[c] = __fdiv_rn(p[c], se);   // se = 0 only for an all-zero accumulator row: p̃ = 0
+        if (c == arg) p_arg = p[c];
+      }
+    }
     if (labels_out) labels_out[pos] = static_cast<uint8_t>(arg);
     if (proba_out) {
 #pragma unroll
@@ -1673,7 +1702,11 @@ prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float 
         if (c < K && p[c] > 0.f) hb = fmaf(-p[c], logf(p[c]), hb);
       hb = fmaxf(hb, 0.f);   // p̄_c may exceed 1 by an ulp
       float mi = 0.f;
-      if (u.ent) mi = fmaxf(hb - __fmul_rn(scale, __ldg(u.ent + n * dhw + pos)), 0.f);
+      if constexpr (TEMP) {
+        if (u.ent) mi = fmaxf(fmaxf(hb_bar, 0.f) - __fmul_rn(scale, __ldg(u.ent + n * dhw + pos)), 0.f);
+      } else {
+        if (u.ent) mi = fmaxf(hb - __fmul_rn(scale, __ldg(u.ent + n * dhw + pos)), 0.f);
+      }
       if (u.entropy_out) static_cast<__half*>(u.entropy_out)[n * dhw + pos] = __float2half_rn(hb);
       if (u.mi_out) static_cast<__half*>(u.mi_out)[n * dhw + pos] = __float2half_rn(mi);
       h_sum += __float2ll_rn(hb * kFix24);
@@ -1706,7 +1739,7 @@ prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float 
           }
           if constexpr (UNC) {
             if (Tc) {
-              const float conf = __fmul_rn(scale, mx);   // p̄_arg
+              const float conf = TEMP ? p_arg : __fmul_rn(scale, mx);   // p̄_arg (p̃_arg)
               const int bin = min(static_cast<int>(__fmul_rn(conf, static_cast<float>(Tc))), Tc - 1);
               const long long cfix = __float2ll_rn(conf * kFix24);
               const unsigned int correct = arg == lab ? 1u : 0u;
@@ -1838,6 +1871,136 @@ prob_finalize_kernel(const float* __restrict__ acc, int K, long long dhw, float 
   }
 }
 
+// prob_temp_fit_kernel: the statistics of the temperature fit on the pooled p̄ = scale * acc. A voxel counts when its
+// label y is in [0, K) and not ignore_index. With l_c = log p̄_c, m = l_arg (the first maximum of acc, as in
+// prob_finalize_kernel) and d_c = l_c - m over the classes c != arg with p̄_c > 0, for each grid value β_g:
+//   f(β)  = log sum_c exp(β l_c) - β l_y = β (m - l_y) + log1p(s1),            s1 = sum_c exp(β d_c),
+//   f'(β) = sum_c p̃_c l_c - l_y         = (m - l_y) + sum_c exp(β d_c) d_c / (1 + s1),
+// the forms without cancellation when y = arg; a voxel with p̄_y = 0 adds -log FLT_MIN to f and 0 to f' (the nll rule
+// of prob_finalize_kernel). Accurate logf / expf / log1pf. Each warp takes tiles of 32 voxels of the flattened
+// [N*D*H*W] grid: lane i stages voxel i's d_c and m - l_y in shared memory, then lane j evaluates grid points j and
+// j + 32 over the tile's voxels (broadcast reads) and adds f, f' into fp64 registers. The block's sums (warps added in
+// order) and its count go to partial[block][2G + 1] (count as u64 bits); prob_temp_fit_reduce_kernel adds the blocks in
+// order. No floating-point atomics, so the result is bit-reproducible for a given grid; fp64 cannot overflow.
+constexpr int kTfThreads = 256, kTfBlocksPerSm = 4, kTfMaxG = 64;
+constexpr float kTfSkip = -1.f, kTfZeroY = -2.f;   // staged m - l_y (>= 0 otherwise): not counted, p̄_y = 0
+
+template <typename LabelT>
+__global__ void __launch_bounds__(kTfThreads, kTfBlocksPerSm)
+prob_temp_fit_kernel(const float* __restrict__ acc, int K, long long total, float scale,
+                     const LabelT* __restrict__ labels, int ignore_index, const float* __restrict__ betas, int G,
+                     double* __restrict__ partial) {
+  constexpr int kWarps = kTfThreads / 32;
+  __shared__ float s_d[kWarps][32][kMaxK + 1];   // per voxel of the warp's tile: d_c (-inf: left out), m - l_y
+  __shared__ double s_part[kWarps][2 * kTfMaxG];
+  __shared__ unsigned int s_cnt[kWarps];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  float beta[2];
+#pragma unroll
+  for (int j = 0; j < 2; ++j) beta[j] = lane + 32 * j < G ? __ldg(betas + lane + 32 * j) : 1.f;
+  double sf[2] = {0.0, 0.0}, sd[2] = {0.0, 0.0};
+  unsigned int cnt = 0;
+  const long long ntiles = (total + 31) / 32;
+  for (long long tile = static_cast<long long>(blockIdx.x) * kWarps + warp; tile < ntiles;
+       tile += static_cast<long long>(gridDim.x) * kWarps) {
+    const long long pos = tile * 32 + lane;
+    float dy = kTfSkip;
+    if (pos < total) {
+      const int lab = static_cast<int>(labels[pos]);
+      if (lab != ignore_index && lab >= 0 && lab < K) {
+        ++cnt;
+        float a[kMaxK];
+        const float4* src = reinterpret_cast<const float4*>(acc + pos * kMaxK);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const float4 q = __ldg(src + j);
+          a[4 * j] = q.x;
+          a[4 * j + 1] = q.y;
+          a[4 * j + 2] = q.z;
+          a[4 * j + 3] = q.w;
+        }
+        int arg = 0;
+        float mx = a[0];
+#pragma unroll
+        for (int c = 1; c < kMaxK; ++c)
+          if (c < K && a[c] > mx) {
+            mx = a[c];
+            arg = c;
+          }
+        const float m = logf(__fmul_rn(scale, mx));
+#pragma unroll
+        for (int c = 0; c < kMaxK; ++c) {
+          const float p = __fmul_rn(scale, a[c]);
+          const float l = c < K && p > 0.f ? logf(p) : 0.f;
+          if (c < K) s_d[warp][lane][c] = c != arg && p > 0.f ? l - m : -INFINITY;
+          if (c == lab) dy = p > 0.f ? m - l : kTfZeroY;
+        }
+      }
+    }
+    s_d[warp][lane][kMaxK] = dy;
+    __syncwarp();
+    for (int v = 0; v < 32; ++v) {
+      const float dyv = s_d[warp][v][kMaxK];   // the same for all lanes: no divergence
+      if (dyv == kTfSkip) continue;
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+        if (lane + 32 * j >= G) continue;
+        if (dyv == kTfZeroY) {
+          sf[j] += static_cast<double>(-logf(FLT_MIN));
+          continue;
+        }
+        float s1 = 0.f, t = 0.f;
+#pragma unroll
+        for (int c = 0; c < kMaxK; ++c)
+          if (c < K) {
+            const float dc = s_d[warp][v][c];
+            const float e = expf(beta[j] * dc);   // dc = -inf: e = 0
+            s1 += e;
+            if (e > 0.f) t = fmaf(e, dc, t);
+          }
+        sf[j] += fma(static_cast<double>(beta[j]), static_cast<double>(dyv), static_cast<double>(log1pf(s1)));
+        sd[j] += static_cast<double>(dyv) + static_cast<double>(t / (1.f + s1));
+      }
+    }
+    __syncwarp();   // the tile is read before the next one is staged
+  }
+#pragma unroll
+  for (int j = 0; j < 2; ++j)
+    if (lane + 32 * j < G) {
+      s_part[warp][lane + 32 * j] = sf[j];
+      s_part[warp][G + lane + 32 * j] = sd[j];
+    }
+  for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+  if (lane == 0) s_cnt[warp] = cnt;
+  __syncthreads();
+  double* out = partial + static_cast<long long>(blockIdx.x) * (2 * G + 1);
+  for (int i = threadIdx.x; i < 2 * G; i += blockDim.x) {
+    double s = 0.0;
+    for (int wv = 0; wv < kWarps; ++wv) s += s_part[wv][i];
+    out[i] = s;
+  }
+  if (threadIdx.x == 0) {
+    unsigned long long c = 0;
+    for (int wv = 0; wv < kWarps; ++wv) c += s_cnt[wv];
+    reinterpret_cast<unsigned long long*>(out)[2 * G] = c;
+  }
+}
+
+// sums[i] += the blocks' partial[b][i] added in block order (i < 2G); counted += the blocks' counts
+__global__ void prob_temp_fit_reduce_kernel(const double* __restrict__ partial, int blocks, int G,
+                                            double* __restrict__ sums, unsigned long long* __restrict__ counted) {
+  const int i = threadIdx.x, stride = 2 * G + 1;
+  if (i < 2 * G) {
+    double s = 0.0;
+    for (int b = 0; b < blocks; ++b) s += partial[static_cast<long long>(b) * stride + i];
+    sums[i] += s;
+  } else if (i == 2 * G) {
+    unsigned long long c = 0;
+    for (int b = 0; b < blocks; ++b) c += reinterpret_cast<const unsigned long long*>(partial)[static_cast<long long>(b) * stride + i];
+    *counted += c;
+  }
+}
+
 // ---------------------------------------------------------------------------------------------
 // Adam (torch.optim.Adam semantics, no weight decay / amsgrad)
 // ---------------------------------------------------------------------------------------------
@@ -1956,12 +2119,13 @@ int head_eval_launch(const char* name, const void* x, long long ldx, int cin, co
   return 0;
 }
 
-template <typename LabelT>
+template <typename LabelT, bool TEMP>
 int prob_finalize_hist_attr() {   // once per device, as head_eval_hist_attr
   static bool attr_set[spff::kMaxDevices] = {};
   const int dev = spff::current_device();
   if (!attr_set[dev]) {
-    SPFF_CUDA(cudaFuncSetAttribute(spff::prob_finalize_kernel<LabelT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    SPFF_CUDA(cudaFuncSetAttribute(spff::prob_finalize_kernel<LabelT, true, false, TEMP>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    static_cast<int>(sizeof(unsigned int) * spff::kMaxK * 2 * spff::kHeMaxBins)));
     attr_set[dev] = true;
   }
@@ -2009,12 +2173,12 @@ size_t prob_finalize_smem(bool unc, int k, int bins, int cal_bins) {
               : 0);
 }
 
-template <typename LabelT, bool HIST>
+template <typename LabelT, bool HIST, bool TEMP>
 int prob_finalize_unc_attr() {   // once per device, as head_eval_hist_attr
   static bool attr_set[spff::kMaxDevices] = {};
   const int dev = spff::current_device();
   if (!attr_set[dev]) {
-    SPFF_CUDA(cudaFuncSetAttribute(spff::prob_finalize_kernel<LabelT, HIST, true>,
+    SPFF_CUDA(cudaFuncSetAttribute(spff::prob_finalize_kernel<LabelT, HIST, true, TEMP>,
                                    cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    static_cast<int>(prob_finalize_smem(true, spff::kMaxK, HIST ? spff::kHeMaxBins : 0,
                                                                        kUncMaxBins))));
@@ -2023,39 +2187,43 @@ int prob_finalize_unc_attr() {   // once per device, as head_eval_hist_attr
   return 0;
 }
 
-template <typename LabelT, bool HIST, bool UNC>
+template <typename LabelT, bool HIST, bool UNC, bool TEMP>
 int prob_finalize_run(dim3 grid, size_t smem, cudaStream_t st, const float* acc, int k, long long dhw, float scale,
                       const void* labels, int ignore_index, double* nll, long long* counts, long long* confusion,
                       double* sample_acc, long long* sample_counts, long long* sample_confusion, uint8_t* labels_out,
-                      int T, long long* hist, long long* sample_hist, void* proba_out, const spff_unc_out& u) {
+                      int T, long long* hist, long long* sample_hist, void* proba_out, const spff_unc_out& u,
+                      float inv_t) {
   if constexpr (HIST && !UNC) {
-    const int e = prob_finalize_hist_attr<LabelT>();
+    const int e = prob_finalize_hist_attr<LabelT, TEMP>();
     if (e) return e;
   }
   if constexpr (UNC) {
-    const int e = prob_finalize_unc_attr<LabelT, HIST>();
+    const int e = prob_finalize_unc_attr<LabelT, HIST, TEMP>();
     if (e) return e;
   }
-  spff::prob_finalize_kernel<LabelT, HIST, UNC><<<grid, spff::kPfThreads, smem, st>>>(
+  spff::prob_finalize_kernel<LabelT, HIST, UNC, TEMP><<<grid, spff::kPfThreads, smem, st>>>(
       acc, k, dhw, scale, labels, ignore_index, nll, reinterpret_cast<unsigned long long*>(counts),
       reinterpret_cast<unsigned long long*>(confusion), sample_acc, reinterpret_cast<unsigned long long*>(sample_counts),
       reinterpret_cast<unsigned long long*>(sample_confusion), labels_out, static_cast<__half*>(proba_out), T,
-      reinterpret_cast<unsigned long long*>(hist), reinterpret_cast<unsigned long long*>(sample_hist), u);
+      reinterpret_cast<unsigned long long*>(hist), reinterpret_cast<unsigned long long*>(sample_hist), u, inv_t);
   SPFF_CUDA(cudaGetLastError());
   return 0;
 }
 
-// spff_prob_finalize (with_unc = false) and spff_prob_finalize_unc (with_unc = true, unc required)
+// spff_prob_finalize (with_unc = false), spff_prob_finalize_unc (with_unc = true, unc required) and
+// spff_prob_finalize_tempered (temp = true; with_unc = unc != NULL)
 int prob_finalize_launch(const char* name, bool with_unc, const float* acc, int k, spff_shape s, float scale,
                          const void* labels, int label_bytes, int ignore_index, double* nll, long long* counts,
                          long long* confusion, double* sample_acc, long long* sample_counts, long long* sample_confusion,
                          uint8_t* labels_out, int bins, long long* hist, long long* sample_hist, void* proba_out,
-                         const spff_unc_out* unc, void* stream) {
+                         const spff_unc_out* unc, void* stream, bool temp = false, float inv_t = 1.f) {
   SPFF_REQUIRE(acc, "%s: null accumulator", name);
   SPFF_REQUIRE(k >= 2 && k <= spff::kMaxK, "%s: classes must be in [2, %d] (got %d)", name, spff::kMaxK, k);
   SPFF_REQUIRE((reinterpret_cast<uintptr_t>(acc) & 15) == 0, "%s: acc must be 16-byte aligned", name);
   SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "%s: bad shape (N must be <= 65535)", name);
   SPFF_REQUIRE(scale > 0.f, "%s: scale must be positive", name);
+  SPFF_REQUIRE(!temp || (inv_t > 0.f && std::isfinite(inv_t)), "%s: inv_temperature must be positive and finite (got %g)",
+               name, static_cast<double>(inv_t));
   SPFF_REQUIRE(!labels || label_bytes == 1 || label_bytes == 8, "%s: labels must be uint8 or int64", name);
   SPFF_REQUIRE(labels ? (nll && counts && confusion) : !(nll || counts || confusion || sample_acc || hist),
                "%s: the tally (nll, counts, confusion) is given exactly when the labels are", name);
@@ -2096,8 +2264,21 @@ int prob_finalize_launch(const char* name, bool with_unc, const float* acc, int 
   const size_t smem = prob_finalize_smem(with_unc, k, T, u.cal_bins);
   const bool wide = label_bytes == 8;
 #define SPFF_PF_RUN(L, H, U)                                                                                              \
-  prob_finalize_run<L, H, U>(grid, smem, st, acc, k, dhw, scale, labels, ignore_index, nll, counts, confusion, sample_acc, \
-                             sample_counts, sample_confusion, labels_out, T, hist, sample_hist, proba_out, u)
+  prob_finalize_run<L, H, U, false>(grid, smem, st, acc, k, dhw, scale, labels, ignore_index, nll, counts, confusion,     \
+                                    sample_acc, sample_counts, sample_confusion, labels_out, T, hist, sample_hist,         \
+                                    proba_out, u, 1.f)
+#define SPFF_PF_RUN_T(L, H, U)                                                                                            \
+  prob_finalize_run<L, H, U, true>(grid, smem, st, acc, k, dhw, scale, labels, ignore_index, nll, counts, confusion,      \
+                                   sample_acc, sample_counts, sample_confusion, labels_out, T, hist, sample_hist,          \
+                                   proba_out, u, inv_t)
+  if (temp) {
+    if (!with_unc) {
+      if (!hist) return wide ? SPFF_PF_RUN_T(long long, false, false) : SPFF_PF_RUN_T(uint8_t, false, false);
+      return wide ? SPFF_PF_RUN_T(long long, true, false) : SPFF_PF_RUN_T(uint8_t, true, false);
+    }
+    if (!hist) return wide ? SPFF_PF_RUN_T(long long, false, true) : SPFF_PF_RUN_T(uint8_t, false, true);
+    return wide ? SPFF_PF_RUN_T(long long, true, true) : SPFF_PF_RUN_T(uint8_t, true, true);
+  }
   if (!with_unc) {
     if (!hist) return wide ? SPFF_PF_RUN(long long, false, false) : SPFF_PF_RUN(uint8_t, false, false);
     return wide ? SPFF_PF_RUN(long long, true, false) : SPFF_PF_RUN(uint8_t, true, false);
@@ -2105,6 +2286,23 @@ int prob_finalize_launch(const char* name, bool with_unc, const float* acc, int 
   if (!hist) return wide ? SPFF_PF_RUN(long long, false, true) : SPFF_PF_RUN(uint8_t, false, true);
   return wide ? SPFF_PF_RUN(long long, true, true) : SPFF_PF_RUN(uint8_t, true, true);
 #undef SPFF_PF_RUN
+#undef SPFF_PF_RUN_T
+}
+
+// blocks of prob_temp_fit_kernel (and rows of its workspace): ~one wave of kTfBlocksPerSm resident blocks per SM, no
+// more than the warp tiles need
+long long prob_temp_fit_blocks(spff_shape s) {
+  const long long total = static_cast<long long>(s.n) * s.d * s.h * s.w;
+  const long long tiles = (total + 31) / 32;
+  long long blocks = (tiles + spff::kTfThreads / 32 - 1) / (spff::kTfThreads / 32);
+  const long long cap = static_cast<long long>(spff::num_sms()) * spff::kTfBlocksPerSm;
+  if (blocks > cap) blocks = cap;
+  return blocks < 1 ? 1 : blocks;
+}
+
+bool prob_temp_fit_shape_ok(int k, spff_shape s, int g) {
+  return k >= 2 && k <= spff::kMaxK && g >= 1 && g <= spff::kTfMaxG && s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 &&
+         s.w > 0;
 }
 
 }  // namespace
@@ -2389,6 +2587,53 @@ int spff_prob_finalize_unc(const float* acc, int k, spff_shape s, float scale, c
   return prob_finalize_launch("prob_finalize_unc", true, acc, k, s, scale, labels, label_bytes, ignore_index, nll, counts,
                               confusion, sample_acc, sample_counts, sample_confusion, labels_out, bins, hist, sample_hist,
                               proba_out, unc, stream);
+}
+
+int spff_prob_finalize_tempered(const float* acc, int k, spff_shape s, float scale, const void* labels, int label_bytes,
+                                int ignore_index, double* nll, long long* counts, long long* confusion,
+                                double* sample_acc, long long* sample_counts, long long* sample_confusion,
+                                uint8_t* labels_out, int bins, long long* hist, long long* sample_hist, void* proba_out,
+                                const spff_unc_out* unc, float inv_temperature, void* stream) {
+  SPFF_ENTRY_CHECK();
+  return prob_finalize_launch("prob_finalize_tempered", unc != nullptr, acc, k, s, scale, labels, label_bytes,
+                              ignore_index, nll, counts, confusion, sample_acc, sample_counts, sample_confusion,
+                              labels_out, bins, hist, sample_hist, proba_out, unc, stream, true, inv_temperature);
+}
+
+size_t spff_prob_temp_fit_workspace(int k, spff_shape s, int g) {
+  if (!prob_temp_fit_shape_ok(k, s, g)) return 0;
+  return static_cast<size_t>(prob_temp_fit_blocks(s)) * (2 * g + 1) * sizeof(double);
+}
+
+int spff_prob_temp_fit(const float* acc, int k, spff_shape s, float scale, const void* labels, int label_bytes,
+                       int ignore_index, const float* betas, int g, double* sums, long long* counted, void* workspace,
+                       size_t workspace_bytes, void* stream) {
+  SPFF_ENTRY_CHECK();
+  SPFF_REQUIRE(acc && labels && betas && sums && counted && workspace, "prob_temp_fit: null pointer");
+  SPFF_REQUIRE(k >= 2 && k <= spff::kMaxK, "prob_temp_fit: classes must be in [2, %d] (got %d)", spff::kMaxK, k);
+  SPFF_REQUIRE(g >= 1 && g <= spff::kTfMaxG, "prob_temp_fit: grid points must be in [1, %d] (got %d)", spff::kTfMaxG, g);
+  SPFF_REQUIRE((reinterpret_cast<uintptr_t>(acc) & 15) == 0, "prob_temp_fit: acc must be 16-byte aligned");
+  SPFF_REQUIRE(s.n > 0 && s.n <= 65535 && s.d > 0 && s.h > 0 && s.w > 0, "prob_temp_fit: bad shape (N must be <= 65535)");
+  SPFF_REQUIRE(scale > 0.f, "prob_temp_fit: scale must be positive");
+  SPFF_REQUIRE(label_bytes == 1 || label_bytes == 8, "prob_temp_fit: labels must be uint8 or int64");
+  if (workspace_bytes < spff_prob_temp_fit_workspace(k, s, g)) {
+    spff::set_error("prob_temp_fit: workspace too small");
+    return SPFF_ERR_WORKSPACE;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long total = static_cast<long long>(s.n) * s.d * s.h * s.w;
+  const int blocks = static_cast<int>(prob_temp_fit_blocks(s));
+  auto part = static_cast<double*>(workspace);
+  if (label_bytes == 1)
+    spff::prob_temp_fit_kernel<uint8_t><<<blocks, spff::kTfThreads, 0, st>>>(
+        acc, k, total, scale, static_cast<const uint8_t*>(labels), ignore_index, betas, g, part);
+  else
+    spff::prob_temp_fit_kernel<long long><<<blocks, spff::kTfThreads, 0, st>>>(
+        acc, k, total, scale, static_cast<const long long*>(labels), ignore_index, betas, g, part);
+  spff::prob_temp_fit_reduce_kernel<<<1, 160, 0, st>>>(part, blocks, g, sums,
+                                                       reinterpret_cast<unsigned long long*>(counted));
+  SPFF_CUDA(cudaGetLastError());
+  return 0;
 }
 
 int spff_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr,

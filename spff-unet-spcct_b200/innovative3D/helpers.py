@@ -342,6 +342,75 @@ def sample_calibration(per_sample_calib, per_sample_brier=None, ece_bins: int = 
     return out
 
 
+def temperature_grid(t_max: float = 8.0, points: int = 33) -> np.ndarray:
+    """The inverse temperatures β = 1/T of `SpctEnsemble.fit_temperature`'s grid, ascending, rounded to fp32 (the values
+    the fit kernel evaluates): `points` (odd, 5..63) temperatures spaced geometrically over [1/t_max, t_max] (t_max > 1
+    and finite), so that T = 1 is the middle point, exactly."""
+    if isinstance(points, bool) or int(points) != points or not 5 <= points <= 63 or points % 2 == 0:
+        raise ValueError(f"points must be an odd integer in [5, 63], got {points!r}")
+    if not (math.isfinite(t_max) and t_max > 1.0):
+        raise ValueError(f"t_max must be finite and > 1, got {t_max!r}")
+    half = (int(points) - 1) // 2
+    e = np.arange(-half, half + 1, dtype=np.float64) / half
+    beta = np.power(float(t_max), e)
+    beta[half] = 1.0
+    return beta.astype(np.float32).astype(np.float64)
+
+
+def temperature_from_sums(betas, sums, counted) -> dict:
+    """The temperature that minimises the mean nll of the tempered pooled softmax, from the fit statistics of
+    `ops.prob_temp_fit` on a grid of inverse temperatures: betas [G] ascending, sums [2,G] (sum over the counted voxels
+    of the nll f(β_g) and of its derivative f'(β_g) = dnll/dβ), counted voxels.
+
+    f is convex in β, so f' is non-decreasing: the minimum lies in the interval where the summed f' changes sign. There
+    the estimate is the minimiser of the cubic Hermite interpolant of the nll from its values and derivatives at both
+    ends (the secant root of f' if the cubic has no minimum inside); with no sign change on the grid it is the end point
+    the slope points to and `at_bound` is True.
+
+    Returns {"temperature": 1/β̂, "nll": the INTERPOLATED mean nll at β̂, "nll_at_1": the mean nll at β = 1 (None when
+    1 is not a grid point), "grid": {"temperature": 1/betas, "nll": mean f, "dnll": mean f' (per unit β)},
+    "counted", "at_bound"}. ValueError when no voxel was counted."""
+    b = np.asarray(_as_numpy(betas), dtype=np.float64).reshape(-1)
+    s = np.asarray(_as_numpy(sums), dtype=np.float64)
+    n = int(np.asarray(_as_numpy(counted) if torch.is_tensor(counted) else counted).reshape(-1)[0])
+    if s.shape != (2, b.size):
+        raise ValueError(f"sums must be [2,{b.size}], got {s.shape}")
+    if b.size < 2 or np.any(np.diff(b) <= 0) or b[0] <= 0 or not np.all(np.isfinite(b)):
+        raise ValueError("betas must be at least two positive, finite, strictly ascending values")
+    if n <= 0:
+        raise ValueError("no counted voxel: every label is ignore_index or outside [0, K)")
+    f, d = s[0] / n, s[1] / n
+    at_bound = False
+    if d[0] >= 0.0 or d[-1] <= 0.0:
+        i = 0 if d[0] >= 0.0 else b.size - 1
+        at_bound = d[i] != 0.0
+        beta, nll = b[i], f[i]
+    else:
+        i = int(np.argmax(d >= 0.0)) - 1           # d[i] < 0 <= d[i + 1]
+        a, h = b[i], b[i + 1] - b[i]
+        c1 = h * d[i]
+        c2 = 3.0 * (f[i + 1] - f[i]) - h * (2.0 * d[i] + d[i + 1])
+        c3 = 2.0 * (f[i] - f[i + 1]) + h * (d[i] + d[i + 1])
+        t = None
+        if c3 != 0.0:                              # p'(t) = c1 + 2 c2 t + 3 c3 t^2: the root where p'' > 0
+            disc = c2 * c2 - 3.0 * c1 * c3
+            if disc >= 0.0:
+                q = -(c2 + math.copysign(math.sqrt(disc), c2))
+                for r in ((q / (3.0 * c3)) if q != 0.0 else None, (c1 / q) if q != 0.0 else None):
+                    if r is not None and 0.0 <= r <= 1.0 and 2.0 * c2 + 6.0 * c3 * r > 0.0:
+                        t = r
+                        break
+        elif c2 > 0.0:
+            t = -c1 / (2.0 * c2)
+        if t is None or not 0.0 <= t <= 1.0:      # the cubic degenerates: secant root of f'
+            t = -d[i] / (d[i + 1] - d[i])
+        beta = a + t * h
+        nll = f[i] + t * (c1 + t * (c2 + t * c3))
+    one = np.flatnonzero(b == 1.0)
+    return {"temperature": float(1.0 / beta), "nll": float(nll), "nll_at_1": float(f[one[0]]) if one.size else None,
+            "grid": {"temperature": 1.0 / b, "nll": f, "dnll": d}, "counted": n, "at_bound": bool(at_bound)}
+
+
 def per_class_metrics_2d(preds, labels, num_classes, smooth=1e-6, ignore_index=None):
     """2-D twin (helpers.py:728-779): same counting rules on [B,K,H,W] logits."""
     return per_class_metrics_3d(preds, labels, num_classes, smooth, ignore_index)

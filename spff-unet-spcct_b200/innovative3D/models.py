@@ -21,6 +21,7 @@ from __future__ import annotations
 
 import copy
 import dataclasses
+import math
 import os
 from typing import Dict, List, Optional
 
@@ -38,7 +39,8 @@ from spff_b200.sched import PlateauLR
 
 from .config import BEST_LR, IGNORE_INDEX, NUM_CLASSES, NUM_FRAMES
 from .helpers import (LOSS_REGISTRY, calibration_from_hist, ce_plus_macro_dice_loss, curves_from_hist,
-                      metrics_from_confusion, per_class_metrics_2d, per_class_metrics_3d)
+                      metrics_from_confusion, per_class_metrics_2d, per_class_metrics_3d, temperature_from_sums,
+                      temperature_grid)
 
 LOG_PER_CLASS = os.getenv("LOG_PER_CLASS", "1") == "1"
 # samples per group of the engine's schedule (activations of one group live at a time in fit_step)
@@ -1294,9 +1296,16 @@ class SpctEnsemble:
     `predict_uncertainty` gives per-voxel uncertainty maps (the predictive entropy H[p̄] and the mutual information
     between prediction and pass, H[p̄] - mean over passes of H[p]), and `eval_step` / `evaluate(calibration=T)` the
     calibration statistics of p̄ (helpers.calibration_from_hist). For one model, use SpctEnsemble([lit]): its MI is 0
-    and its entropy and calibration are the single model's."""
+    and its entropy and calibration are the single model's.
 
-    def __init__(self, members, tta: Optional[str] = None):
+    `temperature` T (> 0, finite; settable as `ens.temperature`) recalibrates the pooled distribution:
+    p̃_c = p̄_c^(1/T) / sum_c' p̄_c'^(1/T), which is softmax(z / T) for one member without TTA. p̃ replaces p̄ in
+    `predict_proba`, `predict_uncertainty`'s entropy, and the loss, curves and calibration of `eval_step` / `evaluate`;
+    the arg-max (labels, confusion, Dice) does not change, and the mutual information stays H[p̄] - mean H[p] of the
+    untempered passes (a temperature on the pool does not model the members' disagreement), bit for bit.
+    T = 1 is exactly the untempered computation. `fit_temperature` fits T on a validation set in one pass."""
+
+    def __init__(self, members, tta: Optional[str] = None, temperature: float = 1.0):
         if tta not in (None, "flip"):
             raise ValueError(f"tta must be None or 'flip', got {tta!r}")
         members = list(members)
@@ -1328,6 +1337,18 @@ class SpctEnsemble:
         self.num_classes = cfg0.num_classes
         self.flips = (0, 1, 2, 3) if tta == "flip" else (0,)
         self._copy_stream = None
+        self.temperature = temperature
+
+    @property
+    def temperature(self) -> float:
+        return self._temperature
+
+    @temperature.setter
+    def temperature(self, t: float):
+        t = float(t)
+        if not (math.isfinite(t) and t > 0.0):
+            raise ValueError(f"temperature must be positive and finite, got {t}")
+        self._temperature = t
 
     @property
     def device(self) -> torch.device:
@@ -1359,15 +1380,17 @@ class SpctEnsemble:
         engines = self._engines(x.shape[2])
         b, _, d, h, w = x.shape
         out = torch.empty(b, self.num_classes, d, h, w, dtype=torch.float16, device=self.device)
-        run_ensemble(engines, x.to(self.device), self.flips, sample_group or self.cores[0].sample_group, proba_out=out)
+        run_ensemble(engines, x.to(self.device), self.flips, sample_group or self.cores[0].sample_group, proba_out=out,
+                     inv_temperature=1.0 / self.temperature)
         return out
 
     @torch.no_grad()
     def predict_uncertainty(self, x, sample_group: Optional[int] = None) -> Dict[str, torch.Tensor]:
         """One pass over members x flips: {"labels": uint8 [B,F,H,W] (predict_labels), "entropy": float16 [B,F,H,W]
-        (H[p̄] = -sum_c p̄_c log p̄_c, nats), "mutual_info": float16 [B,F,H,W] (H[p̄] - mean over passes of H[p], clamped
-        at 0: the members' / flips' disagreement), "case_entropy", "case_mutual_info": float64 [B] (their means over
-        the voxels of each case, from sums of the per-voxel values rounded to 2^-24)}."""
+        (H[p̄] = -sum_c p̄_c log p̄_c, nats; H[p̃] with a temperature), "mutual_info": float16 [B,F,H,W] (H[p̄] - mean over
+        passes of H[p], clamped at 0: the members' / flips' disagreement; untempered whatever the temperature),
+        "case_entropy", "case_mutual_info": float64 [B] (their means over the voxels of each case, from sums of the
+        per-voxel values rounded to 2^-24)}."""
         x = self._images(x)
         engines = self._engines(x.shape[2])
         b, _, d, h, w = x.shape
@@ -1378,24 +1401,14 @@ class SpctEnsemble:
         sums = torch.zeros(2, dtype=torch.int64, device=dev)
         rows = torch.zeros(b, 2, dtype=torch.int64, device=dev)
         run_ensemble(engines, x.to(dev), self.flips, sample_group or self.cores[0].sample_group, labels_out=labels,
-                     entropy_out=ent, mi_out=mi, unc=sums, sample_unc=rows)
+                     entropy_out=ent, mi_out=mi, unc=sums, sample_unc=rows, inv_temperature=1.0 / self.temperature)
         case = rows.double() * (2.0 ** -24) / (d * h * w)
         return {"labels": labels, "entropy": ent, "mutual_info": mi, "case_entropy": case[:, 0],
                 "case_mutual_info": case[:, 1]}
 
-    @torch.no_grad()
-    def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False,
-                  sample_group: Optional[int] = None, curves=None, calibration=None):
-        """BaseLitModel.eval_step for the ensemble: the tally, per-sample rows, arg-max map and histograms of the
-        averaged softmax p̄ (same arguments, batch forms and return dict).
-
-        `calibration`: a bin count T in [2, 1024] (fresh zeros) or a contiguous int64 [3,T] histogram on the device to
-        accumulate into (as `curves`); adds "calib" ([3,T]: per confidence bin min(floor(conf * T), T - 1), conf = the
-        largest p̄_c, the counted voxels, the correct ones and the summed confidence in units of 2^-24), "brier" (fp64
-        [1], the summed Brier score) and "uncertainty" (int64 [2], the summed H[p̄] and mutual information in units of
-        2^-24 nats); with per_sample=True also "per_sample_calib" [B,3,T], "per_sample_brier" [B] and
-        "per_sample_uncertainty" (float64 [B,2], the mean H[p̄] and MI per case). helpers.calibration_from_hist /
-        sample_calibration turn them into ECE, reliability diagrams and error detection."""
+    def _batch(self, batch, sample_group: Optional[int]):
+        """(engines, images, labels, StagedBatch or None, group) of an evaluation batch: tuple or dict, host or device,
+        uint8 or int64 labels; host batches are staged group by group on the copy stream."""
         imgs, lbls = batch if isinstance(batch, (list, tuple)) else (batch["image"], batch["label"])
         imgs, lbls = self._images(imgs), _pick_first_if_seq(lbls)
         engines = self._engines(imgs.shape[2])
@@ -1412,6 +1425,24 @@ class SpctEnsemble:
         else:
             imgs = imgs.to(dev, non_blocking=True)
             lbls = lbls.to(dev, non_blocking=True)
+        return engines, imgs, lbls, staged, group
+
+    @torch.no_grad()
+    def eval_step(self, batch, tally: Optional[LossTally] = None, per_sample: bool = False, return_labels: bool = False,
+                  sample_group: Optional[int] = None, curves=None, calibration=None):
+        """BaseLitModel.eval_step for the ensemble: the tally, per-sample rows, arg-max map and histograms of the
+        averaged softmax p̄ (same arguments, batch forms and return dict).
+
+        `calibration`: a bin count T in [2, 1024] (fresh zeros) or a contiguous int64 [3,T] histogram on the device to
+        accumulate into (as `curves`); adds "calib" ([3,T]: per confidence bin min(floor(conf * T), T - 1), conf = the
+        largest p̄_c, the counted voxels, the correct ones and the summed confidence in units of 2^-24), "brier" (fp64
+        [1], the summed Brier score) and "uncertainty" (int64 [2], the summed H[p̄] and mutual information in units of
+        2^-24 nats); with per_sample=True also "per_sample_calib" [B,3,T], "per_sample_brier" [B] and
+        "per_sample_uncertainty" (float64 [B,2], the mean H[p̄] and MI per case). helpers.calibration_from_hist /
+        sample_calibration turn them into ECE, reliability diagrams and error detection. With a temperature, everything
+        but the arg-max and the mutual information is computed on p̃ (see the class)."""
+        engines, imgs, lbls, staged, group = self._batch(batch, sample_group)
+        dev = self.device
         k = self.num_classes
         tally = LossTally(k, dev) if tally is None else tally
         bsz = imgs.shape[0]
@@ -1432,7 +1463,8 @@ class SpctEnsemble:
         run_ensemble(engines, imgs, self.flips, group, labels=lbls, tally=tally, ignore_index=IGNORE_INDEX,
                      per_sample=rows, labels_out=labels, hist=hist, sample_hist=sample_hist, staged=staged,
                      unc=cal.get("unc"), sample_unc=cal.get("sample_unc"), calib=cal.get("calib"),
-                     sample_calib=cal.get("sample_calib"), brier=cal.get("brier"), sample_brier=cal.get("sample_brier"))
+                     sample_calib=cal.get("sample_calib"), brier=cal.get("brier"), sample_brier=cal.get("sample_brier"),
+                     inv_temperature=1.0 / self.temperature)
         out = {"loss": tally.loss(), "tally": tally, "per_sample": rows, "labels": labels, "hist": hist,
                "per_sample_hist": sample_hist}
         if calibration is not None:
@@ -1463,6 +1495,37 @@ class SpctEnsemble:
             cal["unc"] += out["uncertainty"]
             return out
         return _evaluate(k, dev, lambda t: t.loss(), batches, step, curves, calibration)
+
+    @torch.no_grad()
+    def fit_temperature(self, batches, t_max: float = 8.0, points: int = 33, sample_group: Optional[int] = None,
+                        apply: bool = True) -> dict:
+        """Temperature scaling fitted on a validation set in ONE pass over `batches` (the batch forms `evaluate` takes):
+        the T that minimises the mean nll of the tempered pooled softmax p̃ over the counted voxels (label in [0, K),
+        not the ignore index). Every group's accumulator is reduced on the device to the nll and its derivative at
+        each of `points` (odd, 5..63) temperatures spaced geometrically over [1/t_max, t_max] (T = 1 among them);
+        no probabilities are kept. Under torch.distributed every rank passes its own batches, the statistics are
+        all-reduced once and every rank gets the same T. The host then takes the minimiser of the cubic Hermite
+        interpolant in the bracketing interval (helpers.temperature_from_sums).
+
+        Returns {"temperature", "nll" (the INTERPOLATED mean nll at that temperature), "nll_at_1" (mean nll at T = 1,
+        untempered), "grid": {"temperature", "nll", "dnll" (d nll / d(1/T))} over the grid, "counted",
+        "at_bound" (True when the slope has no sign change on the grid: the temperature is then the end point; widen
+        t_max)}. With `apply` the ensemble's temperature is set to it. ValueError when no voxel is counted."""
+        betas_h = temperature_grid(t_max, points)
+        g, dev = betas_h.size, self.device
+        betas = torch.tensor(betas_h, dtype=torch.float32, device=dev)
+        sums = torch.zeros(2, g, dtype=torch.float64, device=dev)
+        counted = torch.zeros(1, dtype=torch.int64, device=dev)
+        for batch in batches:
+            engines, imgs, lbls, staged, group = self._batch(batch, sample_group)
+            run_ensemble(engines, imgs, self.flips, group, labels=lbls, ignore_index=IGNORE_INDEX, staged=staged,
+                         temp_fit=(betas, sums, counted))
+        dp.allreduce_temp_fit(sums, counted)
+        host = torch.cat([sums.view(-1), counted.double()]).cpu()   # one copy; the count is exact in fp64 below 2^53
+        out = temperature_from_sums(betas_h, host[:-1].view(2, g).numpy(), int(host[-1]))
+        if apply:
+            self.temperature = out["temperature"]
+        return out
 
 
 # Model families outside the hot path (UNETR / SwinUNETR wrappers, R2U-Net, ResUNet++, their helper blocks and losses:

@@ -102,6 +102,10 @@ _PROTOTYPES = {
     "spff_head_prob_accum_ent": [_P, _LL, c_int, _P, _P, c_int, Shape, c_int, c_int, _P, _P, _P],
     "spff_prob_finalize_unc": [_P, c_int, Shape, c_float, _P, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, c_int, _P, _P, _P,
                                POINTER(UncOut), _P],
+    "spff_prob_finalize_tempered": [_P, c_int, Shape, c_float, _P, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, c_int, _P, _P,
+                                    _P, POINTER(UncOut), c_float, _P],
+    "spff_prob_temp_fit_workspace": [c_int, Shape, c_int],
+    "spff_prob_temp_fit": [_P, c_int, Shape, c_float, _P, c_int, c_int, _P, c_int, _P, _P, _P, c_size_t, _P],
     "spff_count_valid": [_P, c_int, _LL, c_int, _P, _P],
     "spff_scale_by_count": [_P, _LL, _P, c_float, _P],
     "spff_loss_from_tally": [_P, _P, _P, c_int, c_double, _P, _P],
@@ -130,7 +134,7 @@ _SIZE_T_FUNCS = {"spff_conv3d_k3_wgrad_workspace", "spff_conv3d_stem_wgrad_works
                  "spff_convt_k122_wgrad_workspace", "spff_head_bwd_workspace", "spff_head_loss_workspace",
                  "spff_norm_act_reduce_workspace", "spff_norm_act_bwd_reduce_workspace",
                  "spff_convt_k222_wgrad_workspace", "spff_bn_coeffs_workspace", "spff_grid_aug_workspace",
-                 "spff_partial_colsum_workspace"}
+                 "spff_partial_colsum_workspace", "spff_prob_temp_fit_workspace"}
 
 
 def _declare():

@@ -62,6 +62,18 @@ def allreduce_calibration(calib: torch.Tensor, brier: torch.Tensor, unc: torch.T
             dist.all_reduce(t, op=dist.ReduceOp.SUM)
 
 
+def allreduce_temp_fit(sums: torch.Tensor, counted: torch.Tensor) -> None:
+    """Sum the temperature-fit statistics over ranks in place: the fp64 [2,G] sums of the tempered nll and its derivative
+    and the int64 [1] count of their voxels (one all-reduce: the count travels as the fp64 value it is, exact below
+    2^53), so every rank solves for the same temperature."""
+    _, n = world()
+    if n > 1:
+        buf = torch.cat([sums.reshape(-1), counted.to(torch.float64)])
+        dist.all_reduce(buf, op=dist.ReduceOp.SUM)
+        sums.copy_(buf[:-1].view_as(sums))
+        counted.copy_(buf[-1:].to(torch.int64))
+
+
 def shard_range(total: int, rank: int | None = None, world_size: int | None = None) -> Tuple[int, int]:
     """[lo, hi) of the `total` independent units (slices / sliding-window tiles = whole z-slices)
     owned by `rank`: contiguous, sizes differ by at most one. No collective is involved."""

@@ -731,7 +731,8 @@ def run_ensemble(engines: List[SpffEngine], x: torch.Tensor, flips: Tuple[int, .
                  mi_out: Optional[torch.Tensor] = None, unc: Optional[torch.Tensor] = None,
                  sample_unc: Optional[torch.Tensor] = None, calib: Optional[torch.Tensor] = None,
                  sample_calib: Optional[torch.Tensor] = None, brier: Optional[torch.Tensor] = None,
-                 sample_brier: Optional[torch.Tensor] = None):
+                 sample_brier: Optional[torch.Tensor] = None, inv_temperature: float = 1.0,
+                 temp_fit: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None):
     """Averaged softmax of several networks of one NetConfig over input flips (1 = H, 2 = W, 0 = none), sample group by
     sample group, with no logits in memory. Every member runs on the FIRST engine's inference buffers; for each group
     and member (outer) and flip (inner): flip the input (spff_grid_aug), forward, and add the head's softmax, mirrored
@@ -743,10 +744,19 @@ def run_ensemble(engines: List[SpffEngine], x: torch.Tensor, flips: Tuple[int, .
     information H[p̄] - mean over passes of H[p]; unc int64 [2] / sample_unc int64 [B,2] (+=) their sums in units of
     2^-24 nats; with labels calib int64 [3,T] / sample_calib [B,3,T] and brier fp64 [1] / sample_brier fp64 [B] (+=).
     The fp32 [group,d,h,w] expected-entropy plane rides the member x flip loop only when mi_out, unc or sample_unc is
-    given (the mutual information needs it); it is counted in the group size only then."""
+    given (the mutual information needs it); it is counted in the group size only then.
+
+    Temperature scaling: `inv_temperature` β = 1/T tempers p̄ in the finishing pass (ops.prob_finalize; β == 1.0 is the
+    untempered call). `temp_fit` = (betas fp32 [G], sums fp64 [2,G], counted int64 [1]), with labels, replaces the
+    finishing pass by ops.prob_temp_fit on each group's accumulator (+= the tempered nll and its derivative at each
+    β_g, and the counted voxels); no other output may be given then, and nothing is added to the group size."""
     first = engines[0]
     x = first._check_input(x)
     bsz, _, d, h, w = x.shape
+    if temp_fit is not None and (labels is None or tally is not None or per_sample is not None or labels_out is not None
+                                 or proba_out is not None or hist is not None or entropy_out is not None
+                                 or mi_out is not None or unc is not None or calib is not None):
+        raise ValueError("temp_fit needs labels and takes no other output")
     if labels is not None:
         if labels.shape != (bsz, d, h, w):
             raise ValueError(f"labels must be [B,F,H,W] = {(bsz, d, h, w)}, got {tuple(labels.shape)}")
@@ -788,6 +798,10 @@ def run_ensemble(engines: List[SpffEngine], x: torch.Tensor, flips: Tuple[int, .
                 beta = 1
         if staged is not None:
             staged.wait_labels(hi)
+        if temp_fit is not None:
+            ops.prob_temp_fit(a, first.cfg.num_classes, scale, rows(labels, lo, hi), temp_fit[0], temp_fit[1],
+                              ignore_index=ignore_index, counted=temp_fit[2])
+            continue
         u = ops.Uncertainty(ent=ent[:n] if ent is not None else None, entropy_out=rows(entropy_out, lo, hi),
                             mi_out=rows(mi_out, lo, hi), unc=unc, sample_unc=rows(sample_unc, lo, hi), calib=calib,
                             sample_calib=rows(sample_calib, lo, hi), brier=brier,
@@ -795,7 +809,7 @@ def run_ensemble(engines: List[SpffEngine], x: torch.Tensor, flips: Tuple[int, .
         ops.prob_finalize(a, first.cfg.num_classes, scale, labels=rows(labels, lo, hi), ignore_index=ignore_index,
                           tally=tl, per_sample=tuple(t[lo:hi] for t in per_sample) if per_sample is not None else None,
                           labels_out=rows(labels_out, lo, hi), hist=hist, sample_hist=rows(sample_hist, lo, hi),
-                          proba_out=rows(proba_out, lo, hi), unc=u)
+                          proba_out=rows(proba_out, lo, hi), unc=u, inv_temperature=inv_temperature)
 
 
 class StagedBatch:

@@ -9,6 +9,7 @@ from __future__ import annotations
 
 import ctypes
 import dataclasses
+import math
 from typing import Optional
 
 import torch
@@ -460,13 +461,18 @@ def _unc_struct(u: Uncertainty, n: int, vox: int) -> UncOut:
 
 
 def prob_finalize(acc, k: int, scale: float, labels=None, ignore_index: int = 255, tally=None, per_sample=None,
-                  labels_out=None, hist=None, sample_hist=None, proba_out=None, unc: Optional[Uncertainty] = None):
+                  labels_out=None, hist=None, sample_hist=None, proba_out=None, unc: Optional[Uncertainty] = None,
+                  inv_temperature: float = 1.0):
     """One pass over a spff_head_prob_accum accumulator acc (fp32 [n,d,h,w,16]): p̄ = scale * acc. Optional outputs:
     labels_out (uint8 [n,d,h,w], the first arg-max of acc over classes < k), proba_out (fp16 [n,k,d,h,w], p̄), and with
     labels (uint8 / int64 [n,d,h,w]) the tally (nll fp64 [1], count int64 [1], confusion int64 [k,k], +=) of
     head_eval on p̄, per_sample rows (fp64 [n], int64 [n], int64 [n,k,k]), hist (int64 [k,2,T]) and sample_hist
     (int64 [n,k,2,T]) of p̄ (spff_prob_finalize). With `unc` (an Uncertainty) also its maps, sums and calibration
-    histogram (spff_prob_finalize_unc); every other output is the same, bit for bit."""
+    histogram (spff_prob_finalize_unc); every other output is the same, bit for bit.
+
+    `inv_temperature` β = 1/T != 1.0 tempers the pooled distribution, p̃_c ∝ p̄_c^β, and p̃ replaces p̄ in every output
+    but the arg-max and the mutual information (spff_prob_finalize_tempered). β == 1.0 makes exactly the untempered
+    call."""
     assert acc.dtype == torch.float32 and acc.dim() == 5 and acc.shape[-1] == 16 and acc.is_contiguous()
     n, d, h, w, _ = acc.shape
     vox = n * d * h * w
@@ -494,6 +500,15 @@ def prob_finalize(acc, k: int, scale: float, labels=None, ignore_index: int = 25
         assert labels_out.dtype == torch.uint8 and labels_out.is_contiguous() and labels_out.numel() == vox
     if proba_out is not None:
         assert proba_out.dtype == torch.float16 and proba_out.is_contiguous() and tuple(proba_out.shape) == (n, k, d, h, w)
+    beta = float(inv_temperature)
+    if beta != 1.0:
+        if not (math.isfinite(beta) and beta > 0.0):
+            raise ValueError(f"inv_temperature must be positive and finite, got {inv_temperature}")
+        u = _unc_struct(unc, n, vox) if unc is not None else None
+        call("spff_prob_finalize_tempered", ptr(acc), int(k), s, float(scale), ptr(labels), lb, int(ignore_index),
+             ptr(nll), ptr(cnt), ptr(conf), *(ptr(t) for t in per), ptr(labels_out), int(bins), ptr(hist),
+             ptr(sample_hist), ptr(proba_out), ctypes.byref(u) if u is not None else None, beta, stream_ptr())
+        return
     if unc is None:
         call("spff_prob_finalize", ptr(acc), int(k), s, float(scale), ptr(labels), lb, int(ignore_index), ptr(nll),
              ptr(cnt), ptr(conf), *(ptr(t) for t in per), ptr(labels_out), int(bins), ptr(hist), ptr(sample_hist),
@@ -503,6 +518,26 @@ def prob_finalize(acc, k: int, scale: float, labels=None, ignore_index: int = 25
     call("spff_prob_finalize_unc", ptr(acc), int(k), s, float(scale), ptr(labels), lb, int(ignore_index), ptr(nll),
          ptr(cnt), ptr(conf), *(ptr(t) for t in per), ptr(labels_out), int(bins), ptr(hist), ptr(sample_hist),
          ptr(proba_out), ctypes.byref(u), stream_ptr())
+
+
+def prob_temp_fit(acc, k: int, scale: float, labels, betas, sums, ignore_index: int = 255, *, counted):
+    """Temperature-fit statistics on a spff_head_prob_accum accumulator acc (fp32 [n,d,h,w,16], p̄ = scale * acc): for
+    every voxel whose label (uint8 / int64 [n,d,h,w]) is in [0,k) and not ignore_index, and every β_g of `betas` (fp32
+    [G] on the device, G in [1, 64], each positive and finite: the caller's duty, the values are not read back), sums
+    (fp64 [2,G], +=) receives the tempered nll f(β_g) = log sum_c p̄_c^β - β log p̄_y in [0] and its derivative
+    f'(β_g) = sum_c p̃_c log p̄_c - log p̄_y in [1]; counted (int64 [1], +=) the voxels (spff_prob_temp_fit).
+    Bit-reproducible: per-block fp64 partials added in a fixed order."""
+    assert acc.dtype == torch.float32 and acc.dim() == 5 and acc.shape[-1] == 16 and acc.is_contiguous()
+    n, d, h, w, _ = acc.shape
+    s = Shape(n, d, h, w)
+    assert labels.is_contiguous() and labels.numel() == n * d * h * w
+    g = betas.numel()
+    assert betas.dtype == torch.float32 and betas.is_contiguous()
+    assert sums.dtype == torch.float64 and sums.is_contiguous() and tuple(sums.shape) == (2, g)
+    assert counted.dtype == torch.int64 and counted.numel() == 1
+    ws = workspace(int(_lib.lib.spff_prob_temp_fit_workspace(int(k), s, g)), acc.device)
+    call("spff_prob_temp_fit", ptr(acc), int(k), s, float(scale), ptr(labels), _label_bytes(labels), int(ignore_index),
+         ptr(betas), g, ptr(sums), ptr(counted), ptr(ws), ws.numel(), stream_ptr())
 
 
 def scale_by_count(g, count, factor: float = 1.0):
