@@ -894,11 +894,13 @@ ENTRY_POINTS = {
     "conv3d_k3_stat_slots": "size query; the fwd_stats / dgrad_stats replays allocate from it and check every slot",
     "conv3d_stem_stat_slots": "size query; the stem replay allocates from it and checks every slot",
     "gate_tables_fwd": "gate parameter tables [c, frames]: depend on the parameters only, not on the plane size "
-                       "(test_kernels_gpu.py::test_tail_table_grads)",
-    "gate_tables_bwd": "gate parameter tables: parameter-only work (test_kernels_gpu.py::test_tail_table_grads)",
-    "gate_micro_fwd": "works on per-plane statistics [n, d, c]; its cost and indexing do not depend on h, w "
-                      "(test_kernels_gpu.py::test_spff_tail_fwd_bwd)",
-    "gate_micro_bwd": "works on per-plane sums [n, d, c, 6]; independent of h, w (test_kernels_gpu.py::test_spff_tail_fwd_bwd)",
+                       "(test_gates_gpu.py::test_gate_tables_fwd, every frames 1..16 and c 32..512)",
+    "gate_tables_bwd": "gate parameter tables: parameter-only work (test_gates_gpu.py::test_gate_tables_bwd, "
+                       "test_gates_gpu.py::test_variant_configurations_through_gate_tables)",
+    "gate_micro_fwd": "works on per-plane statistics [n, d, c]; h, w enter only as the count h*w "
+                      "(test_gates_gpu.py::test_gate_micro_fwd, planes up to 512 x 512)",
+    "gate_micro_bwd": "works on per-plane sums [n, d, c, 6]; h, w enter only as the count h*w "
+                      "(test_gates_gpu.py::test_gate_micro_bwd, test_gates_gpu.py::test_variant_configurations_through_gate_tables)",
     "adam_step": "flat parameter update; independent of the slice size (test_kernels_gpu.py::test_adam)",
     "workspace": "host-side scratch allocator",
 }
